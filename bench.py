@@ -99,7 +99,12 @@ def parse():
     p.add_argument("--split", action="store_true",
                    help="single-GPU tuning aid: use the two-phase search_begin/search_end path (no reduction)")
     p.add_argument("--sweep-leaves", default="", help="c3: comma list: print recall/QPS for each L (stderr) and exit")
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write the results of the last timed step as DIR/<name>.npy (ids and counts as float64, distances "
+                        "as float32), so that two builds can be compared output for output")
     a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
     for k2, v in DEFAULTS[a.config].items():
         if getattr(a, k2, None) is None:
             setattr(a, k2, v)
@@ -108,6 +113,31 @@ def parse():
 
 def log(*a):
     print(*a, file=sys.stderr, flush=True)
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, ids, dists, counts):
+    """Writes one search step's results ([nq, k] ids and distances, [nq] counts; numpy or torch) as <out_dir>/ids.npy,
+    dists.npy and counts.npy.  Ids and counts are stored as float64, which holds every u32 exactly.  When the arrays
+    exceed DUMP_LIMIT_BYTES, a fixed seeded sample of query rows is written instead, and rows.npy lists which."""
+    arrs = {}
+    for name, v, dt in (("ids", ids, np.float64), ("dists", dists, np.float32), ("counts", counts, np.float64)):
+        v = v.cpu().numpy() if hasattr(v, "cpu") else np.asarray(v)
+        if v.dtype == np.int32:  # device results: the same u32 values as the host API returns (padding = 0xFFFFFFFF)
+            v = v.view(np.uint32)
+        arrs[name] = v.astype(dt)
+    nq = arrs["counts"].shape[0]
+    row_bytes = sum(v.nbytes for v in arrs.values()) // max(nq, 1) + 8
+    if nq * row_bytes > DUMP_LIMIT_BYTES:
+        rows = np.sort(np.random.default_rng(0).choice(nq, DUMP_LIMIT_BYTES // row_bytes, replace=False))
+        arrs = {name: v[rows] for name, v in arrs.items()}
+        arrs["rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in arrs.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v)
+    log(f"dumped {', '.join(f'{n}{list(v.shape)}' for n, v in arrs.items())} to {out_dir}")
 
 
 def noise_sigma(torch, dim, decay, device):
@@ -271,8 +301,10 @@ def reference_arm(a, emit):
         times = []
         for _ in range(steps):
             t = time.perf_counter()
-            oracle.bf_search(hx, hq[:nqs], a.k, measure, nthreads=nthreads)
+            res = oracle.bf_search(hx, hq[:nqs], a.k, measure, nthreads=nthreads)
             times.append(time.perf_counter() - t)
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, *res[1:4])
         cfg = bf_config(a)
         return finish(nqs, times, cfg, f"{nqs} queries per step against the full {a.n}x{a.dim} database; oracle/ C++ "
                                        "restatement of BruteForceSearcher::search_batched (one task per query)")
@@ -299,9 +331,11 @@ def reference_arm(a, emit):
     times = []
     for _ in range(steps):
         t = time.perf_counter()
-        oracle.treex_search(hc, hcb, hoff, hids, hpacked, raw, hq, min(a.leaves, hc.shape[0]), a.reorder, a.k,
-                            lut16=True, use_residuals=True, reorder_measure=measure, nthreads=nthreads)
+        res = oracle.treex_search(hc, hcb, hoff, hids, hpacked, raw, hq, min(a.leaves, hc.shape[0]), a.reorder, a.k,
+                                  lut16=True, use_residuals=True, reorder_measure=measure, nthreads=nthreads)
         times.append(time.perf_counter() - t)
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, *res[1:4])
     if a.config == "c3":
         cfg = c3_config(a, hc.shape[0], max(1, a.gpus), a.shard)
         sample = (f"{hq.shape[0]} queries per step of the same workload (index trained and encoded with plain torch ops, "
@@ -357,7 +391,7 @@ def bench_bf(a, emit, torch, pkg, dev, local_rank):
     torch.cuda.synchronize()
     e0.record()
     for st in range(a.steps):
-        s.search_batched(queries[st % 2], a.k)
+        last = s.search_batched(queries[st % 2], a.k)
     e1.record()
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1)
@@ -403,6 +437,8 @@ def bench_bf(a, emit, torch, pkg, dev, local_rank):
         out["cpu_baseline"] = {"value": nqc / (time.perf_counter() - t), "unit": "queries/s", "cores": nthreads,
                                "kind": "port", "sample": f"{nqc} queries of the same batch against the full database; "
                                "oracle/ C++ restatement of BruteForceSearcher::search_batched"}
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, *last)
     emit(out)
     return 0
 
@@ -732,9 +768,11 @@ def bench_sharded(a, emit, torch, dist, pkg, dev, rank, world, local_rank):
         barrier()
         e0.record()
         for s in range(a.steps):
-            step_device(queries[s % n_batches], L)
+            last = step_device(queries[s % n_batches], L)
         e1.record()
         barrier()
+        if L == L0:
+            head_out = last
         ms = e0.elapsed_time(e1)
         tcp = searcher.tc_profile()
         prof, launches = searcher.get_profile()
@@ -789,6 +827,8 @@ def bench_sharded(a, emit, torch, dist, pkg, dev, rank, world, local_rank):
            "scan_path": dict(zip(("tensor_core_chunks", "register_lut_chunks"), searcher.path_stats())),
            "sweep": [results[L] for L in sorted(results)], "checks": checks, "clocks": clocks,
            "build_seconds": time.time() - t0}
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, *head_out)
     emit(out)
     return 0
 
@@ -823,6 +863,7 @@ def recompute_lut16(torch, q, ids, dists, centers, codebook, index_ids, packed, 
 # ======================================================================================== main
 def main():
     a = parse()
+    sys.dont_write_bytecode = True  # the benchmark writes nothing into the tree (it may be read-only)
     # keep stdout clean for the single JSON line: libraries (NCCL banner, …) write to fd 1
     json_fd = os.dup(1)
     os.dup2(2, 1)
@@ -850,7 +891,7 @@ def main():
         dist.init_process_group("nccl", device_id=dev)
 
     pkg = importlib.import_module("scann-rust_b200")
-    pkg.build_lib.build()
+    pkg.load()  # the library __graft_entry__.build() compiled; missing is an error, never a rebuild
     if a.config in ("c1", "c2"):
         if rank != 0:
             return 0
@@ -1054,7 +1095,7 @@ def bench_c3(a, emit, torch, dist, pkg, dev, rank, world, local_rank):
     barrier()
     e0.record()
     for s in range(a.steps):
-        step_device(queries[s % n_batches], timed=True, nxt=queries[(s + 1) % n_batches])
+        last = step_device(queries[s % n_batches], timed=True, nxt=queries[(s + 1) % n_batches])
     e1.record()
     barrier()
     ms = e0.elapsed_time(e1)
@@ -1145,6 +1186,8 @@ def bench_c3(a, emit, torch, dist, pkg, dev, rank, world, local_rank):
         out["cpu_baseline"] = {"value": nqc / secs, "unit": "queries/s", "cores": nthreads, "kind": "port",
                                "sample": f"{nqc} queries of the same batch on the same index; oracle/ C++ restatement "
                                          "of the reference algorithm, one task per query over all host threads"}
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, *last)
     emit(out)
     return 0
 

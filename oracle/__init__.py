@@ -24,10 +24,16 @@ def build(force: bool = False) -> str:
     import fcntl
 
     src = os.path.join(_HERE, "scann_oracle.cpp")
+
+    def stale():
+        return force or not os.path.exists(_LIB_PATH) or os.path.getmtime(_LIB_PATH) < os.path.getmtime(src)
+
+    if not stale():  # up to date: touch nothing, so a built tree can be used read-only
+        return _LIB_PATH
     with open(os.path.join(_HERE, ".build.lock"), "w") as lock:  # ranks of one torchrun serialise here
         fcntl.flock(lock, fcntl.LOCK_EX)
         try:
-            if force or not os.path.exists(_LIB_PATH) or os.path.getmtime(_LIB_PATH) < os.path.getmtime(src):
+            if stale():
                 subprocess.check_call(["make", "-C", _HERE, "-B", "libscann_oracle.so"], stdout=subprocess.DEVNULL)
         finally:
             fcntl.flock(lock, fcntl.LOCK_UN)

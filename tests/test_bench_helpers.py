@@ -63,6 +63,51 @@ def test_reference_arm_runs_without_the_product_library():
     assert "libscann_b200" not in r.stderr and "libscann_oracle" in r.stderr
 
 
+def test_dump_outputs_is_identical_run_to_run(tmp_path):
+    """--dump-outputs writes the last timed step's results; with the same arguments two runs write the same arrays"""
+    dumps = []
+    for run in range(2):
+        out = tmp_path / f"run{run}"
+        cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--n", "20000", "--partitions",
+               "16", "--latent", "32", "--nq", "32", "--ref-queries", "16", "--steps", "2", "--warmup", "1", "--leaves",
+               "8", "--dump-outputs", str(out)]
+        r = subprocess.run(cmd, capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-2000:]
+        dumps.append({p.name: np.load(p) for p in sorted(out.iterdir())})
+    assert sorted(dumps[0]) == ["counts.npy", "dists.npy", "ids.npy"]
+    ids, dists, counts = dumps[0]["ids.npy"], dumps[0]["dists.npy"], dumps[0]["counts.npy"]
+    assert ids.shape == dists.shape == (16, 10) and counts.shape == (16,)
+    assert ids.dtype == counts.dtype == np.float64 and dists.dtype == np.float32
+    assert (counts == 10).all() and (np.diff(dists, axis=1) >= 0).all()
+    for name, v in dumps[0].items():
+        assert np.array_equal(v, dumps[1][name]), name
+
+
+def test_dump_outputs_samples_rows_above_the_size_cap(tmp_path, monkeypatch):
+    sys.path.insert(0, ROOT)
+    import bench
+
+    nq, k = 1000, 10
+    ids = np.arange(nq * k, dtype=np.int32).reshape(nq, k)
+    ids[0, -1] = -1  # device padding reads as the host API's 0xFFFFFFFF
+    dists = np.arange(nq * k, dtype=np.float32).reshape(nq, k)
+    counts = np.full(nq, k, np.uint32)
+    bench.dump_outputs(str(tmp_path / "all"), ids, dists, counts)
+    got = np.load(tmp_path / "all" / "ids.npy")
+    assert got.shape == (nq, k) and got[0, -1] == 0xFFFFFFFF and not (tmp_path / "all" / "rows.npy").exists()
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 64 << 10)
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), ids, dists, counts)
+    rows = np.load(tmp_path / "a" / "rows.npy")
+    assert np.array_equal(rows, np.load(tmp_path / "b" / "rows.npy"))  # a fixed sample
+    assert 0 < len(rows) < nq and (np.diff(rows) > 0).all()
+    total = sum(os.path.getsize(p) for p in (tmp_path / "a").iterdir())
+    assert total <= (64 << 10) + 4 * 128  # + the .npy headers
+    r = rows.astype(np.int64)
+    assert np.array_equal(np.load(tmp_path / "a" / "dists.npy"), dists[r])
+    assert np.array_equal(np.load(tmp_path / "a" / "ids.npy"), ids.view(np.uint32)[r].astype(np.float64))
+
+
 def test_ann_benchmark_recall_kat_and_flags():
     """src/bin/ann_benchmark.rs:481-492 (recall_at_k_basic) and the CLI spellings (:22-33,63-73)"""
     sys.path.insert(0, os.path.join(ROOT, "tools"))
