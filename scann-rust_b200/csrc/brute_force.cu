@@ -503,13 +503,21 @@ struct BfCore {
     }
     SCANN_TRY(launch_tc_scores(p, s));
     bf_overflow_kernel<<<static_cast<unsigned>((nqc + 255) / 256), 256, 0, s>>>(cnt, nqc, kTcCap, flag);
-    SCANN_CUDA(cudaMemcpyAsync(h_flag, flag, 4, cudaMemcpyDeviceToHost, s));
     // d. exact re-score (harmless if a list overflowed: the outputs are rewritten by the legacy chunk)
     SCANN_TRY(launch_rescore_lists(rescore_params(qsrc), lists, cnt, nqc, kTcCap, k, n, oid, od, oc, s,
                                    __builtin_huge_valf(), nullptr, qn, xmax2));
-    SCANN_CUDA(cudaStreamSynchronize(s));
-    *overflow = *h_flag != 0;
+    uint32_t f = 0;
+    SCANN_TRY(read_flag(s, &f));
+    *overflow = f != 0;
     if (!*overflow) ++stat_tc_chunks;
+    return SCANN_OK;
+  }
+
+  // the device flag (d_small[1]) once the work enqueued on s has finished
+  scann_status read_flag(cudaStream_t s, uint32_t* v) {
+    SCANN_CUDA(cudaMemcpyAsync(h_flag, d_small.p + 1, 4, cudaMemcpyDeviceToHost, s));
+    SCANN_CUDA(cudaStreamSynchronize(s));
+    *v = *h_flag;
     return SCANN_OK;
   }
 
@@ -520,13 +528,10 @@ struct BfCore {
     if (nq == 0) return SCANN_OK;
     SCANN_REQUIRE(queries && counts, SCANN_INVALID_ARGUMENT, "NULL buffer");
     std::lock_guard<std::mutex> lock(mu);
-    DeviceGuard g(device);
-    cudaStream_t s = memspace == SCANN_DEVICE ? static_cast<cudaStream_t>(user_stream)
-                                               : (user_stream ? static_cast<cudaStream_t>(user_stream) : stream);
-    StreamOrderScope in_order(order, s);
-    const bool host = memspace == SCANN_HOST;
+    CallScope call(device, order, memspace, user_stream, stream);
+    const cudaStream_t s = call.s;
     if (n == 0) {
-      if (host) memset(counts, 0, nq * sizeof(uint32_t));
+      if (memspace == SCANN_HOST) memset(counts, 0, nq * sizeof(uint32_t));
       else SCANN_CUDA(cudaMemsetAsync(counts, 0, nq * sizeof(uint32_t), s));
       return SCANN_OK;
     }
@@ -537,37 +542,24 @@ struct BfCore {
     const size_t k = max_results;
     const size_t chunk = std::min<size_t>(kTcQTile, nq);
     const size_t kpad = tc_kpad(dim), rpad = tc_rows_pad(n);
-    size_t need = Workspace::padded(tc_queries_pad(chunk, dim) * kpad * 2) + Workspace::padded(tc_queries_pad(chunk, dim) * 4) +
-                  Workspace::padded(chunk * 4) * 2 + Workspace::padded(chunk * kTcCap * 8) + 4096;
-    if (host) need += Workspace::padded(chunk * dim * 4) + 2 * Workspace::padded(chunk * k * 4) + Workspace::padded(chunk * 4);
-    SCANN_TRY(ws.reserve(need));
-    uint16_t* qbf = ws.take<uint16_t>(tc_queries_pad(chunk, dim) * kpad);
-    float* qn = ws.take<float>(tc_queries_pad(chunk, dim));
-    float* thr = ws.take<float>(chunk);
-    uint32_t* cnt = ws.take<uint32_t>(chunk);
-    unsigned long long* lists = ws.take<unsigned long long>(chunk * kTcCap);
-    float* hq = nullptr;
-    uint32_t *hids = nullptr, *hcounts = nullptr;
-    float* hd = nullptr;
-    if (host) {
-      hq = ws.take<float>(chunk * dim);
-      hids = ws.take<uint32_t>(chunk * k);
-      hd = ws.take<float>(chunk * k);
-      hcounts = ws.take<uint32_t>(chunk);
-    }
+    const QueryOut outs[] = {{ids, k * 4}, {dists, k * 4}, {counts, 4}};
+    SCANN_TRY(ws.reserve(Workspace::padded(tc_queries_pad(chunk, dim) * kpad * 2) +
+                         Workspace::padded(tc_queries_pad(chunk, dim) * 4) + Workspace::padded(chunk * 4) * 2 +
+                         Workspace::padded(chunk * kTcCap * 8) + 4096 + staging_bytes(memspace, chunk, dim, outs)));
+    // the flag collects every chunk's truncation (the kernels only set bits); every chunk is finished before the
+    // truncation is reported: all outputs are written
     uint32_t* flag = reinterpret_cast<uint32_t*>(d_small.p + 1);
-    bool truncated = false;  // every chunk is finished before the truncation is reported: all outputs are written
-    for (size_t q0 = 0; q0 < nq; q0 += chunk) {
-      const size_t nqc = std::min(chunk, nq - q0);
-      const float* qsrc = queries + q0 * dim;
-      if (host) {
-        SCANN_CUDA(cudaMemcpyAsync(hq, qsrc, nqc * dim * 4, cudaMemcpyHostToDevice, s));
-        qsrc = hq;
-      }
+    SCANN_CUDA(cudaMemsetAsync(flag, 0, 4, s));
+    SCANN_TRY(run_query_chunks(ws, memspace, s, queries, nq, dim, chunk, outs,
+                               [&](const float* qsrc, size_t, size_t nqc, void* const* o) -> scann_status {
+      uint16_t* qbf = ws.take<uint16_t>(tc_queries_pad(chunk, dim) * kpad);
+      float* qn = ws.take<float>(tc_queries_pad(chunk, dim));
+      float* thr = ws.take<float>(chunk);
+      uint32_t* cnt = ws.take<uint32_t>(chunk);
+      unsigned long long* lists = ws.take<unsigned long long>(chunk * kTcCap);
       SCANN_TRY(tc_prepare_queries(qsrc, nqc, dim, i8 ? scale : 1.0f, qbf, qn, s));
       bf_radius_thr_kernel<<<static_cast<unsigned>((nqc + 255) / 256), 256, 0, s>>>(qn, xmax2, radius, measure, nqc, i8 ? 1 : 0, thr);
       SCANN_CUDA(cudaMemsetAsync(cnt, 0, nqc * 4, s));
-      SCANN_CUDA(cudaMemsetAsync(flag, 0, 4, s));
       TcScoreParams p;
       p.q_bf16 = qbf;
       p.nq = nqc;
@@ -588,19 +580,11 @@ struct BfCore {
       p.sms = sm_count(device);
       SCANN_TRY(launch_tc_scores(p, s));
       bf_overflow_kernel<<<static_cast<unsigned>((nqc + 255) / 256), 256, 0, s>>>(cnt, nqc, kTcCap, flag);
-      uint32_t* oid = host ? hids : ids + q0 * k;
-      float* od = host ? hd : dists + q0 * k;
-      uint32_t* oc = host ? hcounts : counts + q0;
-      SCANN_TRY(launch_rescore_lists(rescore_params(qsrc), lists, cnt, nqc, kTcCap, k, n, oid, od, oc, s, radius, flag));
-      SCANN_CUDA(cudaMemcpyAsync(h_flag, flag, 4, cudaMemcpyDeviceToHost, s));
-      if (host) {
-        SCANN_CUDA(cudaMemcpyAsync(ids + q0 * k, hids, nqc * k * 4, cudaMemcpyDeviceToHost, s));
-        SCANN_CUDA(cudaMemcpyAsync(dists + q0 * k, hd, nqc * k * 4, cudaMemcpyDeviceToHost, s));
-        SCANN_CUDA(cudaMemcpyAsync(counts + q0, hcounts, nqc * 4, cudaMemcpyDeviceToHost, s));
-      }
-      SCANN_CUDA(cudaStreamSynchronize(s));
-      truncated = truncated || *h_flag != 0;
-    }
+      return launch_rescore_lists(rescore_params(qsrc), lists, cnt, nqc, kTcCap, k, n, static_cast<uint32_t*>(o[0]),
+                                  static_cast<float*>(o[1]), static_cast<uint32_t*>(o[2]), s, radius, flag);
+    }));
+    uint32_t truncated = 0;
+    SCANN_TRY(read_flag(s, &truncated));
     SCANN_REQUIRE(!truncated, SCANN_RESOURCE_EXHAUSTED,
                   "more than max_results = %zu points lie within the radius for some query (results are truncated "
                   "to the nearest ones)", max_results);
@@ -612,13 +596,10 @@ struct BfCore {
     if (nq == 0) return SCANN_OK;  // searcher.rs:175-177
     SCANN_REQUIRE(queries && counts, SCANN_INVALID_ARGUMENT, "NULL buffer");
     std::lock_guard<std::mutex> lock(mu);
-    DeviceGuard g(device);
-    cudaStream_t s = memspace == SCANN_DEVICE ? static_cast<cudaStream_t>(user_stream)
-                                               : (user_stream ? static_cast<cudaStream_t>(user_stream) : stream);
-    StreamOrderScope in_order(order, s);
-    const bool host = memspace == SCANN_HOST;
+    CallScope call(device, order, memspace, user_stream, stream);
+    const cudaStream_t s = call.s;
     if (n == 0) {  // empty dataset -> Ok(vec![]) (searcher.rs:78-80) before any dimension check
-      if (host) memset(counts, 0, nq * sizeof(uint32_t));
+      if (memspace == SCANN_HOST) memset(counts, 0, nq * sizeof(uint32_t));
       else SCANN_CUDA(cudaMemsetAsync(counts, 0, nq * sizeof(uint32_t), s));
       return SCANN_OK;
     }
@@ -634,64 +615,27 @@ struct BfCore {
     const size_t chunk = std::min<size_t>(use_tc ? kTcQTile : kQTile, nq);
     size_t need = legacy_need(chunk, kc);
     if (use_tc) need = std::max(need, tc_need(chunk, kk));
-    if (host)
-      need += Workspace::padded(chunk * dim * 4) + 2 * Workspace::padded(chunk * k * 4) + Workspace::padded(chunk * 4);
-    need += 4096;
-    SCANN_TRY(ws.reserve(need));
-    float* hq = nullptr;
-    uint32_t *hids = nullptr, *hcounts = nullptr;
-    float* hd = nullptr;
-    if (host) {
-      hq = ws.take<float>(chunk * dim);
-      hids = ws.take<uint32_t>(chunk * k);
-      hd = ws.take<float>(chunk * k);
-      hcounts = ws.take<uint32_t>(chunk);
-    }
-    const size_t ws_mark = ws.used;
-
-    for (size_t q0 = 0; q0 < nq; q0 += chunk) {
-      const size_t nqc = std::min(chunk, nq - q0);
-      const float* qsrc = queries + q0 * dim;
-      if (host) {
-        SCANN_CUDA(cudaMemcpyAsync(hq, qsrc, nqc * dim * 4, cudaMemcpyHostToDevice, s));
-        qsrc = hq;
-      }
-      uint32_t* oid = host ? hids : ids + q0 * k;
-      float* od = host ? hd : dists + q0 * k;
-      uint32_t* oc = host ? hcounts : counts + q0;
+    const QueryOut outs[] = {{ids, k * 4}, {dists, k * 4}, {counts, 4}};
+    SCANN_TRY(ws.reserve(need + staging_bytes(memspace, chunk, dim, outs) + 4096));
+    return run_query_chunks(ws, memspace, s, queries, nq, dim, chunk, outs,
+                            [&](const float* qsrc, size_t, size_t nqc, void* const* o) -> scann_status {
+      uint32_t* oid = static_cast<uint32_t*>(o[0]);
+      float* od = static_cast<float*>(o[1]);
+      uint32_t* oc = static_cast<uint32_t*>(o[2]);
+      const size_t mark = ws.used;
       bool overflow = true;
-      if (use_tc) {
-        ws.used = ws_mark;
-        SCANN_TRY(tc_chunk(qsrc, nqc, k, kk, oid, od, oc, s, &overflow));
-      }
+      if (use_tc) SCANN_TRY(tc_chunk(qsrc, nqc, k, kk, oid, od, oc, s, &overflow));
       if (overflow) {
-        ws.used = ws_mark;
+        ws.used = mark;
         SCANN_TRY(legacy_chunk(qsrc, nqc, k, kc, oid, od, oc, s));
       }
-      if (host) {
-        SCANN_CUDA(cudaMemcpyAsync(ids + q0 * k, hids, nqc * k * 4, cudaMemcpyDeviceToHost, s));
-        SCANN_CUDA(cudaMemcpyAsync(dists + q0 * k, hd, nqc * k * 4, cudaMemcpyDeviceToHost, s));
-        SCANN_CUDA(cudaMemcpyAsync(counts + q0, hcounts, nqc * 4, cudaMemcpyDeviceToHost, s));
-        SCANN_CUDA(cudaStreamSynchronize(s));
-      }
-    }
-    return SCANN_OK;
+      return SCANN_OK;
+    });
   }
 
-  void destroy() {
-    DeviceGuard g(device);
-    cudaDeviceSynchronize();
-    ws.release();
-    rows_f.free_();
-    rows_i.free_();
-    xn.free_();
-    rows_bf.free_();
-    hx.free_();
-    d_small.free_();
+  ~BfCore() {
     if (h_flag) cudaFreeHost(h_flag);
-    h_flag = nullptr;
     if (stream) cudaStreamDestroy(stream);
-    stream = nullptr;
   }
 };
 
@@ -828,8 +772,7 @@ scann_status scann_bf_create(const float* db, size_t n, size_t dim, size_t strid
   scann_bf* h = new scann_bf();
   scann_status st = h->core.init(db, n, dim, stride, measure, false, 1.0f, device, memspace);
   if (st != SCANN_OK) {
-    h->core.destroy();
-    delete h;
+    scann_bf_destroy(h);
     return st;
   }
   *out = h;
@@ -860,7 +803,8 @@ scann_status scann_bf_path_stats(scann_bf* h, uint64_t* tc_chunks, uint64_t* leg
 
 void scann_bf_destroy(scann_bf* h) {
   if (!h) return;
-  h->core.destroy();
+  scann::DeviceGuard g(h->core.device);
+  cudaDeviceSynchronize();
   delete h;
 }
 
@@ -878,8 +822,7 @@ scann_status scann_sq8_create(const int8_t* codes, size_t n, size_t dim, float s
   scann_sq8* h = new scann_sq8();
   scann_status st = h->core.init(codes, n, dim, dim, measure, true, scale, device, memspace);
   if (st != SCANN_OK) {
-    h->core.destroy();
-    delete h;
+    scann_sq8_destroy(h);
     return st;
   }
   *out = h;
@@ -903,7 +846,8 @@ scann_status scann_sq8_path_stats(scann_sq8* h, uint64_t* tc_chunks, uint64_t* l
 
 void scann_sq8_destroy(scann_sq8* h) {
   if (!h) return;
-  h->core.destroy();
+  scann::DeviceGuard g(h->core.device);
+  cudaDeviceSynchronize();
   delete h;
 }
 

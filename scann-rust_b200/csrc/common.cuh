@@ -67,11 +67,19 @@ struct StreamOrder {
     if (done) cudaEventDestroy(done);
   }
 };
-struct StreamOrderScope {
-  StreamOrder& o;
+
+// The device, stream and stream order of one call on a handle; the caller holds the handle's lock.  A SCANN_DEVICE call
+// runs on the caller's stream; a SCANN_HOST call on the caller's stream when one is given, else on the handle's own
+// (scann_b200.h).
+struct CallScope {
+  DeviceGuard g;
   cudaStream_t s;
-  StreamOrderScope(StreamOrder& o_, cudaStream_t s_) : o(o_), s(s_) { o.enter(s); }
-  ~StreamOrderScope() { o.leave(s); }
+  StreamOrder& order;
+  CallScope(int device, StreamOrder& o, int memspace, void* user_stream, cudaStream_t own)
+      : g(device), s(memspace == SCANN_DEVICE || user_stream ? static_cast<cudaStream_t>(user_stream) : own), order(o) {
+    order.enter(s);
+  }
+  ~CallScope() { order.leave(s); }
 };
 
 // grow-only device arena; one per handle, guarded by the handle's mutex
@@ -79,6 +87,10 @@ struct Workspace {
   char* base = nullptr;
   size_t cap = 0;
   size_t used = 0;
+  Workspace() = default;
+  Workspace(const Workspace&) = delete;
+  Workspace& operator=(const Workspace&) = delete;
+  ~Workspace() { release(); }
   scann_status reserve(size_t bytes);
   void reset() { used = 0; }
   template <class T>
@@ -97,6 +109,23 @@ template <class T>
 struct DevBuf {
   T* p = nullptr;
   size_t n = 0;
+  DevBuf() = default;
+  DevBuf(const DevBuf&) = delete;
+  DevBuf& operator=(const DevBuf&) = delete;
+  DevBuf(DevBuf&& o) noexcept : p(o.p), n(o.n) {
+    o.p = nullptr;
+    o.n = 0;
+  }
+  DevBuf& operator=(DevBuf&& o) noexcept {
+    if (this != &o) {
+      free_();
+      p = o.p;
+      n = o.n;
+      o.p = nullptr;
+      o.n = 0;
+    }
+    return *this;
+  }
   scann_status alloc(size_t count) {
     free_();
     n = count;
@@ -128,6 +157,56 @@ inline cudaMemcpyKind in_kind(int memspace) {
 }
 inline cudaMemcpyKind out_kind(int memspace) {
   return memspace == SCANN_DEVICE ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost;
+}
+
+// One output of a query-batched call: the caller's array, `bytes` per query; p == NULL: optional and not requested.
+struct QueryOut {
+  void* p;
+  size_t bytes;
+};
+
+// Workspace bytes run_query_chunks takes for staging: on SCANN_HOST the chunk's queries and every requested output.
+template <size_t N>
+size_t staging_bytes(int memspace, size_t chunk, size_t dim, const QueryOut (&outs)[N]) {
+  if (memspace != SCANN_HOST) return 0;
+  size_t b = Workspace::padded(chunk * dim * sizeof(float));
+  for (const QueryOut& o : outs)
+    if (o.p) b += Workspace::padded(chunk * o.bytes);
+  return b;
+}
+
+// Runs a batch of nq queries [nq][dim] in chunks of at most `chunk` queries as
+//   run(const float* device_queries, size_t q0, size_t nqc, void* const* device_outs)  -> scann_status
+// where device_outs[i] is outs[i] of the chunk (NULL when not requested).  SCANN_DEVICE: the caller's arrays at q0;
+// nothing is copied or synchronised.  SCANN_HOST: staging buffers taken from `ws` once (reserve staging_bytes() for
+// them); per chunk one copy of the queries in, one copy of every requested output out, one stream synchronisation.
+// The workspace is reset to the mark above the staging before every chunk: run takes its scratch from there.
+template <size_t N, class Run>
+scann_status run_query_chunks(Workspace& ws, int memspace, cudaStream_t s, const float* queries, size_t nq, size_t dim,
+                              size_t chunk, const QueryOut (&outs)[N], Run run) {
+  const bool host = memspace == SCANN_HOST;
+  float* hq = host ? ws.take<float>(chunk * dim) : nullptr;
+  void* stage[N];
+  for (size_t i = 0; i < N; ++i) stage[i] = host && outs[i].p ? ws.take<uint8_t>(chunk * outs[i].bytes) : nullptr;
+  const size_t mark = ws.used;
+  for (size_t q0 = 0; q0 < nq; q0 += chunk) {
+    const size_t nqc = nq - q0 < chunk ? nq - q0 : chunk;
+    ws.used = mark;
+    if (!host) {
+      void* dout[N];
+      for (size_t i = 0; i < N; ++i) dout[i] = outs[i].p ? static_cast<char*>(outs[i].p) + q0 * outs[i].bytes : nullptr;
+      SCANN_TRY(run(queries + q0 * dim, q0, nqc, dout));
+      continue;
+    }
+    SCANN_CUDA(cudaMemcpyAsync(hq, queries + q0 * dim, nqc * dim * sizeof(float), cudaMemcpyHostToDevice, s));
+    SCANN_TRY(run(static_cast<const float*>(hq), q0, nqc, stage));
+    for (size_t i = 0; i < N; ++i)
+      if (outs[i].p)
+        SCANN_CUDA(cudaMemcpyAsync(static_cast<char*>(outs[i].p) + q0 * outs[i].bytes, stage[i], nqc * outs[i].bytes,
+                                   cudaMemcpyDeviceToHost, s));
+    SCANN_CUDA(cudaStreamSynchronize(s));
+  }
+  return SCANN_OK;
 }
 
 int sm_count(int device);

@@ -226,38 +226,26 @@ __global__ void ids_in_range_kernel(const uint32_t* __restrict__ ids, size_t n, 
 struct scann_ivf {
   int device = 0;
   size_t K = 0, dim = 0, n = 0, num_raw = 0, stride = 0, S = 0, C = 0, ds = 0;
-  scann::DevBuf<float> centers, centersT, raw, codebook;
+  scann::CentreScorer part;
+  scann::DevBuf<float> raw, codebook;
   scann::DevBuf<uint32_t> ids;
   scann::DevBuf<uint64_t> pt_off;
   scann::DevBuf<uint8_t> codes;
-  scann::PartTc ptc;
   scann::Workspace ws;
   std::mutex mu;
   scann::StreamOrder order;
   cudaStream_t stream = nullptr;
-  int sms = 148;
+  ~scann_ivf() {
+    if (stream) cudaStreamDestroy(stream);
+  }
 };
 
 extern "C" {
 
 void scann_ivf_destroy(scann_ivf* h) {
   if (!h) return;
-  {
-    scann::DeviceGuard g(h->device);
-    cudaDeviceSynchronize();
-    h->ws.release();
-    h->centers.free_();
-    h->centersT.free_();
-    h->raw.free_();
-    h->codebook.free_();
-    h->ids.free_();
-    h->pt_off.free_();
-    h->codes.free_();
-    h->ptc.cbf.free_();
-    h->ptc.hx.free_();
-    h->ptc.small.free_();
-    if (h->stream) cudaStreamDestroy(h->stream);
-  }
+  scann::DeviceGuard g(h->device);
+  cudaDeviceSynchronize();
   delete h;
 }
 
@@ -292,7 +280,6 @@ scann_status scann_ivf_create(const float* centers, size_t K, size_t dim, const 
   h->S = codebook ? S : 0;
   h->C = codebook ? C : 0;
   h->ds = codebook ? dim / S : 0;
-  h->sms = sm_count(device);
   scann_status st = SCANN_OK;
   do {
     if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess) {
@@ -314,10 +301,7 @@ scann_status scann_ivf_create(const float* centers, size_t K, size_t dim, const 
       st = SCANN_INVALID_ARGUMENT;
       break;
     }
-    if ((st = h->centers.upload(centers, K * dim, memspace, s)) != SCANN_OK) break;
-    if ((st = h->centersT.alloc(K * dim)) != SCANN_OK) break;
-    launch_transpose(h->centers.p, K, dim, h->centersT.p, s);
-    if (part_tc_usable(K, dim) && (st = part_tc_prepare(h->centers.p, K, dim, &h->ptc, s)) != SCANN_OK) break;
+    if ((st = h->part.set(centers, K, dim, memspace, s)) != SCANN_OK) break;
     if ((st = h->ids.upload(ids, n, memspace, s)) != SCANN_OK) break;
     if ((st = h->pt_off.upload(off.data(), K + 1, SCANN_HOST, s)) != SCANN_OK) break;
     if (raw && (st = h->raw.upload(raw, num_raw * stride, memspace, s)) != SCANN_OK) break;
@@ -375,77 +359,50 @@ scann_status scann_ivf_search(scann_ivf* h, int mode, const float* queries, size
   if (mode == 1) SCANN_REQUIRE(h->codes.p != nullptr, SCANN_FAILED_PRECONDITION, "index has no hasher");
   if (reorder_measure >= 0) SCANN_REQUIRE(h->raw.p != nullptr, SCANN_FAILED_PRECONDITION, "Dataset not stored");
   std::lock_guard<std::mutex> lock(h->mu);
-  DeviceGuard g(h->device);
-  cudaStream_t s = memspace == SCANN_DEVICE ? static_cast<cudaStream_t>(stream)
-                                             : (stream ? static_cast<cudaStream_t>(stream) : h->stream);
-  StreamOrderScope in_order(h->order, s);
-  const bool host = memspace == SCANN_HOST;
+  CallScope call(h->device, h->order, memspace, stream, h->stream);
   const size_t K = h->K;
   if (L > K) L = K;
   size_t chunk = std::min(nq, std::max<size_t>(1, (size_t(256) << 20) / (K * 4)));
-  const size_t scr = std::max(chunk * K * 4, h->ptc.ready ? part_tc_scratch_bytes(K, h->dim, chunk) : size_t(0));
-  size_t need = Workspace::padded(scr) + Workspace::padded(chunk * L * 4) + 4096;
-  if (host) need += Workspace::padded(chunk * h->dim * 4) + 2 * Workspace::padded(chunk * k * 4) + Workspace::padded(chunk * 4);
-  SCANN_TRY(h->ws.reserve(need));
-  float* scratch = reinterpret_cast<float*>(h->ws.take<uint8_t>(scr));
-  uint32_t* tokens = h->ws.take<uint32_t>(chunk * L);
-  float* hq = nullptr;
-  uint32_t *hids = nullptr, *hcnt = nullptr;
-  float* hd = nullptr;
-  if (host) {
-    hq = h->ws.take<float>(chunk * h->dim);
-    hids = h->ws.take<uint32_t>(chunk * k);
-    hd = h->ws.take<float>(chunk * k);
-    hcnt = h->ws.take<uint32_t>(chunk);
-  }
+  const size_t scr = h->part.scratch_bytes(chunk);
+  const QueryOut outs[] = {{ids, k * 4}, {dists, k * 4}, {counts, 4}};
+  SCANN_TRY(h->ws.reserve(Workspace::padded(scr) + Workspace::padded(chunk * L * 4) + 4096 +
+                          staging_bytes(memspace, chunk, h->dim, outs)));
   const int p2 = next_pow2(static_cast<int>(k));
   const size_t smem = (k + kIvfChunk + p2) * 8 + 264 * 4 + (L + 1) * 4 + ((h->dim + 3) & ~size_t(3)) * 4 +
                       (mode == 1 ? h->S * h->C * 4 : 0) + 16;
   SCANN_REQUIRE(smem <= 227 * 1024, SCANN_RESOURCE_EXHAUSTED, "search needs %zu B of shared memory", smem);
   SCANN_CUDA(cudaFuncSetAttribute(ivf_topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-  for (size_t q0 = 0; q0 < nq; q0 += chunk) {
-    const size_t nqc = std::min(chunk, nq - q0);
-    const float* dq = queries + q0 * h->dim;
-    if (host) {
-      SCANN_CUDA(cudaMemcpyAsync(hq, dq, nqc * h->dim * 4, cudaMemcpyHostToDevice, s));
-      dq = hq;
-    }
-    if (h->ptc.ready)
-      SCANN_TRY(launch_partition_tc(h->ptc, h->centers.p, K, h->dim, dq, nqc, L, tokens, nullptr, scratch, h->sms, s));
-    else
-      SCANN_TRY(launch_partition(h->centersT.p, K, h->dim, dq, nqc, L, tokens, nullptr, scratch, s));
-    IvfArgs a;
-    a.tokens = tokens;
-    a.pt_off = h->pt_off.p;
-    a.ids = h->ids.p;
-    a.raw = h->raw.p;
-    a.stride = h->stride;
-    a.queries = dq;
-    a.codebook = h->codebook.p;
-    a.codes = h->codes.p;
-    a.dim = static_cast<int>(h->dim);
-    a.L = static_cast<int>(L);
-    a.k = static_cast<int>(k);
-    a.measure = measure;
-    a.lut_mode = mode;
-    a.S = static_cast<int>(h->S);
-    a.C = static_cast<int>(h->C);
-    a.ds = static_cast<int>(h->ds);
-    a.K = static_cast<uint32_t>(K);
-    a.reorder_measure = reorder_measure;
-    a.out_ids = host ? hids : ids + q0 * k;
-    a.out_dists = host ? hd : dists + q0 * k;
-    a.out_counts = host ? hcnt : counts + q0;
-    ivf_topk_kernel<<<static_cast<unsigned>(nqc), 256, smem, s>>>(a);
-    SCANN_CUDA(cudaGetLastError());
-    if (host) {
-      SCANN_CUDA(cudaMemcpyAsync(ids + q0 * k, hids, nqc * k * 4, cudaMemcpyDeviceToHost, s));
-      SCANN_CUDA(cudaMemcpyAsync(dists + q0 * k, hd, nqc * k * 4, cudaMemcpyDeviceToHost, s));
-      SCANN_CUDA(cudaMemcpyAsync(counts + q0, hcnt, nqc * 4, cudaMemcpyDeviceToHost, s));
-      SCANN_CUDA(cudaStreamSynchronize(s));
-    }
-  }
-  return SCANN_OK;
+  return run_query_chunks(h->ws, memspace, call.s, queries, nq, h->dim, chunk, outs,
+                          [&](const float* dq, size_t, size_t nqc, void* const* o) -> scann_status {
+                            void* scratch = h->ws.take<uint8_t>(scr);
+                            uint32_t* tokens = h->ws.take<uint32_t>(chunk * L);
+                            SCANN_TRY(h->part.select(dq, nqc, L, tokens, nullptr, scratch, call.s));
+                            IvfArgs a;
+                            a.tokens = tokens;
+                            a.pt_off = h->pt_off.p;
+                            a.ids = h->ids.p;
+                            a.raw = h->raw.p;
+                            a.stride = h->stride;
+                            a.queries = dq;
+                            a.codebook = h->codebook.p;
+                            a.codes = h->codes.p;
+                            a.dim = static_cast<int>(h->dim);
+                            a.L = static_cast<int>(L);
+                            a.k = static_cast<int>(k);
+                            a.measure = measure;
+                            a.lut_mode = mode;
+                            a.S = static_cast<int>(h->S);
+                            a.C = static_cast<int>(h->C);
+                            a.ds = static_cast<int>(h->ds);
+                            a.K = static_cast<uint32_t>(K);
+                            a.reorder_measure = reorder_measure;
+                            a.out_ids = static_cast<uint32_t*>(o[0]);
+                            a.out_dists = static_cast<float*>(o[1]);
+                            a.out_counts = static_cast<uint32_t*>(o[2]);
+                            ivf_topk_kernel<<<static_cast<unsigned>(nqc), 256, smem, call.s>>>(a);
+                            SCANN_CUDA(cudaGetLastError());
+                            return SCANN_OK;
+                          });
 }
 
 }  // extern "C"

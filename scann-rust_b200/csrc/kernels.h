@@ -5,11 +5,9 @@
 
 namespace scann {
 
-// partition.cu — exact centroid scoring + top-L (src/partitioning/tree_partitioner.rs:175-229)
-//   centersT: [dim][K] transposed centres; scratch: [nq][K] f32; tokens [nq][L]; dists [nq][L] or null
-scann_status launch_partition(const float* centersT, size_t K, size_t dim, const float* queries, size_t nq, size_t L,
-                              uint32_t* tokens, float* dists, float* scratch, cudaStream_t s);
-// tensor-core variant (tc_gemm.cu scores + exact re-score of the survivors; identical tokens and distances)
+// partition.cu — the partition stage: exact squared-L2 centroid scoring + top-L (src/partitioning/tree_partitioner.rs:
+// 175-229).  The centres are scored on the tensor cores (tc_gemm.cu scores + exact re-score of the survivors) when the
+// shape allows it, else on the CUDA cores; tokens and distances are identical either way.
 struct PartTc {
   DevBuf<uint16_t> cbf;  // centres as bf16 [tc_rows_pad(K)][tc_kpad(dim)]
   DevBuf<float> hx;      // |c|^2 / 2
@@ -17,14 +15,24 @@ struct PartTc {
   float cmax2 = 0.0f;    // max |c|^2
   bool ready = false;
 };
-bool part_tc_usable(size_t K, size_t dim);
-size_t part_tc_scratch_bytes(size_t K, size_t dim, size_t nq);
-scann_status part_tc_prepare(const float* centers /* device [K][dim] */, size_t K, size_t dim, PartTc* out,
-                             cudaStream_t s);
-scann_status launch_partition_tc(const PartTc& tc, const float* centers, size_t K, size_t dim, const float* queries,
-                                 size_t nq, size_t L, uint32_t* tokens, float* dists, void* scratch, int sms,
-                                 cudaStream_t s);
-void launch_transpose(const float* in, size_t rows, size_t cols, float* out, cudaStream_t s);
+class CentreScorer {
+ public:
+  // (re)loads the centres [K][dim] and derives the scoring operands; synchronises s
+  scann_status set(const float* centers, size_t K, size_t dim, int memspace, cudaStream_t s);
+  // device scratch select() needs for a batch of nq queries
+  size_t scratch_bytes(size_t nq) const;
+  // tokens [nq][L] (0xFFFFFFFF past min(L, K)), dists [nq][L] or null; all device pointers
+  scann_status select(const float* queries, size_t nq, size_t L, uint32_t* tokens, float* dists, void* scratch,
+                      cudaStream_t s) const;
+  const float* centers() const { return centers_.p; }  // device [K][dim] f32
+  int launches() const { return tc_.ready ? 3 : 2; }    // kernels one select() enqueues
+
+ private:
+  size_t K_ = 0, dim_ = 0;
+  DevBuf<float> centers_, centersT_;  // centersT_: [dim][K]
+  PartTc tc_;
+  int sms_ = 148;
+};
 
 // select.cu — final exact re-score + (dist, id) order, and the multi-GPU merge
 //   cand: [nq][kc] candidate row ids (0xFFFFFFFF = empty); writes ids/dists [nq][k], counts [nq]

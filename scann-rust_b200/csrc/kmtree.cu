@@ -211,6 +211,9 @@ struct scann_kmtree {
   std::mutex mu;
   scann::StreamOrder order;
   cudaStream_t stream = nullptr;
+  ~scann_kmtree() {
+    if (stream) cudaStreamDestroy(stream);
+  }
 };
 
 namespace scann {
@@ -448,28 +451,11 @@ scann_status scann_kmtree_search_leaves(scann_kmtree* h, const float* queries, s
                 qdim, h->dim);
   SCANN_REQUIRE(k <= 1024, SCANN_INVALID_ARGUMENT, "k %zu > 1024 unsupported", k);
   std::lock_guard<std::mutex> lock(h->mu);
-  DeviceGuard g(h->device);
-  cudaStream_t s = memspace == SCANN_DEVICE ? static_cast<cudaStream_t>(stream) : h->stream;
-  StreamOrderScope in_order(h->order, s);
-  const bool host = memspace == SCANN_HOST;
-  const size_t kk = std::max<size_t>(k, 1);
+  CallScope call(h->device, h->order, memspace, stream, h->stream);
   const size_t per_q = static_cast<size_t>(h->levels) * h->max_children * 8;
   size_t chunk = std::min(nq, std::max<size_t>(1, (size_t(256) << 20) / per_q));
-  size_t need = Workspace::padded(chunk * per_q);
-  if (host) need += Workspace::padded(chunk * h->dim * 4) + Workspace::padded(chunk * kk * 4) * 3 + Workspace::padded(chunk * 4);
-  SCANN_TRY(h->ws.reserve(need));
-  h->ws.reset();
-  unsigned long long* scratch = h->ws.take<unsigned long long>(chunk * per_q / 8);
-  float* dq = nullptr;
-  uint32_t *dn = nullptr, *dd = nullptr, *dc = nullptr;
-  float* ddist = nullptr;
-  if (host) {
-    dq = h->ws.take<float>(chunk * h->dim);
-    dn = h->ws.take<uint32_t>(chunk * kk);
-    ddist = h->ws.take<float>(chunk * kk);
-    dd = h->ws.take<uint32_t>(chunk * kk);
-    dc = h->ws.take<uint32_t>(chunk);
-  }
+  const QueryOut outs[] = {{leaf_nodes, k * 4}, {dists, k * 4}, {depths, k * 4}, {counts, 4}};
+  SCANN_TRY(h->ws.reserve(Workspace::padded(chunk * per_q) + staging_bytes(memspace, chunk, h->dim, outs)));
   TreeArgs t{h->centers.p, h->depth.p, h->child_begin.p, h->child_count.p, h->children.p, static_cast<int>(h->dim),
              h->max_children, h->levels};
   int mc2 = 1;
@@ -481,42 +467,21 @@ scann_status scann_kmtree_search_leaves(scann_kmtree* h, const float* queries, s
                       ((h->dim + 3) & ~size_t(3)) * 4;
   if (smem > 48 * 1024)
     SCANN_CUDA(cudaFuncSetAttribute(kmtree_search_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-  for (size_t q0 = 0; q0 < nq; q0 += chunk) {
-    const size_t nqc = std::min(chunk, nq - q0);
-    const float* q = queries + q0 * h->dim;
-    if (host) {
-      SCANN_CUDA(cudaMemcpyAsync(dq, q, nqc * h->dim * 4, cudaMemcpyHostToDevice, s));
-      q = dq;
-    }
-    kmtree_search_kernel<<<static_cast<unsigned>(nqc), 32, smem, s>>>(
-        t, q, static_cast<int>(nqc), static_cast<int>(k), scratch, host ? dn : leaf_nodes + q0 * k,
-        host ? ddist : (dists ? dists + q0 * k : nullptr), host ? dd : (depths ? depths + q0 * k : nullptr),
-        host ? dc : counts + q0);
-    SCANN_CUDA(cudaGetLastError());
-    if (host) {
-      if (k) SCANN_CUDA(cudaMemcpyAsync(leaf_nodes + q0 * k, dn, nqc * k * 4, cudaMemcpyDeviceToHost, s));
-      if (k && dists) SCANN_CUDA(cudaMemcpyAsync(dists + q0 * k, ddist, nqc * k * 4, cudaMemcpyDeviceToHost, s));
-      if (k && depths) SCANN_CUDA(cudaMemcpyAsync(depths + q0 * k, dd, nqc * k * 4, cudaMemcpyDeviceToHost, s));
-      SCANN_CUDA(cudaMemcpyAsync(counts + q0, dc, nqc * 4, cudaMemcpyDeviceToHost, s));
-      SCANN_CUDA(cudaStreamSynchronize(s));
-    }
-  }
-  return SCANN_OK;
+  return run_query_chunks(h->ws, memspace, call.s, queries, nq, h->dim, chunk, outs,
+                          [&](const float* q, size_t, size_t nqc, void* const* o) -> scann_status {
+                            unsigned long long* scratch = h->ws.take<unsigned long long>(chunk * per_q / 8);
+                            kmtree_search_kernel<<<static_cast<unsigned>(nqc), 32, smem, call.s>>>(
+                                t, q, static_cast<int>(nqc), static_cast<int>(k), scratch, static_cast<uint32_t*>(o[0]),
+                                static_cast<float*>(o[1]), static_cast<uint32_t*>(o[2]), static_cast<uint32_t*>(o[3]));
+                            SCANN_CUDA(cudaGetLastError());
+                            return SCANN_OK;
+                          });
 }
 
 void scann_kmtree_destroy(scann_kmtree* h) {
   if (!h) return;
-  {
-    scann::DeviceGuard g(h->device);
-    cudaDeviceSynchronize();
-    h->ws.release();
-    h->centers.free_();
-    h->depth.free_();
-    h->child_begin.free_();
-    h->child_count.free_();
-    h->children.free_();
-    if (h->stream) cudaStreamDestroy(h->stream);
-  }
+  scann::DeviceGuard g(h->device);
+  cudaDeviceSynchronize();
   delete h;
 }
 

@@ -230,20 +230,20 @@ static size_t part_tc_smem(int cap, size_t dim) {
   return static_cast<size_t>(kPtWarps) * (cap * 8 + 256 * 4 + cap * 4 + ((dim + 3) & ~size_t(3)) * 4);
 }
 
-bool part_tc_usable(size_t K, size_t dim) {
+static bool part_tc_usable(size_t K, size_t dim) {
   const char* e = getenv("SCANN_PART_NO_TC");
   if (e && e[0] == '1') return false;
   return tc_supported(dim) && K >= 256;  // small K: the exact kernel alone is cheaper than the extra launches
 }
 
-size_t part_tc_scratch_bytes(size_t K, size_t dim, size_t nq) {
+static size_t part_tc_scratch_bytes(size_t K, size_t dim, size_t nq) {
   return Workspace::padded(tc_queries_pad(nq, dim) * tc_kpad(dim) * 2) + Workspace::padded(tc_queries_pad(nq, dim) * 4) +
          Workspace::padded(nq * tc_rows_pad(K) * 4) + 1024;
 }
 
-scann_status part_tc_prepare(const float* centers, size_t K, size_t dim, PartTc* out, cudaStream_t s) {
+static scann_status part_tc_prepare(const float* centers, size_t K, size_t dim, PartTc* out, cudaStream_t s) {
   const size_t kpad = tc_kpad(dim), rpad = tc_rows_pad(K);
-  if (out->cbf.n != rpad * kpad) SCANN_TRY(out->cbf.alloc(rpad * kpad));  // kept across scann_part_update
+  if (out->cbf.n != rpad * kpad) SCANN_TRY(out->cbf.alloc(rpad * kpad));  // kept across CentreScorer::set
   if (out->hx.n != rpad) SCANN_TRY(out->hx.alloc(rpad));
   if (out->small.n != 1) SCANN_TRY(out->small.alloc(1));
   SCANN_TRY(tc_prepare_rows(centers, false, K, dim, dim, 1.0f, true, out->cbf.p, out->hx.p, out->small.p, s));
@@ -253,9 +253,9 @@ scann_status part_tc_prepare(const float* centers, size_t K, size_t dim, PartTc*
   return SCANN_OK;
 }
 
-scann_status launch_partition_tc(const PartTc& tc, const float* centers, size_t K, size_t dim, const float* queries,
-                                 size_t nq, size_t L, uint32_t* tokens, float* dists, void* scratch, int sms,
-                                 cudaStream_t s) {
+static scann_status launch_partition_tc(const PartTc& tc, const float* centers, size_t K, size_t dim,
+                                        const float* queries, size_t nq, size_t L, uint32_t* tokens, float* dists,
+                                        void* scratch, int sms, cudaStream_t s) {
   if (nq == 0 || L == 0) return SCANN_OK;
   SCANN_REQUIRE(L <= 1024, SCANN_INVALID_ARGUMENT, "partitions_to_search %zu > 1024 unsupported", L);
   const size_t kpad = tc_kpad(dim), rpad = tc_rows_pad(K), qpad = tc_queries_pad(nq, dim);
@@ -322,13 +322,14 @@ __global__ void transpose_kernel(const float* __restrict__ in, size_t rows, size
   }
 }
 
-void launch_transpose(const float* in, size_t rows, size_t cols, float* out, cudaStream_t s) {
+static void launch_transpose(const float* in, size_t rows, size_t cols, float* out, cudaStream_t s) {
   dim3 grid(static_cast<unsigned>((cols + 31) / 32), static_cast<unsigned>((rows + 31) / 32));
   transpose_kernel<<<grid, dim3(32, 8), 0, s>>>(in, rows, cols, out);
 }
 
-scann_status launch_partition(const float* centersT, size_t K, size_t dim, const float* queries, size_t nq, size_t L,
-                              uint32_t* tokens, float* dists, float* scratch, cudaStream_t s) {
+// centersT: [dim][K] transposed centres; scratch: [nq][K] f32
+static scann_status launch_partition(const float* centersT, size_t K, size_t dim, const float* queries, size_t nq,
+                                     size_t L, uint32_t* tokens, float* dists, float* scratch, cudaStream_t s) {
   if (nq == 0 || L == 0) return SCANN_OK;
   SCANN_REQUIRE(L <= 1024, SCANN_INVALID_ARGUMENT, "partitions_to_search %zu > 1024 unsupported", L);
   {
@@ -354,19 +355,46 @@ scann_status launch_partition(const float* centersT, size_t K, size_t dim, const
   return SCANN_OK;
 }
 
+scann_status CentreScorer::set(const float* centers, size_t K, size_t dim, int memspace, cudaStream_t s) {
+  K_ = K;
+  dim_ = dim;
+  if (centers_.n != K * dim) SCANN_TRY(centers_.alloc(K * dim));
+  if (centersT_.n != K * dim) SCANN_TRY(centersT_.alloc(K * dim));
+  SCANN_CUDA(cudaMemcpyAsync(centers_.p, centers, K * dim * sizeof(float), in_kind(memspace), s));
+  launch_transpose(centers_.p, K, dim, centersT_.p, s);
+  int device = 0;
+  SCANN_CUDA(cudaGetDevice(&device));
+  sms_ = sm_count(device);
+  tc_.ready = false;
+  if (part_tc_usable(K, dim)) SCANN_TRY(part_tc_prepare(centers_.p, K, dim, &tc_, s));
+  SCANN_CUDA(cudaStreamSynchronize(s));
+  return SCANN_OK;
+}
+
+size_t CentreScorer::scratch_bytes(size_t nq) const {
+  return std::max(nq * K_ * sizeof(float), tc_.ready ? part_tc_scratch_bytes(K_, dim_, nq) : size_t(0));
+}
+
+scann_status CentreScorer::select(const float* queries, size_t nq, size_t L, uint32_t* tokens, float* dists,
+                                  void* scratch, cudaStream_t s) const {
+  if (tc_.ready) return launch_partition_tc(tc_, centers_.p, K_, dim_, queries, nq, L, tokens, dists, scratch, sms_, s);
+  return launch_partition(centersT_.p, K_, dim_, queries, nq, L, tokens, dists, static_cast<float*>(scratch), s);
+}
+
 }  // namespace scann
 
 // ------------------------------------------------------------------------------------------ C ABI
 struct scann_part {
   int device = 0;
   size_t K = 0, dim = 0;
-  scann::DevBuf<float> centersT, centers;
-  scann::PartTc ptc;
-  int sms = 148;
+  scann::CentreScorer scorer;
   scann::Workspace ws;
   std::mutex mu;
   scann::StreamOrder order;
   cudaStream_t stream = nullptr;
+  ~scann_part() {
+    if (stream) cudaStreamDestroy(stream);
+  }
 };
 
 extern "C" {
@@ -384,26 +412,11 @@ scann_status scann_part_create(const float* centers, size_t K, size_t dim, int d
   h->device = device;
   h->K = K;
   h->dim = dim;
-  scann_status st = SCANN_OK;
-  do {
-    if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess) {
-      st = cuda_fail(cudaGetLastError(), "cudaStreamCreate", __FILE__, __LINE__);
-      break;
-    }
-    DevBuf<float> tmp;
-    if ((st = tmp.upload(centers, K * dim, memspace, h->stream)) != SCANN_OK) break;
-    if ((st = h->centersT.alloc(K * dim)) != SCANN_OK) break;
-    launch_transpose(tmp.p, K, dim, h->centersT.p, h->stream);
-    h->sms = sm_count(device);
-    if (part_tc_usable(K, dim)) {
-      if ((st = h->centers.upload(tmp.p, K * dim, SCANN_DEVICE, h->stream)) != SCANN_OK) break;
-      if ((st = part_tc_prepare(h->centers.p, K, dim, &h->ptc, h->stream)) != SCANN_OK) break;
-    }
-    if (cudaStreamSynchronize(h->stream) != cudaSuccess) {
-      st = cuda_fail(cudaGetLastError(), "sync", __FILE__, __LINE__);
-      break;
-    }
-  } while (0);
+  scann_status st;
+  if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess)
+    st = cuda_fail(cudaGetLastError(), "cudaStreamCreate", __FILE__, __LINE__);
+  else
+    st = h->scorer.set(centers, K, dim, memspace, h->stream);
   if (st != SCANN_OK) {
     scann_part_destroy(h);
     return st;
@@ -418,20 +431,8 @@ scann_status scann_part_update(scann_part* h, const float* centers, int memspace
   SCANN_REQUIRE(centers != nullptr, SCANN_INVALID_ARGUMENT, "NULL buffer");
   std::lock_guard<std::mutex> lock(h->mu);
   DeviceGuard g(h->device);
-  const float* src = centers;
-  DevBuf<float> tmp;
   if (memspace == SCANN_DEVICE) SCANN_CUDA(cudaDeviceSynchronize());  // the caller's array was produced on another stream
-  if (h->ptc.ready) {  // the tensor-core operands are derived from h->centers
-    SCANN_CUDA(cudaMemcpyAsync(h->centers.p, centers, h->K * h->dim * sizeof(float), in_kind(memspace), h->stream));
-    src = h->centers.p;
-  } else if (memspace == SCANN_HOST) {
-    SCANN_TRY(tmp.upload(centers, h->K * h->dim, SCANN_HOST, h->stream));
-    src = tmp.p;
-  }
-  launch_transpose(src, h->K, h->dim, h->centersT.p, h->stream);
-  if (h->ptc.ready) SCANN_TRY(part_tc_prepare(h->centers.p, h->K, h->dim, &h->ptc, h->stream));
-  SCANN_CUDA(cudaStreamSynchronize(h->stream));
-  return SCANN_OK;
+  return h->scorer.set(centers, h->K, h->dim, memspace, h->stream);
 }
 
 scann_status scann_part_select(scann_part* h, const float* queries, size_t nq, size_t qdim, size_t L,
@@ -444,62 +445,25 @@ scann_status scann_part_select(scann_part* h, const float* queries, size_t nq, s
                 qdim, h->dim);
   SCANN_REQUIRE(L <= 1024, SCANN_INVALID_ARGUMENT, "partitions_to_search %zu > 1024 unsupported", L);
   std::lock_guard<std::mutex> lock(h->mu);
-  DeviceGuard g(h->device);
-  cudaStream_t s = memspace == SCANN_DEVICE ? static_cast<cudaStream_t>(stream)
-                                             : (stream ? static_cast<cudaStream_t>(stream) : h->stream);
-  StreamOrderScope in_order(h->order, s);
+  CallScope call(h->device, h->order, memspace, stream, h->stream);
   // bounded scratch: process the batch in chunks of queries
   size_t chunk = (size_t(2) << 30) / (h->K * sizeof(float));  // dense score scratch: 2 GiB keeps >= 8192 rows per pass at K = 65,536
   if (chunk < 1) chunk = 1;
   if (chunk > nq) chunk = nq;
-  size_t need = Workspace::padded(std::max(chunk * h->K * sizeof(float),
-                                           h->ptc.ready ? part_tc_scratch_bytes(h->K, h->dim, chunk) : size_t(0)));
-  if (memspace == SCANN_HOST)
-    need += Workspace::padded(chunk * h->dim * 4) + Workspace::padded(chunk * L * 4) * 2;
-  SCANN_TRY(h->ws.reserve(need));
-  float* scratch = reinterpret_cast<float*>(h->ws.take<uint8_t>(std::max(
-      chunk * h->K * sizeof(float), h->ptc.ready ? part_tc_scratch_bytes(h->K, h->dim, chunk) : size_t(0))));
-  auto run = [&](const float* q, size_t nqc, uint32_t* tok, float* dd) -> scann_status {
-    if (h->ptc.ready)
-      return launch_partition_tc(h->ptc, h->centers.p, h->K, h->dim, q, nqc, L, tok, dd, scratch, h->sms, s);
-    return launch_partition(h->centersT.p, h->K, h->dim, q, nqc, L, tok, dd, scratch, s);
-  };
-  float* dq = nullptr;
-  uint32_t* dtok = nullptr;
-  float* ddist = nullptr;
-  if (memspace == SCANN_HOST) {
-    dq = h->ws.take<float>(chunk * h->dim);
-    dtok = h->ws.take<uint32_t>(chunk * L);
-    ddist = h->ws.take<float>(chunk * L);
-  }
-  for (size_t q0 = 0; q0 < nq; q0 += chunk) {
-    size_t nqc = nq - q0 < chunk ? nq - q0 : chunk;
-    const float* qin = queries + q0 * h->dim;
-    if (memspace == SCANN_HOST) {
-      SCANN_CUDA(cudaMemcpyAsync(dq, qin, nqc * h->dim * 4, cudaMemcpyHostToDevice, s));
-      SCANN_TRY(run(dq, nqc, dtok, ddist));
-      SCANN_CUDA(cudaMemcpyAsync(tokens + q0 * L, dtok, nqc * L * 4, cudaMemcpyDeviceToHost, s));
-      if (dists) SCANN_CUDA(cudaMemcpyAsync(dists + q0 * L, ddist, nqc * L * 4, cudaMemcpyDeviceToHost, s));
-      SCANN_CUDA(cudaStreamSynchronize(s));
-    } else {
-      SCANN_TRY(run(qin, nqc, tokens + q0 * L, dists ? dists + q0 * L : nullptr));
-    }
-  }
-  return SCANN_OK;
+  const size_t scratch_bytes = h->scorer.scratch_bytes(chunk);
+  const QueryOut outs[] = {{tokens, L * sizeof(uint32_t)}, {dists, L * sizeof(float)}};
+  SCANN_TRY(h->ws.reserve(Workspace::padded(scratch_bytes) + staging_bytes(memspace, chunk, h->dim, outs)));
+  return run_query_chunks(h->ws, memspace, call.s, queries, nq, h->dim, chunk, outs,
+                          [&](const float* q, size_t, size_t nqc, void* const* o) {
+                            return h->scorer.select(q, nqc, L, static_cast<uint32_t*>(o[0]), static_cast<float*>(o[1]),
+                                                    h->ws.take<uint8_t>(scratch_bytes), call.s);
+                          });
 }
 
 void scann_part_destroy(scann_part* h) {
   if (!h) return;
-  {
-    scann::DeviceGuard g(h->device);
-    h->ws.release();
-    h->centersT.free_();
-    h->centers.free_();
-    h->ptc.cbf.free_();
-    h->ptc.hx.free_();
-    h->ptc.small.free_();
-    if (h->stream) cudaStreamDestroy(h->stream);
-  }
+  scann::DeviceGuard g(h->device);
+  cudaDeviceSynchronize();
   delete h;
 }
 

@@ -457,7 +457,8 @@ struct scann_treeah {
   size_t K = 0, dim = 0, S = 0, ds = 0, SG = 0, n = 0, num_raw = 0, stride = 0;
   int use_residuals = 1, reorder_measure = SCANN_SQL2, pos_bits = 18;
   uint32_t max_leaf = 0;
-  scann::DevBuf<float> centers, centersT, codebook, raw;
+  scann::CentreScorer part;  // the partition stage; part.centers() are the f32 centres of the residual LUTs
+  scann::DevBuf<float> codebook, raw;
   const float* raw_p = nullptr;  // raw.p, or the caller's device array (SCANN_TREEAH_BORROW_RAW)
   bool raw_by_pos = false;       // SCANN_TREEAH_RAW_BY_POSITION
   bool reorder_on = true;        // scann_treeah_set_reorder: exact re-score of the R candidates (needs raw)
@@ -471,7 +472,6 @@ struct scann_treeah {
   size_t num_blocks = 0;
   scann::DevBuf<uint64_t> pt_off;
   scann::DevBuf<unsigned long long> stats;  // [0] algorithmic scan bytes, [1] pairs of the last search
-  scann::PartTc ptc;                        // tensor-core centroid scoring operands (partition.cu)
   scann::Workspace ws;
   std::mutex mu;
   scann::StreamOrder order;  // device work of successive calls, across streams
@@ -527,6 +527,10 @@ struct scann_treeah {
       for (cudaEvent_t e : t.e)
         if (e) cudaEventDestroy(e);
     tc_spans.clear();
+  }
+  ~scann_treeah() {
+    clear_spans();
+    if (stream) cudaStreamDestroy(stream);
   }
 };
 
@@ -651,9 +655,7 @@ static scann_status treeah_phase1(scann_treeah* h, const float* dq, size_t nq, s
   size_t max_items = P / G + 2 * std::min<size_t>(K, P) + 1;
 
   // centre-score scratch of the partition stage (not needed when the caller partitioned)
-  float* scratch = tokens_in ? nullptr
-                             : reinterpret_cast<float*>(h->ws.take<uint8_t>(std::max(
-                                   nq * K * 4, h->ptc.ready ? part_tc_scratch_bytes(K, h->dim, nq) : size_t(0))));
+  void* scratch = tokens_in ? nullptr : h->ws.take<uint8_t>(h->part.scratch_bytes(nq));
   uint32_t* tokens = h->ws.take<uint32_t>(P);
   if (tokens_in) tokens = const_cast<uint32_t*>(tokens_in);  // the caller partitioned (and keeps the array alive)
   uint32_t* leaf_cnt = h->ws.take<uint32_t>(2 * K + 4 * K * kWlPad);  // counts of the 2K virtual leaves + padded counters / cursors
@@ -672,12 +674,7 @@ static scann_status treeah_phase1(scann_treeah* h, const float* dq, size_t nq, s
 
   // 1. partition (K == 1 still goes through it: one centre, token 0)
   h->span_begin(0, s);
-  if (tokens_in) {
-  } else if (h->ptc.ready) {
-    SCANN_TRY(launch_partition_tc(h->ptc, h->centers.p, K, h->dim, dq, nq, L, tokens, nullptr, scratch, h->sms, s));
-  } else {
-    SCANN_TRY(launch_partition(h->centersT.p, K, h->dim, dq, nq, L, tokens, nullptr, scratch, s));
-  }
+  if (!tokens_in) SCANN_TRY(h->part.select(dq, nq, L, tokens, nullptr, scratch, s));
   h->span_end(s);
   // 2. worklist
   h->span_begin(1, s);
@@ -701,7 +698,7 @@ static scann_status treeah_phase1(scann_treeah* h, const float* dq, size_t nq, s
   a.codes = reinterpret_cast<const uint4*>(h->codes.p);
   a.blk_off = h->blk_off.p;
   a.pt_off = h->pt_off.p;
-  a.centers = h->centers.p;
+  a.centers = h->part.centers();
   a.codebook = h->codebook.p;
   a.queries = dq;
   a.items = items;
@@ -737,7 +734,7 @@ static scann_status treeah_phase1(scann_treeah* h, const float* dq, size_t nq, s
   h->ck.cand = cand;
   h->ck.cand_cnt = cand_cnt;
   h->ck.qthr = qthr;
-  h->prof_launches += (tokens_in ? 0 : (h->ptc.ready ? 3 : 2)) + 7;  // partition (2 or 3 kernels) + 7 worklist kernels
+  h->prof_launches += (tokens_in ? 0 : h->part.launches()) + 7;  // partition + 7 worklist kernels
   if (two_phase) {
     // 3a. probe of the class-A items: the first probe_blocks() blocks of every query's closest leaf prove a bound in
     // bounded time (a full scan of the largest leaves would serialise on a few CTAs); phase 2 scans them in full
@@ -789,7 +786,7 @@ static scann_status treeah_phase2(scann_treeah* h, bool two_phase, const float* 
     tp.leaf_perm = h->leaf_perm.p;
     tp.codes_rm = h->packed_rm.p;
     tp.queries = h->ck.dq;
-    tp.centers = h->centers.p;
+    tp.centers = h->part.centers();
     tp.codebook = h->codebook.p;
     tp.qthr = h->ck.qthr;
     tp.use_residuals = h->use_residuals;
@@ -877,12 +874,11 @@ static scann_status treeah_search_chunk(scann_treeah* h, const float* dq, size_t
   return treeah_phase2(h, tc, nullptr, d_ids, d_dists, d_counts, d_cand_ids, d_cand_dists, d_cand_counts, s);
 }
 
-static size_t treeah_chunk_bytes(const scann_treeah* h, size_t nq, size_t L, size_t R, size_t k, bool host,
-                                 bool have_tokens = false) {
+static size_t treeah_chunk_bytes(const scann_treeah* h, size_t nq, size_t L, size_t R, bool have_tokens = false) {
   size_t K = h->K, P = nq * L;
   size_t b = 0;
   auto add = [&](size_t bytes) { b += Workspace::padded(bytes); };
-  if (!have_tokens) add(std::max(nq * K * 4, h->ptc.ready ? part_tc_scratch_bytes(K, h->dim, nq) : size_t(0)));
+  if (!have_tokens) add(h->part.scratch_bytes(nq));
   add(P * 4);
   add((2 * K + 4 * K * kWlPad) * 4);
   add((2 * K + 1) * 4);
@@ -897,15 +893,6 @@ static size_t treeah_chunk_bytes(const scann_treeah* h, size_t nq, size_t L, siz
   add(P * 4);
   add(nq * 4);
   if (treeah_use_tc(h, nq, L, R)) b += tc_scan_workspace_bytes(nq, L, K, h->S, h->max_leaf, tc_qcap(R));
-  if (host) {
-    add(nq * h->dim * 4);
-    add(nq * k * 4);
-    add(nq * k * 4);
-    add(nq * 4);
-    add(nq * R * 4);
-    add(nq * R * 4);
-    add(nq * 4);
-  }
   return b + 4096;
 }
 
@@ -1010,10 +997,7 @@ scann_status scann_treeah_create_ex(const float* centers, size_t K, size_t dim, 
     DevBuf<uint32_t>& d_blk_leaf = h->blk_leaf;
     h->num_blocks = nb;
     size_t bpp = (S + 1) / 2;
-    if ((st = h->centers.upload(centers, K * dim, memspace, s)) != SCANN_OK) break;
-    if ((st = h->centersT.alloc(K * dim)) != SCANN_OK) break;
-    launch_transpose(h->centers.p, K, dim, h->centersT.p, s);
-    if (part_tc_usable(K, dim) && (st = part_tc_prepare(h->centers.p, K, dim, &h->ptc, s)) != SCANN_OK) break;
+    if ((st = h->part.set(centers, K, dim, memspace, s)) != SCANN_OK) break;
     if ((st = h->codebook.upload(codebook, S * 16 * h->ds, memspace, s)) != SCANN_OK) break;
     if ((st = h->ids.upload(ids, n, memspace, s)) != SCANN_OK) break;
     if ((st = h->pt_off.upload(off.data(), K + 1, SCANN_HOST, s)) != SCANN_OK) break;
@@ -1035,10 +1019,7 @@ scann_status scann_treeah_create_ex(const float* centers, size_t K, size_t dim, 
     }
     if (h->tc_ok) {  // the tensor-core scan reads the row-major PackedCodes4Bit rows (one point per thread)
       cudaStreamSynchronize(s);  // the repack kernel has read d_packed
-      h->packed_rm.p = d_packed.p;
-      h->packed_rm.n = d_packed.n;
-      d_packed.p = nullptr;
-      d_packed.n = 0;
+      h->packed_rm = std::move(d_packed);
     }
     h->raw_by_pos = raw != nullptr && (flags & SCANN_TREEAH_RAW_BY_POSITION) != 0;
     if (raw && (flags & SCANN_TREEAH_BORROW_RAW)) {
@@ -1077,61 +1058,35 @@ scann_status scann_treeah_search(scann_treeah* h, const float* queries, size_t n
                 "cand_ids and cand_dists go together");
   std::lock_guard<std::mutex> lock(h->mu);
   SCANN_REQUIRE(!h->split_active, SCANN_FAILED_PRECONDITION, "a split search is in flight on this handle");
-  DeviceGuard g(h->device);
-  cudaStream_t s = memspace == SCANN_DEVICE ? static_cast<cudaStream_t>(stream)
-                                             : (stream ? static_cast<cudaStream_t>(stream) : h->stream);
-  StreamOrderScope in_order(h->order, s);
+  CallScope call(h->device, h->order, memspace, stream, h->stream);
+  const cudaStream_t s = call.s;
   if (L > h->K) L = h->K;  // partition() returns min(L, K) tokens (tree_partitioner.rs:214)
   const size_t Reff = R < 1 ? 1 : R;  // R == 0 (k*multiplier < 1) -> no candidates
   // chunk the batch so that the candidate buffer stays <= 1 GiB and the centre-distance scratch <= 512 MiB
   size_t chunk = nq;
   chunk = std::min(chunk, std::max<size_t>(1, (size_t(1) << 30) / (L * Reff * 8)));
   chunk = std::min(chunk, std::max<size_t>(1, (size_t(512) << 20) / (h->K * 4)));
-  const bool host = memspace == SCANN_HOST;
-  SCANN_TRY(h->ws.reserve(treeah_chunk_bytes(h, chunk, L, Reff, k, host)));
+  const QueryOut outs[] = {{ids, k * 4}, {dists, k * 4}, {counts, 4},
+                           {cand_ids, R * 4}, {cand_dists, R * 4}, {cand_counts, 4}};
+  SCANN_TRY(h->ws.reserve(treeah_chunk_bytes(h, chunk, L, Reff) + staging_bytes(memspace, chunk, h->dim, outs)));
   SCANN_CUDA(cudaMemsetAsync(h->stats.p, 0, 4 * sizeof(unsigned long long), s));
-  for (size_t q0 = 0; q0 < nq; q0 += chunk) {
-    size_t nqc = std::min(chunk, nq - q0);
-    h->ws.reset();
-    const float* dq = queries + q0 * h->dim;
-    uint32_t *d_ids = ids + q0 * k, *d_counts = counts + q0;
-    float* d_dists = dists + q0 * k;
-    uint32_t* d_cid = cand_ids ? cand_ids + q0 * R : nullptr;
-    float* d_cd = cand_dists ? cand_dists + q0 * R : nullptr;
-    uint32_t* d_cc = cand_counts ? cand_counts + q0 : nullptr;
-    if (host) {
-      float* t = h->ws.take<float>(nqc * h->dim);
-      SCANN_CUDA(cudaMemcpyAsync(t, dq, nqc * h->dim * 4, cudaMemcpyHostToDevice, s));
-      dq = t;
-      d_ids = h->ws.take<uint32_t>(nqc * k);
-      d_dists = h->ws.take<float>(nqc * k);
-      d_counts = h->ws.take<uint32_t>(nqc);
-      d_cid = h->ws.take<uint32_t>(nqc * Reff);
-      d_cd = h->ws.take<float>(nqc * Reff);
-      d_cc = h->ws.take<uint32_t>(nqc);
-    }
+  return run_query_chunks(h->ws, memspace, s, queries, nq, h->dim, chunk, outs,
+                          [&](const float* dq, size_t, size_t nqc, void* const* o) -> scann_status {
+    uint32_t* d_ids = static_cast<uint32_t*>(o[0]);
+    float* d_dists = static_cast<float*>(o[1]);
+    uint32_t* d_counts = static_cast<uint32_t*>(o[2]);
+    uint32_t* d_cc = static_cast<uint32_t*>(o[5]);
     if (R == 0) {
       // (k as f32 * multiplier) as usize == 0: FastTopNeighbors(0) keeps nothing -> empty results
       SCANN_CUDA(cudaMemsetAsync(d_ids, 0xFF, nqc * k * 4, s));
       SCANN_CUDA(cudaMemsetAsync(d_dists, 0x7F, nqc * k * 4, s));  // 0x7F7F7F7F = 3.39e38: padding, never uninitialised
       SCANN_CUDA(cudaMemsetAsync(d_counts, 0, nqc * 4, s));
       if (d_cc) SCANN_CUDA(cudaMemsetAsync(d_cc, 0, nqc * 4, s));
-    } else {
-      SCANN_TRY(treeah_search_chunk(h, dq, nqc, L, R, k, d_ids, d_dists, d_counts, d_cid, d_cd, d_cc, s));
+      return SCANN_OK;
     }
-    if (host) {
-      SCANN_CUDA(cudaMemcpyAsync(ids + q0 * k, d_ids, nqc * k * 4, cudaMemcpyDeviceToHost, s));
-      SCANN_CUDA(cudaMemcpyAsync(dists + q0 * k, d_dists, nqc * k * 4, cudaMemcpyDeviceToHost, s));
-      SCANN_CUDA(cudaMemcpyAsync(counts + q0, d_counts, nqc * 4, cudaMemcpyDeviceToHost, s));
-      if (cand_ids && R > 0) {
-        SCANN_CUDA(cudaMemcpyAsync(cand_ids + q0 * R, d_cid, nqc * R * 4, cudaMemcpyDeviceToHost, s));
-        SCANN_CUDA(cudaMemcpyAsync(cand_dists + q0 * R, d_cd, nqc * R * 4, cudaMemcpyDeviceToHost, s));
-      }
-      if (cand_counts) SCANN_CUDA(cudaMemcpyAsync(cand_counts + q0, d_cc, nqc * 4, cudaMemcpyDeviceToHost, s));
-      SCANN_CUDA(cudaStreamSynchronize(s));
-    }
-  }
-  return SCANN_OK;
+    return treeah_search_chunk(h, dq, nqc, L, R, k, d_ids, d_dists, d_counts, static_cast<uint32_t*>(o[3]),
+                               static_cast<float*>(o[4]), d_cc, s);
+  });
 }
 
 scann_status scann_treeah_last_scan_bytes(scann_treeah* h, uint64_t* bytes, uint64_t* pairs) {
@@ -1162,19 +1117,14 @@ scann_status scann_treeah_partition(scann_treeah* h, const float* queries, size_
   SCANN_REQUIRE(!h->split_active, SCANN_FAILED_PRECONDITION, "a split search is in flight on this handle");
   std::lock_guard<std::mutex> lock(h->mu);
   SCANN_REQUIRE(!h->split_active, SCANN_FAILED_PRECONDITION, "a split search is in flight on this handle");
-  DeviceGuard g(h->device);
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  StreamOrderScope in_order(h->order, s);
+  CallScope call(h->device, h->order, SCANN_DEVICE, stream, h->stream);
   const size_t K = h->K;
   const size_t Leff = std::min(L, K);
   SCANN_REQUIRE(Leff == L, SCANN_INVALID_ARGUMENT, "partitions_to_search %zu > %zu partitions", L, K);
-  const size_t need = std::max(nq * K * 4, h->ptc.ready ? part_tc_scratch_bytes(K, h->dim, nq) : size_t(0)) + 4096;
-  SCANN_TRY(h->ws.reserve(need));
-  float* scratch = reinterpret_cast<float*>(h->ws.take<uint8_t>(need - 4096));
-  h->prof_launches += h->ptc.ready ? 3 : 2;
-  if (h->ptc.ready)
-    return launch_partition_tc(h->ptc, h->centers.p, K, h->dim, queries, nq, L, tokens, nullptr, scratch, h->sms, s);
-  return launch_partition(h->centersT.p, K, h->dim, queries, nq, L, tokens, nullptr, scratch, s);
+  const size_t scratch_bytes = h->part.scratch_bytes(nq);
+  SCANN_TRY(h->ws.reserve(scratch_bytes + 4096));
+  h->prof_launches += h->part.launches();
+  return h->part.select(queries, nq, L, tokens, nullptr, h->ws.take<uint8_t>(scratch_bytes), call.s);
 }
 
 scann_status scann_treeah_search_begin(scann_treeah* h, const float* queries, size_t nq, size_t qdim, size_t L,
@@ -1192,17 +1142,12 @@ scann_status scann_treeah_search_begin(scann_treeah* h, const float* queries, si
                 SCANN_INVALID_ARGUMENT, "batch of %zu queries is too large for the split search (split it)", nq);
   std::lock_guard<std::mutex> lock(h->mu);
   SCANN_REQUIRE(!h->split_active, SCANN_FAILED_PRECONDITION, "scann_treeah_search_begin called twice without _end");
-  DeviceGuard g(h->device);
-  cudaStream_t s = static_cast<cudaStream_t>(stream);
-  h->order.enter(s);
-  scann_status st = h->ws.reserve(treeah_chunk_bytes(h, nq, L, R, k, false, tokens != nullptr));
-  if (st == SCANN_OK) {
-    cudaMemsetAsync(h->stats.p, 0, 4 * sizeof(unsigned long long), s);
-    h->ws.reset();
-    st = treeah_phase1(h, queries, nq, L, R, k, true, tau_out, tokens, s);
+  {
+    CallScope call(h->device, h->order, SCANN_DEVICE, stream, h->stream);
+    SCANN_TRY(h->ws.reserve(treeah_chunk_bytes(h, nq, L, R, tokens != nullptr)));
+    cudaMemsetAsync(h->stats.p, 0, 4 * sizeof(unsigned long long), call.s);
+    SCANN_TRY(treeah_phase1(h, queries, nq, L, R, k, true, tau_out, tokens, call.s));
   }
-  h->order.leave(s);
-  if (st != SCANN_OK) return st;
   // The handle is marked busy, not locked: every other entry point answers FAILED_PRECONDITION until _end (or _abort),
   // so nothing can be left locked by a caller that fails between the two calls.
   h->split_active = true;
@@ -1228,10 +1173,8 @@ scann_status scann_treeah_search_end(scann_treeah* h, const float* tau_in, uint3
     set_error("NULL buffer");
     st = SCANN_INVALID_ARGUMENT;
   } else {
-    DeviceGuard g(h->device);
-    cudaStream_t s = static_cast<cudaStream_t>(stream);
-    StreamOrderScope in_order(h->order, s);
-    st = treeah_phase2(h, true, tau_in, ids, dists, counts, nullptr, nullptr, nullptr, s);
+    CallScope call(h->device, h->order, SCANN_DEVICE, stream, h->stream);
+    st = treeah_phase2(h, true, tau_in, ids, dists, counts, nullptr, nullptr, nullptr, call.s);
   }
   h->split_active = false;
   return st;
@@ -1339,28 +1282,8 @@ scann_status scann_treeah_set_reorder(scann_treeah* h, int enable) {
 
 void scann_treeah_destroy(scann_treeah* h) {
   if (!h) return;
-  {
-    scann::DeviceGuard g(h->device);
-    cudaDeviceSynchronize();
-    h->ws.release();
-    h->centers.free_();
-    h->centersT.free_();
-    h->codebook.free_();
-    h->raw.free_();
-    h->codes.free_();
-    h->ids.free_();
-    h->blk_off.free_();
-    h->pt_off.free_();
-    h->leaf_perm.free_();
-    h->blk_leaf.free_();
-    h->allow_blk.free_();
-    h->packed_rm.free_();
-    h->ptc.cbf.free_();
-    h->ptc.hx.free_();
-    h->ptc.small.free_();
-    h->stats.free_();
-    if (h->stream) cudaStreamDestroy(h->stream);
-  }
+  scann::DeviceGuard g(h->device);
+  cudaDeviceSynchronize();
   delete h;
 }
 
