@@ -229,6 +229,45 @@ __device__ __forceinline__ void scan_block(const uint4* __restrict__ blk, int SG
 }
 
 // ---- warp-level exact selection on u32 keys in shared memory -----------------------------------
+// One radix digit: given a 256-bin histogram (shared memory of the warp) of the keys still in play and the rank
+// need >= 1 among them, d = the bin that holds the need-th smallest and below = the keys in the bins before it.
+__device__ __forceinline__ void warp_hist_digit(const uint32_t* hist, uint32_t need, int lane, uint32_t& d,
+                                                uint32_t& below) {
+  uint32_t h[8];
+  uint32_t s = 0;
+#pragma unroll
+  for (int j = 0; j < 8; ++j) {
+    h[j] = hist[lane * 8 + j];
+    s += h[j];
+  }
+  uint32_t incl = s;
+#pragma unroll
+  for (int o = 1; o < 32; o <<= 1) {
+    uint32_t v = __shfl_up_sync(0xFFFFFFFFu, incl, o);
+    if (lane >= o) incl += v;
+  }
+  uint32_t excl = incl - s;
+  bool mine = (excl < need) && (need <= incl);
+  d = 0;
+  below = 0;
+  if (mine) {
+    uint32_t run = excl;
+    bool found = false;
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      if (!found && run + h[j] >= need) {
+        d = lane * 8 + j;
+        below = run;
+        found = true;
+      }
+      if (!found) run += h[j];
+    }
+  }
+  uint32_t owner = __ffs(__ballot_sync(0xFFFFFFFFu, mine)) - 1;
+  d = __shfl_sync(0xFFFFFFFFu, d, owner);
+  below = __shfl_sync(0xFFFFFFFFu, below, owner);
+}
+
 // Finds T = the R-th smallest of the c distinct keys in buf (1 <= R < c), compacts buf in place to the
 // R keys <= T and returns T.  hist: 256 u32 of shared memory private to the warp.
 __device__ __forceinline__ uint32_t warp_select_u32(uint32_t* buf, int c, int R, uint32_t* hist, int lane) {
@@ -243,38 +282,8 @@ __device__ __forceinline__ uint32_t warp_select_u32(uint32_t* buf, int c, int R,
       if ((k & mask) == prefix) atomicAdd(&hist[(k >> shift) & 255u], 1u);
     }
     __syncwarp();
-    uint32_t h[8];
-    uint32_t s = 0;
-#pragma unroll
-    for (int j = 0; j < 8; ++j) {
-      h[j] = hist[lane * 8 + j];
-      s += h[j];
-    }
-    uint32_t incl = s;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      uint32_t v = __shfl_up_sync(0xFFFFFFFFu, incl, o);
-      if (lane >= o) incl += v;
-    }
-    uint32_t excl = incl - s;
-    bool mine = (excl < need) && (need <= incl);
-    uint32_t d = 0, below = 0;
-    if (mine) {
-      uint32_t run = excl;
-      bool found = false;
-#pragma unroll
-      for (int j = 0; j < 8; ++j) {
-        if (!found && run + h[j] >= need) {
-          d = lane * 8 + j;
-          below = run;
-          found = true;
-        }
-        if (!found) run += h[j];
-      }
-    }
-    uint32_t owner = __ffs(__ballot_sync(0xFFFFFFFFu, mine)) - 1;
-    d = __shfl_sync(0xFFFFFFFFu, d, owner);
-    below = __shfl_sync(0xFFFFFFFFu, below, owner);
+    uint32_t d, below;
+    warp_hist_digit(hist, need, lane, d, below);
     need -= below;
     prefix |= d << shift;
     mask |= 0xFFu << shift;

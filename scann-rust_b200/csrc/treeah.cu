@@ -293,6 +293,46 @@ __global__ void tau_out_kernel(const uint32_t* __restrict__ qthr, size_t nq, flo
   tau[q] = k == 0xFFFFFFFFu ? __int_as_float(0x7F800000) : key_f32(k);
 }
 
+// Tensor-core mode, after the full scan of the class-A ranks: one warp per query lowers qthr[q] to the R-th smallest
+// approx distance over the union of its T class-A lists, when they hold at least R points.  Any R points of the probed
+// leaves prove a bound, and the R-th of the union is never above the R-th of one of its lists (the bound a single leaf
+// publishes).  Distances of different leaves have different quantisations, so the select runs on the f32 keys.
+__global__ void __launch_bounds__(256) union_bound_kernel(const uint2* __restrict__ cand,
+                                                          const uint32_t* __restrict__ cand_cnt, size_t nq, uint32_t L,
+                                                          uint32_t T, uint32_t R, uint32_t* __restrict__ qthr) {
+  __shared__ uint32_t hist_all[8][256];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  uint32_t* hist = hist_all[warp];
+  const size_t q = static_cast<size_t>(blockIdx.x) * 8 + warp;
+  if (q >= nq) return;
+  const size_t pair0 = q * L;
+  uint32_t total = 0;
+  for (uint32_t r = 0; r < T; ++r) total += cand_cnt[pair0 + r];
+  if (total < R) return;
+  uint32_t prefix = 0, mask = 0, need = R;
+  for (int shift = 24; shift >= 0; shift -= 8) {
+#pragma unroll
+    for (int k = 0; k < 8; ++k) hist[lane + 32 * k] = 0;
+    __syncwarp();
+    for (uint32_t r = 0; r < T; ++r) {
+      const uint32_t c = cand_cnt[pair0 + r];
+      const uint2* list = cand + (pair0 + r) * R;
+      for (uint32_t i = lane; i < c; i += 32) {
+        const uint32_t k = f32_key(__uint_as_float(list[i].x));
+        if ((k & mask) == prefix) atomicAdd(&hist[(k >> shift) & 255u], 1u);
+      }
+    }
+    __syncwarp();
+    uint32_t d, below;
+    warp_hist_digit(hist, need, lane, d, below);
+    need -= below;
+    prefix |= d << shift;
+    mask |= 0xFFu << shift;
+    __syncwarp();
+  }
+  if (lane == 0) qthr[q] = min(qthr[q], prefix);
+}
+
 // --------------------------------------------------------------------------- merge + exact reorder
 struct MergeArgs {
   const uint2* cand;
@@ -744,10 +784,18 @@ static scann_status treeah_phase1(scann_treeah* h, const float* dq, size_t nq, s
     // come back to them); otherwise a bounded probe of the closest leaf
     a.max_blocks = h->ck.use_tc ? 0 : probe_blocks();
     SCANN_TRY(launch_scan_g(h->ck.G, a, h->sms, s));
-    if (tau_out) tau_out_kernel<<<static_cast<unsigned>((nq + 255) / 256), 256, 0, s>>>(qthr, nq, tau_out);
+    h->prof_launches += 1;
+    if (h->ck.use_tc) {  // the class-A lists are final: their union bounds the tensor-core pass
+      union_bound_kernel<<<static_cast<unsigned>((nq + 7) / 8), 256, 0, s>>>(
+          cand, cand_cnt, nq, static_cast<uint32_t>(L), static_cast<uint32_t>(h->ck.T), static_cast<uint32_t>(R), qthr);
+      h->prof_launches += 1;
+    }
+    if (tau_out) {
+      tau_out_kernel<<<static_cast<unsigned>((nq + 255) / 256), 256, 0, s>>>(qthr, nq, tau_out);
+      h->prof_launches += 1;
+    }
     SCANN_CUDA(cudaGetLastError());
     h->span_end(s);
-    h->prof_launches += 2;
   }
   return SCANN_OK;
 }
