@@ -172,8 +172,24 @@ void scann_treeah_destroy(scann_treeah* h);
  * (restricts/mod.rs:17-31) as a bitmap over datapoint ids — bit i of byte i/8 (LSB first) set = datapoint i may be
  * returned; ids >= num_ids are not allowed.  Applies to every following search on the handle (plain and split) until
  * cleared with allow_by_id = NULL.  Filtered-out points are skipped inside the LUT16 scan exactly where the reference
- * skips them (before the per-leaf top-R), so a leaf contributes its R best ALLOWED points. */
+ * skips them (before the per-leaf top-R), so a leaf contributes its R best ALLOWED points.  Setting or clearing
+ * synchronises the device; filters that belong to one call (one per query, safe across threads) are
+ * scann_treeah_search_filtered's. */
 scann_status scann_treeah_set_filter(scann_treeah* h, const uint8_t* allow_by_id, size_t num_ids, int memspace);
+/* Per-query restrict filters of ONE call ← search_with_filter with the filter as an argument of the call: nothing is
+ * stored on the handle, so concurrent calls with different filters are safe, and queries with different filters share
+ * one batch.  allow = [num_filters][ceil(num_ids/8)] bytes, each row a bitmap in the convention of
+ * scann_treeah_set_filter (ids >= num_ids are not allowed); query q uses row filter_of_query[q].  allow and
+ * filter_of_query live in `memspace`, like the queries.  Everything else (limits, chunking, outputs, R == 0) is
+ * scann_treeah_search.  Errors: INVALID_ARGUMENT for num_filters == 0, a NULL allow / filter_of_query, or (SCANN_HOST)
+ * a row index >= num_filters; FAILED_PRECONDITION while a handle-wide filter is set or a split search is in flight.
+ * SCANN_DEVICE does not synchronise to check the rows: a query whose row is >= num_filters is allowed nothing and
+ * returns count 0. */
+scann_status scann_treeah_search_filtered(scann_treeah* h, const float* queries, size_t nq, size_t qdim, size_t L,
+                                          size_t R, size_t k, const uint8_t* allow, size_t num_filters, size_t num_ids,
+                                          const uint32_t* filter_of_query, uint32_t* ids, float* dists,
+                                          uint32_t* counts, uint32_t* cand_ids, float* cand_dists,
+                                          uint32_t* cand_counts, int memspace, void* stream);
 /* AsymmetricHasher::search vs ::search_with_reordering (src/hashes/hasher.rs:162-229) on one handle: enable = 0 makes the
  * following searches return the R best approximate (LUT16) distances without the exact re-score even though the handle
  * holds raw rows; enable = 1 (default) restores the re-score.  Handle-wide state, like the filter. */

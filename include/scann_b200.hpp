@@ -13,6 +13,7 @@
 // `Result<T>` carries {code, message} like `Result<T, ScannError>`; nothing throws across the ABI.
 #pragma once
 
+#include <algorithm>
 #include <cstdint>
 #include <limits>
 #include <string>
@@ -298,17 +299,50 @@ class TreeXHybridSearcher {
     if (b.ok() && !b.value.empty()) r.value = std::move(b.value[0]);
     return r;
   }
-  // search_with_filter(&[f32], k, Some(filter)) (:245-250): `allowed[i]` = RestrictFilter::is_allowed(i)
+  // search_with_filter(&[f32], k, Some(filter)) (:245-250): `allowed[i]` = RestrictFilter::is_allowed(i).  The filter
+  // belongs to this call only (scann_treeah_search_filtered), so concurrent calls with different filters are safe.
   Result<NNResultsVector> search_with_filter(const std::vector<float>& query, size_t k,
                                              const std::vector<bool>& allowed) const {
-    std::vector<uint8_t> bits((allowed.size() + 7) / 8, 0);
-    for (size_t i = 0; i < allowed.size(); ++i)
-      if (allowed[i]) bits[i >> 3] |= static_cast<uint8_t>(1u << (i & 7));
+    auto b = search_batched_with_filter({query}, k, {allowed}, {0u});
     Result<NNResultsVector> r;
-    r.error = make_error(scann_treeah_set_filter(h_, bits.data(), allowed.size(), SCANN_HOST));
-    if (!r.ok()) return r;
-    r = search(query, k);
-    scann_treeah_set_filter(h_, nullptr, 0, SCANN_HOST);
+    r.error = b.error;
+    if (b.ok() && !b.value.empty()) r.value = std::move(b.value[0]);
+    return r;
+  }
+  // One batch, one filter per query: query q may only return datapoints i with filters[filter_of_query[q]][i] true.
+  // filter_of_query[q] >= filters.size() -> InvalidArgument.  Filters shorter than the dataset do not allow the ids
+  // beyond their end.
+  Result<std::vector<NNResultsVector>> search_batched_with_filter(const std::vector<std::vector<float>>& queries,
+                                                                  size_t k,
+                                                                  const std::vector<std::vector<bool>>& filters,
+                                                                  const std::vector<uint32_t>& filter_of_query) const {
+    Result<std::vector<NNResultsVector>> r;
+    if (filter_of_query.size() != queries.size()) {
+      r.error = {ErrorCode::InvalidArgument, "filter_of_query must hold one filter index per query"};
+      return r;
+    }
+    if (queries.empty()) return r;
+    std::vector<float> flat;
+    size_t dim;
+    if (!detail::flatten(queries, &flat, &dim)) {
+      r.error = {ErrorCode::InvalidArgument, "Query dimensionality mismatch"};
+      return r;
+    }
+    size_t num_ids = 0;
+    for (const auto& f : filters) num_ids = std::max(num_ids, f.size());
+    const size_t row = (num_ids + 7) / 8;
+    std::vector<uint8_t> bits(std::max<size_t>(1, filters.size() * row), 0);  // never NULL: empty filters allow nothing
+    for (size_t f = 0; f < filters.size(); ++f)
+      for (size_t i = 0; i < filters[f].size(); ++i)
+        if (filters[f][i]) bits[f * row + (i >> 3)] |= static_cast<uint8_t>(1u << (i & 7));
+    const size_t nq = queries.size(), R = cfg_.pre_reorder_k(k);
+    std::vector<uint32_t> ids(nq * k), counts(nq);
+    std::vector<float> dists(nq * k);
+    r.error = make_error(scann_treeah_search_filtered(h_, flat.data(), nq, dim, cfg_.partitions_to_search, R, k,
+                                                      bits.data(), filters.size(), num_ids, filter_of_query.data(),
+                                                      ids.data(), dists.data(), counts.data(), nullptr, nullptr,
+                                                      nullptr, SCANN_HOST, nullptr));
+    if (r.ok()) r.value = detail::unflatten(ids, dists, counts, k);
     return r;
   }
   // build(dataset) (:131-209) on the GPU: k-means partition centres, residual PQ codebook (16 codes), exact assignment

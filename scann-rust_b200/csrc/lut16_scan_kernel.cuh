@@ -34,8 +34,8 @@ struct ScanArgs {
   const uint32_t* sorted_pairs;
   uint32_t* counters;  // [0] total items, [1] next item, [2] class-A items (closest-leaf pairs, scanned first)
   int end_idx;         // this launch stops at counters[end_idx]: 0 = every item, 2 = the class-A items only
-  const uint8_t* allow;  // restrict filter (search_with_filter): [total blocks][32] bytes, bit i of byte (block, lane) =
-                         // point lane*8+i of that block is allowed; nullptr = no filter
+  const uint8_t* allow;  // restrict filters (search_with_filter): [num_filters][total blocks * 32] bytes, bit i of byte
+                         // (row, block, lane) = point lane*8+i of that block is allowed by filter `row`; nullptr = none
   uint32_t sentinel;     // 255*S + 1: the integer score given to filtered-out points (above every real score)
   int max_blocks;      // > 0: probe launch — scan only the first max_blocks 256-point blocks of each leaf and publish
                        // the bound they prove (any R points give a valid bound); candidates are not written
@@ -44,6 +44,9 @@ struct ScanArgs {
   uint32_t* cand_cnt;  // [P]
   int dim, S, ds, SG, L, R, cap, pos_bits, use_residuals;
   AccMul mul;
+  size_t allow_stride;    // bytes per filter row of `allow`
+  const uint32_t* qfilt;  // [nq] filter row of every query of the chunk; nullptr = row 0 for every query
+  uint32_t num_filters;   // rows of `allow`: a query whose row is >= num_filters is allowed nothing
 };
 
 // largest integer score s with dequant(s) <= tau, as an exclusive key bound ((s+1) << pos_bits);
@@ -81,6 +84,7 @@ __global__ void __launch_bounds__(NW * 32, 16 / NW) lut16_scan_kernel(const Scan
   uint32_t* s_pair = s_cnt + G;                                // pair id (q * L + rank)
   uint32_t* s_tau = s_pair + G;                                // last tau key seen per query
   uint32_t* s_item = s_tau + G;
+  uint32_t* s_row = s_item + 1;                                // FILT: filter row per query (0xFFFFFFFF = none allowed)
 
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const uint32_t total_items = a.counters[a.end_idx];
@@ -116,6 +120,10 @@ __global__ void __launch_bounds__(NW * 32, 16 / NW) lut16_scan_kernel(const Scan
       qres[idx] = v;
     }
     if (tid < G) s_pair[tid] = tid < ng ? a.sorted_pairs[pbeg + tid] : 0xFFFFFFFFu;
+    if (FILT && tid < ng) {
+      const uint32_t row = a.qfilt ? a.qfilt[a.sorted_pairs[pbeg + tid] / static_cast<uint32_t>(a.L)] : 0u;
+      s_row[tid] = row < a.num_filters ? row : 0xFFFFFFFFu;
+    }
     __syncthreads();
 
     // (2) LUT16 build (warp g builds query g's table) and (3) the bound for this leaf
@@ -174,21 +182,24 @@ __global__ void __launch_bounds__(NW * 32, 16 / NW) lut16_scan_kernel(const Scan
         }
         if (FILT) {
           // RestrictFilter::is_allowed (tree_x_hybrid/mod.rs:327-332): filtered-out points never enter a top-R; here
-          // their score becomes the sentinel, which sorts after every real score and is dropped at the output
-          const uint32_t am = a.allow[(static_cast<size_t>(blk0) + b) * 32 + lane];
-          if (am != 0xFFu) {
+          // their score becomes the sentinel, which sorts after every real score and is dropped at the output.  Every
+          // query of the item reads the byte of its own filter row.
+          const size_t at = (static_cast<size_t>(blk0) + b) * 32 + lane;
+#pragma unroll
+          for (int g = 0; g < G; ++g) {
+            if (g >= ng) continue;
+            const uint32_t row = s_row[g];
+            const uint32_t am = row == 0xFFFFFFFFu ? 0u : a.allow[row * a.allow_stride + at];
+            if (am == 0xFFu) continue;
             const uint32_t lo = 0x0000FFFFu, hi = 0xFFFF0000u, sl = a.sentinel, sh = a.sentinel << 16;
             const uint32_t k_ea = ((am & 1u) ? lo : 0u) | ((am & 4u) ? hi : 0u), k_xa = ((am & 2u) ? lo : 0u) | ((am & 8u) ? hi : 0u);
             const uint32_t k_eb = ((am & 16u) ? lo : 0u) | ((am & 64u) ? hi : 0u), k_xb = ((am & 32u) ? lo : 0u) | ((am & 128u) ? hi : 0u);
             const uint32_t v_ea = ((am & 1u) ? 0u : sl) | ((am & 4u) ? 0u : sh), v_xa = ((am & 2u) ? 0u : sl) | ((am & 8u) ? 0u : sh);
             const uint32_t v_eb = ((am & 16u) ? 0u : sl) | ((am & 64u) ? 0u : sh), v_xb = ((am & 32u) ? 0u : sl) | ((am & 128u) ? 0u : sh);
-#pragma unroll
-            for (int g = 0; g < G; ++g) {
-              ps[g].ea = (ps[g].ea & k_ea) | v_ea;
-              ps[g].xa = (ps[g].xa & k_xa) | v_xa;
-              ps[g].eb = (ps[g].eb & k_eb) | v_eb;
-              ps[g].xb = (ps[g].xb & k_xb) | v_xb;
-            }
+            ps[g].ea = (ps[g].ea & k_ea) | v_ea;
+            ps[g].xa = (ps[g].xa & k_xa) | v_xa;
+            ps[g].eb = (ps[g].eb & k_eb) | v_eb;
+            ps[g].xb = (ps[g].xb & k_xb) | v_xb;
           }
         }
         const uint32_t pos0 = static_cast<uint32_t>(b) * kBlockPts + lane * 8;
@@ -289,9 +300,9 @@ __global__ void __launch_bounds__(NW * 32, 16 / NW) lut16_scan_kernel(const Scan
   }
 }
 
-inline size_t scan_smem_bytes(int G, int S4, int dim, int cap, int NW) {
+inline size_t scan_smem_bytes(int G, int S4, int dim, int cap, int NW, bool filt) {
   return static_cast<size_t>(G) * S4 * 16 + static_cast<size_t>((G * dim + 3) & ~3) * 4 +
-         static_cast<size_t>(G) * cap * 4 + NW * 256 * 4 + static_cast<size_t>(G) * 6 * 4 + 16;
+         static_cast<size_t>(G) * cap * 4 + NW * 256 * 4 + static_cast<size_t>(G) * (filt ? 7 : 6) * 4 + 16;
 }
 
 }  // namespace scann

@@ -488,13 +488,33 @@ struct TcsArgs {
   int L;
 };
 
-// A survivor (LUT row = (group, query column), accumulator, position in the leaf) -> the query's candidate list
-__device__ __forceinline__ void tcs_emit(const TcsArgs& a, uint32_t lut_row, uint32_t acc, uint32_t pos) {
+// restrict filters of the filtered instantiation (TcScanParams).  A kernel parameter of its own: widening TcsArgs alone
+// made ptxas spill in the unfiltered EG = 4 kernel.
+struct TcsFilter {
+  const uint8_t* allow;
+  size_t allow_stride;
+  const uint32_t* qfilt;
+  const uint32_t* blk_off;
+  uint32_t num_filters;
+};
+
+// A survivor (LUT row = (group, query column), accumulator, position in the leaf) -> the query's candidate list.
+// FILT: a point the query's filter row does not allow is dropped first, so filtered-out points cannot overflow a list.
+template <bool FILT>
+__device__ __forceinline__ void tcs_emit(const TcsArgs& a, const TcsFilter& f, uint32_t lut_row, uint32_t acc, uint32_t pos,
+                                         uint32_t leaf) {
   const uint4 m = __ldg(a.meta + lut_row);
   const uint32_t q = m.w / static_cast<uint32_t>(a.L), rank = m.w - q * static_cast<uint32_t>(a.L);
   if (m.w == kNoKey || q >= a.nq) {  // a padding row can never pass the threshold: protocol error, counted
     atomicAdd(a.err, 1u);
     return;
+  }
+  if (FILT) {  // bit pos % 8 of byte (block blk_off[leaf] + pos / 256, lane (pos % 256) / 8) of the query's row
+    const uint32_t row = f.qfilt ? __ldg(f.qfilt + q) : 0u;
+    if (row >= f.num_filters) return;
+    const size_t at = row * f.allow_stride + (static_cast<size_t>(__ldg(f.blk_off + leaf)) + (pos >> 8)) * 32 +
+                      ((pos & 255u) >> 3);
+    if (!((__ldg(f.allow + at) >> (pos & 7u)) & 1u)) return;
   }
   const uint32_t sum = acc - m.z;  // acc = sum + (BIG - smax)
   const float dist = lut16_dequant(sum, __uint_as_float(m.x), __uint_as_float(m.y));
@@ -504,11 +524,14 @@ __device__ __forceinline__ void tcs_emit(const TcsArgs& a, uint32_t lut_row, uin
         (static_cast<unsigned long long>(f32_key(dist)) << 32) | (static_cast<unsigned long long>(rank) << 22) | pos;
 }
 
-constexpr int kWqCap = 320;    // entries of one epilogue warp's survivor queue (uint4 {lut_row, acc, pos, -})
+constexpr int kWqCap = 320;    // entries of one epilogue warp's survivor queue (uint4 {lut_row, acc, pos, leaf (FILT)})
 constexpr int kWqStep = 256;   // most entries one filter step (32 lanes x 8 columns) can add
 
-template <int EG>  // expander groups: 2 (one per pipeline) or 4 (two per pipeline, alternate chunks)
-__global__ void __launch_bounds__(ts_threads(EG), 1) tc_scan_kernel(const __grid_constant__ CUtensorMap tmB, const TcsArgs a) {
+// EG: expander groups, 2 (one per pipeline) or 4 (two per pipeline, alternate chunks); FILT: restrict filters (a template
+// flag, so the unfiltered kernel carries none of it)
+template <int EG, bool FILT>
+__global__ void __launch_bounds__(ts_threads(EG), 1) tc_scan_kernel(const __grid_constant__ CUtensorMap tmB, const TcsArgs a,
+                                                                    const TcsFilter filt) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* sB = smem;  // [KA + 1] atom tiles
@@ -699,14 +722,16 @@ __global__ void __launch_bounds__(ts_threads(EG), 1) tc_scan_kernel(const __grid
       const uint32_t nw = *wq_cnt;
       for (uint32_t i = lane; i < nw; i += 32) {
         const uint4 e = wq[i];
-        tcs_emit(a, e.x, e.y, e.z);
+        tcs_emit<FILT>(a, filt, e.x, e.y, e.z, FILT ? e.w : 0u);
       }
       __syncwarp();
       if (lane == 0) *wq_cnt = 0;
       __syncwarp();
     };
     // threshold test of 32 accumulator columns starting at column c0 (nlive = 16 or 32 of them are real)
-    auto filter32 = [&](const uint32_t (&v)[32], uint32_t c0, uint32_t nlive, bool valid, uint32_t lut_row0, uint32_t p) {
+    // leaf: of the current item, carried in the queue entry for the restrict filter (FILT)
+    auto filter32 = [&](const uint32_t (&v)[32], uint32_t c0, uint32_t nlive, bool valid, uint32_t lut_row0, uint32_t p,
+                        uint32_t leaf) {
       uint32_t m8[4];
 #pragma unroll
       for (int g8 = 0; g8 < 4; ++g8) {
@@ -728,7 +753,7 @@ __global__ void __launch_bounds__(ts_threads(EG), 1) tc_scan_kernel(const __grid
               for (int j = 0; j < 8; ++j)
                 if (v[8 * g8 + j] <= kTsBig)
                   wq[atomicAdd(const_cast<uint32_t*>(wq_cnt), 1u)] =
-                      make_uint4(lut_row0 + c0 + 8 * g8 + j, v[8 * g8 + j], p, 0u);
+                      make_uint4(lut_row0 + c0 + 8 * g8 + j, v[8 * g8 + j], p, FILT ? leaf : 0u);
             }
             __syncwarp();
           }
@@ -760,14 +785,14 @@ __global__ void __launch_bounds__(ts_threads(EG), 1) tc_scan_kernel(const __grid
           __syncwarp();
           if (lane == 0) mbar_arrive(bar(kTEmpty + as));
         }
-        if (nmine > 0) filter32(v0, cb, min(32u, nmine), valid, lut_row0, p);
+        if (nmine > 0) filter32(v0, cb, min(32u, nmine), valid, lut_row0, p, I.w);
         if (nmine > 32) {
           tc_ld32_nowait(taddr + 32, v0);
           tc_wait_ld();
           tc_fence_before();
           __syncwarp();
           if (lane == 0) mbar_arrive(bar(kTEmpty + as));
-          filter32(v0, cb + 32, nmine - 32, valid, lut_row0, p);
+          filter32(v0, cb + 32, nmine - 32, valid, lut_row0, p, I.w);
         }
       }
     }
@@ -936,13 +961,21 @@ scann_status launch_tc_scan(const TcScanParams& p, Workspace& ws, TcScanOut* out
   a.KA = static_cast<int>(S / 8);
   a.bpp = static_cast<int>(S / 2);
   a.L = static_cast<int>(p.L);
+  TcsFilter tf;
+  tf.allow = p.allow;
+  tf.allow_stride = p.allow_stride;
+  tf.qfilt = p.qfilt;
+  tf.blk_off = p.blk_off;
+  tf.num_filters = p.num_filters;
+  const bool filt = p.allow != nullptr;
   // >= 120 KB keeps it at one CTA per SM for every S (a second resident CTA would block in tcgen05.alloc)
   const size_t smem = std::max<size_t>(120 * 1024, 1024 + static_cast<size_t>(a.KA + 1) * kTsAtom + 32 * 8 + 64 +
                                                        8 * kWqCap * 16 + 64);
   const char* eg_env = getenv("SCANN_TC_EXP");
   const bool eg4 = eg_env && eg_env[0] == '4';
-  if (eg4) SCANN_CUDA(cudaFuncSetAttribute(tc_scan_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
-  else SCANN_CUDA(cudaFuncSetAttribute(tc_scan_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+  auto kern = eg4 ? (filt ? tc_scan_kernel<4, true> : tc_scan_kernel<4, false>)
+                  : (filt ? tc_scan_kernel<2, true> : tc_scan_kernel<2, false>);
+  SCANN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
   static uint32_t* h_dbg = nullptr;
   if (dbg && h_dbg == nullptr) {
     uint32_t* d_dbg = nullptr;
@@ -952,8 +985,7 @@ scann_status launch_tc_scan(const TcScanParams& p, Workspace& ws, TcScanOut* out
       cudaMemcpyToSymbol(g_tcs_dbg, &d_dbg, sizeof(d_dbg));
     }
   }
-  if (eg4) tc_scan_kernel<4><<<p.sms, ts_threads(4), smem, s>>>(tmB, a);
-  else tc_scan_kernel<2><<<p.sms, ts_threads(2), smem, s>>>(tmB, a);
+  kern<<<p.sms, ts_threads(eg4 ? 4 : 2), smem, s>>>(tmB, a, tf);
   SCANN_CUDA(cudaGetLastError());
   if (dbg) {
     cudaError_t e = cudaStreamSynchronize(s);

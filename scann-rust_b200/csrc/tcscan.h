@@ -31,6 +31,13 @@ struct TcScanParams {
   const uint32_t* wl_cnt = nullptr;          // [K] pairs of rank >= T per leaf
   const uint32_t* wl_pair_start = nullptr;   // [K] first entry of the leaf's list in wl_sorted_pairs
   const uint32_t* wl_sorted_pairs = nullptr; // pair indices (q * L + rank), grouped by leaf
+  // optional restrict filters (ScanArgs::allow of lut16_scan_kernel.cuh): a survivor its query's filter row does not
+  // allow is dropped before it takes a list slot
+  const uint8_t* allow = nullptr;            // [num_filters][allow_stride] one byte per (256-point block, lane)
+  size_t allow_stride = 0;
+  const uint32_t* qfilt = nullptr;           // [nq] filter row of every query; nullptr = row 0
+  uint32_t num_filters = 0;                  // a query whose row is >= num_filters is allowed nothing
+  const uint32_t* blk_off = nullptr;         // [K + 1] first 256-point block of every leaf
 };
 
 struct TcScanOut {

@@ -258,8 +258,9 @@ __global__ void wl_items_kernel(const uint32_t* __restrict__ leaf_cnt, uint32_t 
   for (uint32_t g = 0; g * G < c; ++g) items[ib + g] = make_uint4(l, pb + g * G, min(static_cast<uint32_t>(G), c - g * G), 0u);
 }
 
-// restrict filter: id-indexed allow bitmap (bit i of byte i/8, LSB first) -> one byte per (block, lane) in scan order
-__global__ void build_allow_kernel(const uint8_t* __restrict__ allow_by_id, size_t num_ids,
+// restrict filters: F id-indexed allow bitmaps [F][row_bytes] (bit i of byte i/8, LSB first) -> [F][total] bytes, one
+// per (block, lane) in scan order.  One thread per (block, lane) reads its 8 ids once and writes its byte of every row.
+__global__ void build_allow_kernel(const uint8_t* __restrict__ allow_by_id, size_t row_bytes, size_t F, size_t num_ids,
                                    const uint32_t* __restrict__ blk_leaf, const uint32_t* __restrict__ blk_off,
                                    const uint64_t* __restrict__ pt_off, const uint32_t* __restrict__ ids,
                                    size_t total /* blocks * 32 */, uint8_t* __restrict__ out) {
@@ -268,14 +269,17 @@ __global__ void build_allow_kernel(const uint8_t* __restrict__ allow_by_id, size
   const uint32_t gb = static_cast<uint32_t>(t >> 5), lane = static_cast<uint32_t>(t & 31);
   const uint32_t leaf = blk_leaf[gb];
   const uint64_t p0 = pt_off[leaf] + static_cast<uint64_t>(gb - blk_off[leaf]) * kBlockPts + lane * 8, pend = pt_off[leaf + 1];
-  uint32_t m = 0;
-  for (int i = 0; i < 8; ++i) {
-    if (p0 + i < pend) {
-      const uint32_t id = ids[p0 + i];
-      if (id < num_ids && ((allow_by_id[id >> 3] >> (id & 7)) & 1u)) m |= 1u << i;
-    }
+  uint32_t id[8];
+#pragma unroll
+  for (int i = 0; i < 8; ++i) id[i] = p0 + i < pend ? ids[p0 + i] : 0xFFFFFFFFu;  // past the leaf: never allowed
+  for (size_t f = 0; f < F; ++f) {
+    const uint8_t* row = allow_by_id + f * row_bytes;
+    uint32_t m = 0;
+#pragma unroll
+    for (int i = 0; i < 8; ++i)
+      if (id[i] < num_ids && ((row[id[i] >> 3] >> (id[i] & 7)) & 1u)) m |= 1u << i;
+    out[f * total + t] = static_cast<uint8_t>(m);
   }
-  out[t] = static_cast<uint8_t>(m);
 }
 
 // qthr <-> caller-visible f32 bounds (scann_treeah_search_begin / _end)
@@ -579,7 +583,7 @@ namespace scann {
 template <int G, int MODE, int NW, bool FILT>
 static scann_status launch_scan_mode(ScanArgs a, int sms, cudaStream_t s) {
   a.cap = (NW * kBlockPts + 2 * a.R + 31) / 32 * 32;  // one tile of unfiltered points + 2R carried
-  size_t smem = scan_smem_bytes(G, a.SG * 4, a.dim, a.cap, NW);
+  size_t smem = scan_smem_bytes(G, a.SG * 4, a.dim, a.cap, NW, FILT);
   SCANN_REQUIRE(smem <= 227 * 1024, SCANN_RESOURCE_EXHAUSTED, "scan kernel needs %zu B of shared memory (R too large)",
                 smem);
   SCANN_CUDA(cudaFuncSetAttribute(lut16_scan_kernel<G, MODE, NW, FILT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -667,7 +671,7 @@ static size_t tc_qcap(size_t R) { return std::min<size_t>(16384, std::max<size_t
 // tensor-core scan for this chunk?  SCANN_SCAN_TC=0 never, =1 whenever the index supports it, default: when a leaf is
 // probed by enough queries of the batch to fill the 128-wide query tiles
 static bool treeah_use_tc(const scann_treeah* h, size_t nq, size_t L, size_t R) {
-  if (!h->tc_ok || h->filter_on || h->packed_rm.p == nullptr || L > 1024 || R < 1) return false;
+  if (!h->tc_ok || h->packed_rm.p == nullptr || L > 1024 || R < 1) return false;
   const char* e = getenv("SCANN_SCAN_TC");
   if (e && e[0] == '0') return false;
   if (e && e[0] == '1') return true;
@@ -684,10 +688,31 @@ static size_t tc_ranks(size_t L) {
   return std::min(v, L);
 }
 
+// The restrict filters of one chunk: F rows of one byte per (block, lane) in scan order (build_allow_kernel) and the row
+// of every query of the chunk.  allow == nullptr: no filter.
+struct ChunkFilter {
+  const uint8_t* allow = nullptr;
+  size_t stride = 0;               // bytes per row (blocks * 32)
+  uint32_t F = 0;                  // rows; a query whose row is >= F is allowed nothing
+  const uint32_t* qfilt = nullptr; // [nq of the chunk]; nullptr = row 0 for every query
+};
+
+// the handle-wide filter of scann_treeah_set_filter: one row shared by every query
+static ChunkFilter handle_filter(const scann_treeah* h) {
+  ChunkFilter f;
+  if (h->filter_on) {
+    f.allow = h->allow_blk.p;
+    f.stride = h->num_blocks * 32;
+    f.F = 1;
+  }
+  return f;
+}
+
 // Phase 1 of a chunk: partition -> worklist -> (two_phase: scan of the class-A items, i.e. every query's closest leaf
 // on this shard; tau_out receives the bounds they prove).  State for phase 2 stays in h->ck / the workspace.
 static scann_status treeah_phase1(scann_treeah* h, const float* dq, size_t nq, size_t L, size_t R, size_t k,
-                                  bool two_phase, float* tau_out, const uint32_t* tokens_in, cudaStream_t s) {
+                                  bool two_phase, float* tau_out, const uint32_t* tokens_in, const ChunkFilter& filt,
+                                  cudaStream_t s) {
   const size_t K = h->K, P = nq * L;
   // group size: how many queries share a leaf on average
   double avg = static_cast<double>(P) / static_cast<double>(std::min<size_t>(K, P));
@@ -746,7 +771,10 @@ static scann_status treeah_phase1(scann_treeah* h, const float* dq, size_t nq, s
   a.counters = counters;
   a.end_idx = 0;
   a.max_blocks = 0;
-  a.allow = h->filter_on ? h->allow_blk.p : nullptr;
+  a.allow = filt.allow;
+  a.allow_stride = filt.stride;
+  a.qfilt = filt.qfilt;
+  a.num_filters = filt.F;
   a.sentinel = 255u * static_cast<uint32_t>(h->S) + 1u;
   a.cand = cand;
   a.cand_cnt = cand_cnt;
@@ -846,6 +874,12 @@ static scann_status treeah_phase2(scann_treeah* h, bool two_phase, const float* 
     tp.wl_cnt = h->ck.leaf_cnt + K;
     tp.wl_pair_start = h->ck.pair_start + K;
     tp.wl_sorted_pairs = h->ck.sorted_pairs;
+    // restrict filters: survivors a query's filter does not allow are dropped before they take a list slot
+    tp.allow = a.allow;
+    tp.allow_stride = a.allow_stride;
+    tp.qfilt = a.qfilt;
+    tp.num_filters = a.num_filters;
+    tp.blk_off = h->blk_off.p;
     if (h->profiling) {
       scann_treeah::TcSpan sp{{nullptr, nullptr, nullptr}};
       bool ok = true;
@@ -915,17 +949,36 @@ static scann_status treeah_phase2(scann_treeah* h, bool two_phase, const float* 
 
 static scann_status treeah_search_chunk(scann_treeah* h, const float* dq, size_t nq, size_t L, size_t R, size_t k,
                                         uint32_t* d_ids, float* d_dists, uint32_t* d_counts, uint32_t* d_cand_ids,
-                                        float* d_cand_dists, uint32_t* d_cand_counts, cudaStream_t s) {
+                                        float* d_cand_dists, uint32_t* d_cand_counts, const ChunkFilter& filt,
+                                        cudaStream_t s) {
   // with the tensor-core scan the chunk runs as probe (bounds from every query's closest leaf) + bulk scan
   const bool tc = treeah_use_tc(h, nq, L, R);
-  SCANN_TRY(treeah_phase1(h, dq, nq, L, R, k, tc, nullptr, nullptr, s));
+  SCANN_TRY(treeah_phase1(h, dq, nq, L, R, k, tc, nullptr, nullptr, filt, s));
   return treeah_phase2(h, tc, nullptr, d_ids, d_dists, d_counts, d_cand_ids, d_cand_dists, d_cand_counts, s);
 }
 
-static size_t treeah_chunk_bytes(const scann_treeah* h, size_t nq, size_t L, size_t R, bool have_tokens = false) {
+// Per-call restrict filters of scann_treeah_search_filtered (the caller's arrays): F = num_filters rows of
+// ceil(num_ids / 8) bytes, the row of every query.
+struct FilterTable {
+  const uint8_t* allow;
+  size_t F, num_ids;
+  const uint32_t* filter_of_query;
+};
+
+// Workspace of a chunk, plus (ft != nullptr) what a filtered call takes once for the whole batch of nq_call queries:
+// the filters in block order and, on SCANN_HOST, the uploaded bitmaps and rows.
+static size_t treeah_chunk_bytes(const scann_treeah* h, size_t nq, size_t L, size_t R, bool have_tokens = false,
+                                 const FilterTable* ft = nullptr, size_t nq_call = 0, int memspace = SCANN_DEVICE) {
   size_t K = h->K, P = nq * L;
   size_t b = 0;
   auto add = [&](size_t bytes) { b += Workspace::padded(bytes); };
+  if (ft) {
+    add(ft->F * h->num_blocks * 32);
+    if (memspace == SCANN_HOST) {
+      add(ft->F * ((ft->num_ids + 7) / 8));
+      add(nq_call * 4);
+    }
+  }
   if (!have_tokens) add(h->part.scratch_bytes(nq));
   add(P * 4);
   add((2 * K + 4 * K * kWlPad) * 4);
@@ -942,6 +995,93 @@ static size_t treeah_chunk_bytes(const scann_treeah* h, size_t nq, size_t L, siz
   add(nq * 4);
   if (treeah_use_tc(h, nq, L, R)) b += tc_scan_workspace_bytes(nq, L, K, h->S, h->max_leaf, tc_qcap(R));
   return b + 4096;
+}
+
+// scann_treeah_search and scann_treeah_search_filtered (ft != nullptr: per-query filters of this call only)
+static scann_status treeah_search(scann_treeah* h, const float* queries, size_t nq, size_t qdim, size_t L, size_t R,
+                                  size_t k, uint32_t* ids, float* dists, uint32_t* counts, uint32_t* cand_ids,
+                                  float* cand_dists, uint32_t* cand_counts, int memspace, void* stream,
+                                  const FilterTable* ft) {
+  SCANN_REQUIRE(h != nullptr, SCANN_FAILED_PRECONDITION, "searcher not built");
+  if (nq == 0) return SCANN_OK;  // empty batch -> Ok(vec![])
+  SCANN_REQUIRE(queries && ids && dists && counts, SCANN_INVALID_ARGUMENT, "NULL buffer");
+  SCANN_REQUIRE(qdim == h->dim, SCANN_INVALID_ARGUMENT, "Query dimensionality mismatch");  // tree_x_hybrid/mod.rs:251-253
+  SCANN_REQUIRE(L >= 1 && L <= 1024, SCANN_INVALID_ARGUMENT, "partitions_to_search %zu outside 1..1024", L);
+  SCANN_REQUIRE(R <= 2048, SCANN_INVALID_ARGUMENT, "pre_reorder_k %zu > 2048 unsupported", R);
+  SCANN_REQUIRE(k >= 1, SCANN_INVALID_ARGUMENT, "k must be >= 1");
+  SCANN_REQUIRE((cand_ids == nullptr) == (cand_dists == nullptr), SCANN_INVALID_ARGUMENT,
+                "cand_ids and cand_dists go together");
+  if (ft) {
+    SCANN_REQUIRE(ft->F >= 1, SCANN_INVALID_ARGUMENT, "num_filters is 0");
+    SCANN_REQUIRE(ft->F <= 0xFFFFFFFFull, SCANN_INVALID_ARGUMENT, "num_filters %zu does not fit 32 bits", ft->F);
+    SCANN_REQUIRE(ft->allow && ft->filter_of_query, SCANN_INVALID_ARGUMENT, "NULL allow or filter_of_query");
+    if (memspace == SCANN_HOST)  // the device path cannot check without a synchronisation: there such a query gets nothing
+      for (size_t q = 0; q < nq; ++q)
+        SCANN_REQUIRE(ft->filter_of_query[q] < ft->F, SCANN_INVALID_ARGUMENT,
+                      "filter_of_query[%zu] = %u >= num_filters %zu", q, ft->filter_of_query[q], ft->F);
+  }
+  std::lock_guard<std::mutex> lock(h->mu);
+  SCANN_REQUIRE(!h->split_active, SCANN_FAILED_PRECONDITION, "a split search is in flight on this handle");
+  SCANN_REQUIRE(!(ft && h->filter_on), SCANN_FAILED_PRECONDITION,
+                "a handle-wide filter is set (scann_treeah_set_filter): clear it before a filtered search");
+  CallScope call(h->device, h->order, memspace, stream, h->stream);
+  const cudaStream_t s = call.s;
+  if (L > h->K) L = h->K;  // partition() returns min(L, K) tokens (tree_partitioner.rs:214)
+  const size_t Reff = R < 1 ? 1 : R;  // R == 0 (k*multiplier < 1) -> no candidates
+  // chunk the batch so that the candidate buffer stays <= 1 GiB and the centre-distance scratch <= 512 MiB
+  size_t chunk = nq;
+  chunk = std::min(chunk, std::max<size_t>(1, (size_t(1) << 30) / (L * Reff * 8)));
+  chunk = std::min(chunk, std::max<size_t>(1, (size_t(512) << 20) / (h->K * 4)));
+  const QueryOut outs[] = {{ids, k * 4}, {dists, k * 4}, {counts, 4},
+                           {cand_ids, R * 4}, {cand_dists, R * 4}, {cand_counts, 4}};
+  SCANN_TRY(h->ws.reserve(treeah_chunk_bytes(h, chunk, L, Reff, false, ft, nq, memspace) +
+                          staging_bytes(memspace, chunk, h->dim, outs)));
+  SCANN_CUDA(cudaMemsetAsync(h->stats.p, 0, 4 * sizeof(unsigned long long), s));
+  // the filters of the whole batch, once per call (below the staging of run_query_chunks): every chunk reads its slice
+  ChunkFilter filt = handle_filter(h);
+  if (ft) {
+    const size_t total = h->num_blocks * 32, row_bytes = (ft->num_ids + 7) / 8;
+    uint8_t* table = h->ws.take<uint8_t>(ft->F * total);
+    const uint8_t* src = ft->allow;
+    const uint32_t* qf = ft->filter_of_query;
+    if (memspace == SCANN_HOST) {
+      uint8_t* d_src = h->ws.take<uint8_t>(ft->F * row_bytes);
+      uint32_t* d_qf = h->ws.take<uint32_t>(nq);
+      if (ft->F * row_bytes > 0)
+        SCANN_CUDA(cudaMemcpyAsync(d_src, src, ft->F * row_bytes, cudaMemcpyHostToDevice, s));
+      SCANN_CUDA(cudaMemcpyAsync(d_qf, qf, nq * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
+      src = d_src;
+      qf = d_qf;
+    }
+    if (total > 0) {
+      build_allow_kernel<<<static_cast<unsigned>((total + 255) / 256), 256, 0, s>>>(
+          src, row_bytes, ft->F, ft->num_ids, h->blk_leaf.p, h->blk_off.p, h->pt_off.p, h->ids.p, total, table);
+      SCANN_CUDA(cudaGetLastError());
+    }
+    filt.allow = table;
+    filt.stride = total;
+    filt.F = static_cast<uint32_t>(ft->F);
+    filt.qfilt = qf;
+  }
+  return run_query_chunks(h->ws, memspace, s, queries, nq, h->dim, chunk, outs,
+                          [&](const float* dq, size_t q0, size_t nqc, void* const* o) -> scann_status {
+    uint32_t* d_ids = static_cast<uint32_t*>(o[0]);
+    float* d_dists = static_cast<float*>(o[1]);
+    uint32_t* d_counts = static_cast<uint32_t*>(o[2]);
+    uint32_t* d_cc = static_cast<uint32_t*>(o[5]);
+    if (R == 0) {
+      // (k as f32 * multiplier) as usize == 0: FastTopNeighbors(0) keeps nothing -> empty results
+      SCANN_CUDA(cudaMemsetAsync(d_ids, 0xFF, nqc * k * 4, s));
+      SCANN_CUDA(cudaMemsetAsync(d_dists, 0x7F, nqc * k * 4, s));  // 0x7F7F7F7F = 3.39e38: padding, never uninitialised
+      SCANN_CUDA(cudaMemsetAsync(d_counts, 0, nqc * 4, s));
+      if (d_cc) SCANN_CUDA(cudaMemsetAsync(d_cc, 0, nqc * 4, s));
+      return SCANN_OK;
+    }
+    ChunkFilter cf = filt;
+    if (cf.qfilt) cf.qfilt += q0;
+    return treeah_search_chunk(h, dq, nqc, L, R, k, d_ids, d_dists, d_counts, static_cast<uint32_t*>(o[3]),
+                               static_cast<float*>(o[4]), d_cc, cf, s);
+  });
 }
 
 }  // namespace scann
@@ -1094,47 +1234,18 @@ scann_status scann_treeah_create_ex(const float* centers, size_t K, size_t dim, 
 scann_status scann_treeah_search(scann_treeah* h, const float* queries, size_t nq, size_t qdim, size_t L, size_t R,
                                  size_t k, uint32_t* ids, float* dists, uint32_t* counts, uint32_t* cand_ids,
                                  float* cand_dists, uint32_t* cand_counts, int memspace, void* stream) {
-  using namespace scann;
-  SCANN_REQUIRE(h != nullptr, SCANN_FAILED_PRECONDITION, "searcher not built");
-  if (nq == 0) return SCANN_OK;  // empty batch -> Ok(vec![])
-  SCANN_REQUIRE(queries && ids && dists && counts, SCANN_INVALID_ARGUMENT, "NULL buffer");
-  SCANN_REQUIRE(qdim == h->dim, SCANN_INVALID_ARGUMENT, "Query dimensionality mismatch");  // tree_x_hybrid/mod.rs:251-253
-  SCANN_REQUIRE(L >= 1 && L <= 1024, SCANN_INVALID_ARGUMENT, "partitions_to_search %zu outside 1..1024", L);
-  SCANN_REQUIRE(R <= 2048, SCANN_INVALID_ARGUMENT, "pre_reorder_k %zu > 2048 unsupported", R);
-  SCANN_REQUIRE(k >= 1, SCANN_INVALID_ARGUMENT, "k must be >= 1");
-  SCANN_REQUIRE((cand_ids == nullptr) == (cand_dists == nullptr), SCANN_INVALID_ARGUMENT,
-                "cand_ids and cand_dists go together");
-  std::lock_guard<std::mutex> lock(h->mu);
-  SCANN_REQUIRE(!h->split_active, SCANN_FAILED_PRECONDITION, "a split search is in flight on this handle");
-  CallScope call(h->device, h->order, memspace, stream, h->stream);
-  const cudaStream_t s = call.s;
-  if (L > h->K) L = h->K;  // partition() returns min(L, K) tokens (tree_partitioner.rs:214)
-  const size_t Reff = R < 1 ? 1 : R;  // R == 0 (k*multiplier < 1) -> no candidates
-  // chunk the batch so that the candidate buffer stays <= 1 GiB and the centre-distance scratch <= 512 MiB
-  size_t chunk = nq;
-  chunk = std::min(chunk, std::max<size_t>(1, (size_t(1) << 30) / (L * Reff * 8)));
-  chunk = std::min(chunk, std::max<size_t>(1, (size_t(512) << 20) / (h->K * 4)));
-  const QueryOut outs[] = {{ids, k * 4}, {dists, k * 4}, {counts, 4},
-                           {cand_ids, R * 4}, {cand_dists, R * 4}, {cand_counts, 4}};
-  SCANN_TRY(h->ws.reserve(treeah_chunk_bytes(h, chunk, L, Reff) + staging_bytes(memspace, chunk, h->dim, outs)));
-  SCANN_CUDA(cudaMemsetAsync(h->stats.p, 0, 4 * sizeof(unsigned long long), s));
-  return run_query_chunks(h->ws, memspace, s, queries, nq, h->dim, chunk, outs,
-                          [&](const float* dq, size_t, size_t nqc, void* const* o) -> scann_status {
-    uint32_t* d_ids = static_cast<uint32_t*>(o[0]);
-    float* d_dists = static_cast<float*>(o[1]);
-    uint32_t* d_counts = static_cast<uint32_t*>(o[2]);
-    uint32_t* d_cc = static_cast<uint32_t*>(o[5]);
-    if (R == 0) {
-      // (k as f32 * multiplier) as usize == 0: FastTopNeighbors(0) keeps nothing -> empty results
-      SCANN_CUDA(cudaMemsetAsync(d_ids, 0xFF, nqc * k * 4, s));
-      SCANN_CUDA(cudaMemsetAsync(d_dists, 0x7F, nqc * k * 4, s));  // 0x7F7F7F7F = 3.39e38: padding, never uninitialised
-      SCANN_CUDA(cudaMemsetAsync(d_counts, 0, nqc * 4, s));
-      if (d_cc) SCANN_CUDA(cudaMemsetAsync(d_cc, 0, nqc * 4, s));
-      return SCANN_OK;
-    }
-    return treeah_search_chunk(h, dq, nqc, L, R, k, d_ids, d_dists, d_counts, static_cast<uint32_t*>(o[3]),
-                               static_cast<float*>(o[4]), d_cc, s);
-  });
+  return scann::treeah_search(h, queries, nq, qdim, L, R, k, ids, dists, counts, cand_ids, cand_dists, cand_counts,
+                              memspace, stream, nullptr);
+}
+
+scann_status scann_treeah_search_filtered(scann_treeah* h, const float* queries, size_t nq, size_t qdim, size_t L,
+                                          size_t R, size_t k, const uint8_t* allow, size_t num_filters, size_t num_ids,
+                                          const uint32_t* filter_of_query, uint32_t* ids, float* dists,
+                                          uint32_t* counts, uint32_t* cand_ids, float* cand_dists,
+                                          uint32_t* cand_counts, int memspace, void* stream) {
+  const scann::FilterTable ft{allow, num_filters, num_ids, filter_of_query};
+  return scann::treeah_search(h, queries, nq, qdim, L, R, k, ids, dists, counts, cand_ids, cand_dists, cand_counts,
+                              memspace, stream, &ft);
 }
 
 scann_status scann_treeah_last_scan_bytes(scann_treeah* h, uint64_t* bytes, uint64_t* pairs) {
@@ -1194,7 +1305,7 @@ scann_status scann_treeah_search_begin(scann_treeah* h, const float* queries, si
     CallScope call(h->device, h->order, SCANN_DEVICE, stream, h->stream);
     SCANN_TRY(h->ws.reserve(treeah_chunk_bytes(h, nq, L, R, tokens != nullptr)));
     cudaMemsetAsync(h->stats.p, 0, 4 * sizeof(unsigned long long), call.s);
-    SCANN_TRY(treeah_phase1(h, queries, nq, L, R, k, true, tau_out, tokens, call.s));
+    SCANN_TRY(treeah_phase1(h, queries, nq, L, R, k, true, tau_out, tokens, handle_filter(h), call.s));
   }
   // The handle is marked busy, not locked: every other entry point answers FAILED_PRECONDITION until _end (or _abort),
   // so nothing can be left locked by a caller that fails between the two calls.
@@ -1253,7 +1364,7 @@ scann_status scann_treeah_set_filter(scann_treeah* h, const uint8_t* allow_by_id
   SCANN_CUDA(cudaDeviceSynchronize());  // no search may be reading the previous filter
   if (h->allow_blk.n != total) SCANN_TRY(h->allow_blk.alloc(total));
   build_allow_kernel<<<static_cast<unsigned>((total + 255) / 256), 256, 0, h->stream>>>(
-      src, num_ids, h->blk_leaf.p, h->blk_off.p, h->pt_off.p, h->ids.p, total, h->allow_blk.p);
+      src, (num_ids + 7) / 8, 1, num_ids, h->blk_leaf.p, h->blk_off.p, h->pt_off.p, h->ids.p, total, h->allow_blk.p);
   SCANN_CUDA(cudaGetLastError());
   SCANN_CUDA(cudaStreamSynchronize(h->stream));
   h->filter_on = true;

@@ -483,6 +483,42 @@ class TreeXHybridConfig:
         return max(int(v), 0)
 
 
+def _filter_table(allowed, filter_of_query, b: "_Batch"):
+    """Packs per-query restrict filters for scann_treeah_search_filtered where the batch `b` lives → (bitmap pointer,
+    num_filters, num_ids, filter_of_query pointer, arrays to keep alive for the call)."""
+    nq = b.nq
+    if len(allowed.shape) not in (1, 2):
+        raise ScannError(capi.INVALID_ARGUMENT, "allowed must be [num_ids] or [num_filters, num_ids]")
+    one = len(allowed.shape) == 1
+    F = 1 if one else int(allowed.shape[0])
+    num_ids = int(allowed.shape[-1])
+    if filter_of_query is None:
+        if not one and F != nq:
+            raise ScannError(capi.INVALID_ARGUMENT,
+                             f"filter_of_query is needed: {F} filters for {nq} queries")
+        filter_of_query = np.zeros(nq, np.uint32) if one else np.arange(nq, dtype=np.uint32)
+    if int(filter_of_query.shape[0]) != nq or len(filter_of_query.shape) != 1:
+        raise ScannError(capi.INVALID_ARGUMENT, f"filter_of_query must hold one row index per query ({nq})")
+    if b.device:
+        torch = _torch()
+        dev = b.arr.device
+        m = (allowed if _is_torch(allowed) else torch.from_numpy(np.asarray(allowed))).to(dev).reshape(F, num_ids)
+        m = m.to(torch.bool)
+        pad = (-num_ids) % 8
+        if pad:
+            m = torch.nn.functional.pad(m, (0, pad))
+        shifts = torch.arange(8, device=dev, dtype=torch.uint8)
+        bits = (m.reshape(F, -1, 8).to(torch.uint8) << shifts).sum(-1, dtype=torch.uint8).contiguous()
+        fq = filter_of_query if _is_torch(filter_of_query) else torch.from_numpy(np.asarray(filter_of_query))
+        fq = fq.to(device=dev, dtype=torch.int64).to(torch.int32).contiguous()  # u32 bit patterns
+        return C.c_void_p(bits.data_ptr()), F, num_ids, C.c_void_p(fq.data_ptr()), (bits, fq)
+    m = allowed.cpu().numpy() if _is_torch(allowed) else np.asarray(allowed)
+    bits = np.ascontiguousarray(np.packbits(m.reshape(F, num_ids).astype(bool), axis=1, bitorder="little"))
+    fq = filter_of_query.cpu().numpy() if _is_torch(filter_of_query) else np.asarray(filter_of_query)
+    fq = np.ascontiguousarray(fq.astype(np.int64).astype(np.uint32))
+    return capi.np_ptr(bits), F, num_ids, capi.np_ptr(fq), (bits, fq)
+
+
 class TreeXHybridSearcher(_Handle):
     """TreeXHybridSearcher (src/tree_x_hybrid/mod.rs:93-380) with the LUT16 scan.
 
@@ -560,6 +596,10 @@ class TreeXHybridSearcher(_Handle):
 
     def search_batched(self, queries, k: int, partitions_to_search: Optional[int] = None,
                        pre_reorder_k: Optional[int] = None, want_candidates: bool = False):
+        return self._search(queries, k, partitions_to_search, pre_reorder_k, want_candidates)
+
+    def _search(self, queries, k, partitions_to_search, pre_reorder_k, want_candidates, allowed=None,
+                filter_of_query=None):
         if not (self._h and self._h.value):
             raise ScannError(capi.FAILED_PRECONDITION, "searcher not built")
         b = _Batch(queries, self.device)
@@ -581,9 +621,14 @@ class TreeXHybridSearcher(_Handle):
                 cc = np.zeros((b.nq,), np.uint32)
                 pci, pcd, pcc = capi.np_ptr(ci), capi.np_ptr(cd), capi.np_ptr(cc)
             cand = (ci, cd, cc)
-        if b.nq:
+        if b.nq and allowed is None:
             capi.check(capi.load().scann_treeah_search(self._h, b.ptr, b.nq, b.dim, L, R, k, pi, pd, pc, pci, pcd, pcc,
                                                        b.memspace, b.stream))
+        elif b.nq:
+            bits, F, num_ids, fq, keep = _filter_table(allowed, filter_of_query, b)
+            capi.check(capi.load().scann_treeah_search_filtered(self._h, b.ptr, b.nq, b.dim, L, R, k, bits, F, num_ids,
+                                                                fq, pi, pd, pc, pci, pcd, pcc, b.memspace, b.stream))
+            del keep
         if want_candidates:
             return ids, dists, counts, cand
         return ids, dists, counts
@@ -603,14 +648,21 @@ class TreeXHybridSearcher(_Handle):
         bits = np.packbits(m.astype(bool), bitorder="little")
         capi.check(capi.load().scann_treeah_set_filter(self._h, capi.np_ptr(bits), int(m.size), capi.HOST))
 
-    def search_with_filter(self, queries, k: int, allowed=None, **kw):
-        """search_with_filter (tree_x_hybrid/mod.rs:245-294): search_batched restricted to the allowed datapoints."""
-        self.set_filter(allowed)
-        try:
-            return self.search_batched(queries, k, **kw)
-        finally:
-            if allowed is not None:
-                self.set_filter(None)
+    def search_with_filter(self, queries, k: int, allowed=None, filter_of_query=None,
+                           partitions_to_search: Optional[int] = None, pre_reorder_k: Optional[int] = None,
+                           want_candidates: bool = False):
+        """search_with_filter (tree_x_hybrid/mod.rs:245-294): search_batched restricted to the allowed datapoints, with
+        filters that belong to this call only (scann_treeah_search_filtered; safe to call from several threads).
+
+        `allowed`: boolean mask over datapoint ids (True = may be returned), numpy or torch.  1-D [num_ids]: one filter
+        for the whole batch.  2-D [F, num_ids]: F filters, query q uses row filter_of_query[q] (length nq; may be
+        omitted when F == nq: query q uses row q).  None: the plain search.  CUDA queries take the device path and
+        the masks are packed on the device.  Refused while a handle-wide filter (set_filter) is set."""
+        if allowed is None:
+            if filter_of_query is not None:
+                raise ScannError(capi.INVALID_ARGUMENT, "filter_of_query without allowed")
+            return self.search_batched(queries, k, partitions_to_search, pre_reorder_k, want_candidates)
+        return self._search(queries, k, partitions_to_search, pre_reorder_k, want_candidates, allowed, filter_of_query)
 
     def partition_tokens(self, queries, partitions_to_search: Optional[int] = None):
         """The partition stage alone (scann_treeah_partition) for a slice of a batch: torch CUDA queries [m, dim] →
