@@ -300,6 +300,9 @@ __global__ void __launch_bounds__(NW * 32, 16 / NW) lut16_scan_kernel(const Scan
   }
 }
 
+// entries of a query's shared-memory candidate buffer: one tile of unfiltered points + 2R carried, in 32-entry rows
+inline int scan_list_cap(int R, int NW) { return (NW * kBlockPts + 2 * R + 31) / 32 * 32; }
+
 inline size_t scan_smem_bytes(int G, int S4, int dim, int cap, int NW, bool filt) {
   return static_cast<size_t>(G) * S4 * 16 + static_cast<size_t>((G * dim + 3) & ~3) * 4 +
          static_cast<size_t>(G) * cap * 4 + NW * 256 * 4 + static_cast<size_t>(G) * (filt ? 7 : 6) * 4 + 16;

@@ -580,11 +580,16 @@ struct scann_treeah {
 
 namespace scann {
 
+// 8 warps per scan CTA (2 CTAs/SM).  Measured on B200 at C3: 8 warps 35.6 ms, 4 warps 35.8 ms, 2 warps 44.7 ms
+// (profiles/r1_scan_kernel.md).
+constexpr int kScanWarps = 8;
+constexpr size_t kScanSmemMax = 227 * 1024;  // dynamic shared memory a CTA may opt in to
+
 template <int G, int MODE, int NW, bool FILT>
 static scann_status launch_scan_mode(ScanArgs a, int sms, cudaStream_t s) {
-  a.cap = (NW * kBlockPts + 2 * a.R + 31) / 32 * 32;  // one tile of unfiltered points + 2R carried
+  a.cap = scan_list_cap(a.R, NW);
   size_t smem = scan_smem_bytes(G, a.SG * 4, a.dim, a.cap, NW, FILT);
-  SCANN_REQUIRE(smem <= 227 * 1024, SCANN_RESOURCE_EXHAUSTED, "scan kernel needs %zu B of shared memory (R too large)",
+  SCANN_REQUIRE(smem <= kScanSmemMax, SCANN_RESOURCE_EXHAUSTED, "scan kernel needs %zu B of shared memory (R too large)",
                 smem);
   SCANN_CUDA(cudaFuncSetAttribute(lut16_scan_kernel<G, MODE, NW, FILT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   static_cast<int>(smem)));
@@ -596,12 +601,11 @@ static scann_status launch_scan_mode(ScanArgs a, int sms, cudaStream_t s) {
   return SCANN_OK;
 }
 
-// 8 warps per scan CTA (2 CTAs/SM).  Measured on B200 at C3: 8 warps 35.6 ms, 4 warps 35.8 ms, 2 warps 44.7 ms
-// (profiles/r1_scan_kernel.md).  The restrict filter is a template flag so the unfiltered kernel carries none of it.
+// The restrict filter is a template flag so the unfiltered kernel carries none of it.
 template <int G, int MODE>
 static scann_status launch_scan_nw(const ScanArgs& a, int sms, cudaStream_t s) {
-  if (a.allow != nullptr) return launch_scan_mode<G, MODE, 8, true>(a, sms, s);
-  return launch_scan_mode<G, MODE, 8, false>(a, sms, s);
+  if (a.allow != nullptr) return launch_scan_mode<G, MODE, kScanWarps, true>(a, sms, s);
+  return launch_scan_mode<G, MODE, kScanWarps, false>(a, sms, s);
 }
 
 template <int G>
@@ -717,6 +721,12 @@ static scann_status treeah_phase1(scann_treeah* h, const float* dq, size_t nq, s
   // group size: how many queries share a leaf on average
   double avg = static_cast<double>(P) / static_cast<double>(std::min<size_t>(K, P));
   int G = avg >= 6.0 ? 8 : (avg >= 3.0 ? 4 : (avg >= 1.5 ? 2 : 1));
+  // the scan CTA holds G queries' residuals, tables and candidate buffers: smaller groups where they do not fit (each
+  // pair's per-leaf top-R does not depend on which queries share its item, so results stay the same)
+  const int cap = scan_list_cap(static_cast<int>(R), kScanWarps);
+  while (G > 1 && scan_smem_bytes(G, static_cast<int>(h->SG) * 4, static_cast<int>(h->dim), cap, kScanWarps,
+                                  filt.allow != nullptr) > kScanSmemMax)
+    G /= 2;
   size_t max_items = P / G + 2 * std::min<size_t>(K, P) + 1;
 
   // centre-score scratch of the partition stage (not needed when the caller partitioned)
