@@ -190,6 +190,22 @@ scann_status scann_treeah_search_filtered(scann_treeah* h, const float* queries,
                                           const uint32_t* filter_of_query, uint32_t* ids, float* dists,
                                           uint32_t* counts, uint32_t* cand_ids, float* cand_dists,
                                           uint32_t* cand_counts, int memspace, void* stream);
+/* Per-query parameters of ONE call ← Searcher::search_batched_with_params (src/searcher.rs:164-169): query q searches
+ * L_of_query[q] partitions, keeps R_of_query[q] candidates before the reorder and returns k_of_query[q] neighbours, and
+ * queries with different parameters share one batch.  L, R and k are the batch maxima: they are the row strides of the
+ * outputs (ids/dists [nq*k], cand_ids/cand_dists [nq*R]), size the work, and obey the limits of scann_treeah_search.
+ * Each array is optional (NULL = every query uses the scalar) and lives in `memspace`, like the queries.  Row q is bit
+ * for bit what scann_treeah_search returns for query q alone with (L_q, R_q, k_q), padded beyond counts[q] up to k
+ * (0xFFFFFFFF / +inf) and beyond cand_counts[q] up to R; L_q > K clamps to K, and R_q == 0 gives the empty row of a
+ * search with R == 0 (its distances are padded with 0x7F7F7F7F).  Nothing is stored on the handle; the handle-wide filter and scann_treeah_set_reorder apply as for
+ * scann_treeah_search.  Errors: INVALID_ARGUMENT (SCANN_HOST) for an L_q outside 1..L, an R_q > R or a k_q outside
+ * 1..k; FAILED_PRECONDITION while a split search is in flight.  SCANN_DEVICE does not synchronise to check the values:
+ * a query with one out of range returns count 0 and cand_count 0, and the other queries are unaffected. */
+scann_status scann_treeah_search_with_params(scann_treeah* h, const float* queries, size_t nq, size_t qdim, size_t L,
+                                             size_t R, size_t k, const uint32_t* L_of_query, const uint32_t* R_of_query,
+                                             const uint32_t* k_of_query, uint32_t* ids, float* dists, uint32_t* counts,
+                                             uint32_t* cand_ids, float* cand_dists, uint32_t* cand_counts, int memspace,
+                                             void* stream);
 /* AsymmetricHasher::search vs ::search_with_reordering (src/hashes/hasher.rs:162-229) on one handle: enable = 0 makes the
  * following searches return the R best approximate (LUT16) distances without the exact re-score even though the handle
  * holds raw rows; enable = 1 (default) restores the re-score.  Handle-wide state, like the filter. */

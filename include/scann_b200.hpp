@@ -355,8 +355,10 @@ class TreeXHybridSearcher {
                                          kmeans_iters, seed, cfg_.use_residuals ? 1 : 0,
                                          static_cast<int>(cfg_.distance_measure), 1, device, SCANN_HOST, &h_));
   }
-  // Searcher::search_batched_with_params (src/searcher.rs:164-169): one SearchParameters per query; queries that share
-  // their parameters go to the GPU as one batch; queries.len() != params.len() -> InvalidArgument (searcher.rs:233-237)
+  // Searcher::search_batched_with_params (src/searcher.rs:164-169): one SearchParameters per query, the whole batch in
+  // one call (scann_treeah_search_with_params); k_q = num_neighbors (10 when unset), R_q = pre_reordering_num_neighbors
+  // (pre_reorder_k(k_q) when unset); queries.len() != params.len() -> InvalidArgument (searcher.rs:233-237).  An
+  // error aborts the whole batch (searcher.rs:192-208).
   Result<std::vector<NNResultsVector>> search_batched_with_params(const std::vector<std::vector<float>>& queries,
                                                                   const std::vector<SearchParameters>& params) const {
     Result<std::vector<NNResultsVector>> r;
@@ -364,29 +366,36 @@ class TreeXHybridSearcher {
       r.error = {ErrorCode::InvalidArgument, "Number of queries must match number of parameter sets"};
       return r;
     }
-    r.value.resize(queries.size());
-    std::vector<char> done(queries.size(), 0);
-    for (size_t i = 0; i < queries.size(); ++i) {
-      if (done[i]) continue;
-      std::vector<size_t> idx;
-      std::vector<std::vector<float>> sub;
-      for (size_t j = i; j < queries.size(); ++j)
-        if (!done[j] && params[j].num_neighbors == params[i].num_neighbors &&
-            params[j].pre_reordering_num_neighbors == params[i].pre_reordering_num_neighbors) {
-          idx.push_back(j);
-          sub.push_back(queries[j]);
-          done[j] = 1;
-        }
-      const size_t k = params[i].num_neighbors ? params[i].num_neighbors : 10;
-      auto b = search_impl(sub, k, params[i].pre_reordering_num_neighbors ? params[i].pre_reordering_num_neighbors
-                                                                           : cfg_.pre_reorder_k(k));
-      if (!b.ok()) {
-        r.error = b.error;  // the first Err aborts the whole batch (searcher.rs:192-208)
-        r.value.clear();
+    if (queries.empty()) return r;
+    std::vector<float> flat;
+    size_t dim;
+    if (!detail::flatten(queries, &flat, &dim)) {
+      r.error = {ErrorCode::InvalidArgument, "Query dimensionality mismatch"};
+      return r;
+    }
+    const size_t nq = queries.size();
+    std::vector<uint32_t> kq(nq), rq(nq);
+    size_t k = 0, R = 0;
+    for (size_t q = 0; q < nq; ++q) {
+      const size_t kv = params[q].num_neighbors ? params[q].num_neighbors : 10;
+      const size_t rv = params[q].pre_reordering_num_neighbors ? params[q].pre_reordering_num_neighbors
+                                                               : cfg_.pre_reorder_k(kv);
+      if (kv > 0xFFFFFFFFu || rv > 0xFFFFFFFFu) {
+        r.error = {ErrorCode::InvalidArgument, "num_neighbors or pre_reordering_num_neighbors does not fit 32 bits"};
         return r;
       }
-      for (size_t t = 0; t < idx.size(); ++t) r.value[idx[t]] = std::move(b.value[t]);
+      kq[q] = static_cast<uint32_t>(kv);
+      rq[q] = static_cast<uint32_t>(rv);
+      k = std::max(k, kv);
+      R = std::max(R, rv);
     }
+    std::vector<uint32_t> ids(nq * k), counts(nq);
+    std::vector<float> dists(nq * k);
+    r.error = make_error(scann_treeah_search_with_params(h_, flat.data(), nq, dim, cfg_.partitions_to_search, R, k,
+                                                         nullptr, rq.data(), kq.data(), ids.data(), dists.data(),
+                                                         counts.data(), nullptr, nullptr, nullptr, SCANN_HOST,
+                                                         nullptr));
+    if (r.ok()) r.value = detail::unflatten(ids, dists, counts, k);
     return r;
   }
   const TreeXHybridConfig& config() const { return cfg_; }

@@ -47,6 +47,9 @@ struct ScanArgs {
   size_t allow_stride;    // bytes per filter row of `allow`
   const uint32_t* qfilt;  // [nq] filter row of every query of the chunk; nullptr = row 0 for every query
   uint32_t num_filters;   // rows of `allow`: a query whose row is >= num_filters is allowed nothing
+  const uint32_t* qR;     // [nq] pre-reorder R of every query of the chunk (scann_treeah_search_with_params; a query
+                          // with R_q == 0 has no pairs), read where it is used so that the shared-memory layout stays
+                          // as it is; nullptr = R for every query.  The list stride and `cap` stay at R.
 };
 
 // largest integer score s with dequant(s) <= tau, as an exclusive key bound ((s+1) << pos_bits);
@@ -237,12 +240,13 @@ __global__ void __launch_bounds__(NW * 32, 16 / NW) lut16_scan_kernel(const Scan
       for (int g = warp; g < ng; g += NW) {
         int c = static_cast<int>(min(s_cnt[g], static_cast<uint32_t>(a.cap)));
         const uint32_t q = s_pair[g] / static_cast<uint32_t>(a.L);
+        const int R = a.qR ? static_cast<int>(__ldg(a.qR + q)) : a.R;
         uint32_t thr = s_thr[g];
-        if (c > a.R && (t == ntiles - 1 || c > 2 * a.R)) {
-          thr = warp_select_u32(buf + static_cast<size_t>(g) * a.cap, c, a.R, hist + warp * 256, lane);
-          c = a.R;
+        if (c > R && (t == ntiles - 1 || c > 2 * R)) {
+          thr = warp_select_u32(buf + static_cast<size_t>(g) * a.cap, c, R, hist + warp * 256, lane);
+          c = R;
           if (lane == 0) {
-            s_cnt[g] = static_cast<uint32_t>(a.R);
+            s_cnt[g] = static_cast<uint32_t>(R);
             // this leaf alone holds R points at or below dist(thr): publish the bound (unless the R-th entry is a
             // filtered-out point: then fewer than R allowed points were seen and nothing is proved)
             if (!FILT || (thr >> a.pos_bits) < a.sentinel) {
@@ -269,7 +273,8 @@ __global__ void __launch_bounds__(NW * 32, 16 / NW) lut16_scan_kernel(const Scan
     // (6) write this item's candidates: approx distance = sum*multiplier + bias*S (lut16_simd.rs:136-140)
     if (a.max_blocks > 0) continue;  // probe launch: only the bounds matter
     for (int g = warp; g < ng; g += NW) {
-      const int c = static_cast<int>(min(s_cnt[g], static_cast<uint32_t>(a.R)));
+      const uint32_t R = a.qR ? __ldg(a.qR + s_pair[g] / static_cast<uint32_t>(a.L)) : static_cast<uint32_t>(a.R);
+      const int c = static_cast<int>(min(s_cnt[g], R));
       const uint32_t pair = s_pair[g];
       const float mult = s_mult[g], biasS = s_bias[g];
       const uint32_t* bg = buf + static_cast<size_t>(g) * a.cap;

@@ -282,6 +282,28 @@ __global__ void build_allow_kernel(const uint8_t* __restrict__ allow_by_id, size
   }
 }
 
+// Per-query parameters of scann_treeah_search_with_params, after the partition stage of a chunk: a query keeps its
+// first min(L_q, L) tokens (its top-L_q leaves are a prefix of its top-L leaves) and every other rank gets no token, so
+// no later stage sees it (they all skip tokens >= K).  qR / qk receive each query's R and k; a query with a value out
+// of range (1 <= L_q <= L_call, R_q <= R, 1 <= k_q <= k) gets R = 0 and no token, hence count 0.  Lq / Rq / kq:
+// nullptr = the scalar.  One thread per (query, rank).
+__global__ void query_params_kernel(uint32_t* __restrict__ tokens, size_t P, uint32_t L, uint32_t L_call, uint32_t R,
+                                    uint32_t k, const uint32_t* __restrict__ Lq, const uint32_t* __restrict__ Rq,
+                                    const uint32_t* __restrict__ kq, uint32_t* __restrict__ qR,
+                                    uint32_t* __restrict__ qk) {
+  const size_t p = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (p >= P) return;
+  const uint32_t p32 = static_cast<uint32_t>(p);  // 32-bit: see wl_virtual_leaf
+  const uint32_t q = p32 / L, rank = p32 - q * L;
+  const uint32_t lq = Lq ? Lq[q] : L_call, rq = Rq ? Rq[q] : R, kv = kq ? kq[q] : k;
+  const bool ok = lq >= 1 && lq <= L_call && rq <= R && kv >= 1 && kv <= k;
+  if (!ok || rq == 0 || rank >= lq) tokens[p] = 0xFFFFFFFFu;
+  if (rank == 0) {
+    qR[q] = ok ? rq : 0u;
+    qk[q] = ok ? kv : 0u;
+  }
+}
+
 // qthr <-> caller-visible f32 bounds (scann_treeah_search_begin / _end)
 __global__ void tau_in_kernel(const float* __restrict__ tau, size_t nq, uint32_t* __restrict__ qthr) {
   size_t q = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -301,19 +323,23 @@ __global__ void tau_out_kernel(const uint32_t* __restrict__ qthr, size_t nq, flo
 // approx distance over the union of its T class-A lists, when they hold at least R points.  Any R points of the probed
 // leaves prove a bound, and the R-th of the union is never above the R-th of one of its lists (the bound a single leaf
 // publishes).  Distances of different leaves have different quantisations, so the select runs on the f32 keys.
+// qR: per-query R_q <= R (R is the list stride); nullptr = R for every query.
 __global__ void __launch_bounds__(256) union_bound_kernel(const uint2* __restrict__ cand,
                                                           const uint32_t* __restrict__ cand_cnt, size_t nq, uint32_t L,
-                                                          uint32_t T, uint32_t R, uint32_t* __restrict__ qthr) {
+                                                          uint32_t T, uint32_t R, const uint32_t* __restrict__ qR,
+                                                          uint32_t* __restrict__ qthr) {
   __shared__ uint32_t hist_all[8][256];
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   uint32_t* hist = hist_all[warp];
   const size_t q = static_cast<size_t>(blockIdx.x) * 8 + warp;
   if (q >= nq) return;
   const size_t pair0 = q * L;
+  const uint32_t Rq = qR ? qR[q] : R;
+  if (Rq == 0) return;  // no candidates, nothing to bound: a select of 0 points would publish a meaningless key
   uint32_t total = 0;
   for (uint32_t r = 0; r < T; ++r) total += cand_cnt[pair0 + r];
-  if (total < R) return;
-  uint32_t prefix = 0, mask = 0, need = R;
+  if (total < Rq) return;
+  uint32_t prefix = 0, mask = 0, need = Rq;
   for (int shift = 24; shift >= 0; shift -= 8) {
 #pragma unroll
     for (int k = 0; k < 8; ++k) hist[lane + 32 * k] = 0;
@@ -362,13 +388,18 @@ struct MergeArgs {
   const uint32_t* qcnt;
   const uint32_t* qflag;
   uint32_t qcap;
+  // scann_treeah_search_with_params (merge_reorder_kernel<.., PQ = true>): per-query R_q <= R and k_q <= k; R and k
+  // stay the row strides of the candidate lists and the outputs
+  const uint32_t* qR;
+  const uint32_t* qk;
 };
 
 constexpr int kMergeChunk = 2048;       // streaming chunk of the merge when a query can have L * R candidates
 constexpr int kMergeChunkSmall = 512;   // after a tensor-core scan a query has a few hundred: smaller CTAs, 16 per SM
 constexpr int kMergeThreads = 128;
 
-template <int NT, int CHUNK>
+// PQ: per-query R and k (a.qR / a.qk), a template flag so that the plain search's kernel carries none of it
+template <int NT, int CHUNK, bool PQ>
 __global__ void __launch_bounds__(NT) merge_reorder_kernel(const MergeArgs a) {
   extern __shared__ __align__(16) uint8_t sm[];
   const int p2 = next_pow2(a.R < 1 ? 1 : a.R);
@@ -423,7 +454,8 @@ __global__ void __launch_bounds__(NT) merge_reorder_kernel(const MergeArgs a) {
     uint2 c = cq[static_cast<size_t>(lo) * a.R + (i - prefix[lo])];
     return (static_cast<uint64_t>(f32_key(__uint_as_float(c.x))) << 32) | (static_cast<uint64_t>(lo) << 22) | c.y;
   };
-  const int m = block_topr_sorted<NT, CHUNK>(gen, total + nlist, a.R, buf, out, hist);
+  const int Rq = PQ ? static_cast<int>(a.qR[q]) : a.R;
+  const int m = block_topr_sorted<NT, CHUNK>(gen, total + nlist, Rq, buf, out, hist);
 
   // the R approximate candidates, in (approx distance, leaf rank, position) order
   for (int j = tid; j < p2; j += NT) {
@@ -472,7 +504,10 @@ __global__ void __launch_bounds__(NT) merge_reorder_kernel(const MergeArgs a) {
       fin[j] = j < m ? ((out[j] & 0xFFFFFFFF00000000ull) | static_cast<uint32_t>(j)) : ~0ull;
     __syncthreads();
   }
-  int kk = a.k < m ? a.k : m;
+  const int kq = PQ ? static_cast<int>(a.qk[q]) : a.k;
+  // a query with R_q == 0 gets the row of a search with R == 0, whose distances are padded with 0x7F7F7F7F
+  const float pad = PQ && Rq == 0 ? __int_as_float(0x7F7F7F7F) : __int_as_float(0x7F800000);
+  int kk = kq < m ? kq : m;
   while (kk > 0 && fin[kk - 1] == ~0ull) --kk;  // candidates whose raw row does not exist were dropped (sorted last)
   for (int j = tid; j < a.k; j += NT) {
     if (j < kk) {
@@ -481,7 +516,7 @@ __global__ void __launch_bounds__(NT) merge_reorder_kernel(const MergeArgs a) {
       a.out_dists[q * a.k + j] = key_f32(static_cast<uint32_t>(key >> 32));
     } else {
       a.out_ids[q * a.k + j] = 0xFFFFFFFFu;
-      a.out_dists[q * a.k + j] = __int_as_float(0x7F800000);
+      a.out_dists[q * a.k + j] = pad;
     }
   }
   if (tid == 0) a.out_counts[q] = static_cast<uint32_t>(kk);
@@ -535,6 +570,7 @@ struct scann_treeah {
     uint4* items = nullptr;
     bool use_tc = false;
     int T = 1;  // ranks in class A of the worklist
+    const uint32_t *qR = nullptr, *qk = nullptr;  // per-query R / k (scann_treeah_search_with_params), else nullptr
     scann::ScanArgs a;
   } ck;
   bool split_active = false;  // between scann_treeah_search_begin and _end / _abort: other entry points are refused
@@ -712,11 +748,19 @@ static ChunkFilter handle_filter(const scann_treeah* h) {
   return f;
 }
 
+// The per-query L / R / k of one chunk (scann_treeah_search_with_params: device arrays, nullptr = the scalar) and the
+// caller's L, the bound of every L_q (the L of the search is clamped to K).
+struct ChunkParams {
+  const uint32_t *L = nullptr, *R = nullptr, *k = nullptr;
+  size_t L_call = 0;
+  bool any() const { return L || R || k; }
+};
+
 // Phase 1 of a chunk: partition -> worklist -> (two_phase: scan of the class-A items, i.e. every query's closest leaf
 // on this shard; tau_out receives the bounds they prove).  State for phase 2 stays in h->ck / the workspace.
 static scann_status treeah_phase1(scann_treeah* h, const float* dq, size_t nq, size_t L, size_t R, size_t k,
                                   bool two_phase, float* tau_out, const uint32_t* tokens_in, const ChunkFilter& filt,
-                                  cudaStream_t s) {
+                                  const ChunkParams& cp, cudaStream_t s) {
   const size_t K = h->K, P = nq * L;
   // group size: how many queries share a leaf on average
   double avg = static_cast<double>(P) / static_cast<double>(std::min<size_t>(K, P));
@@ -746,10 +790,19 @@ static scann_status treeah_phase1(scann_treeah* h, const float* dq, size_t nq, s
   uint2* cand = h->ws.take<uint2>(P * R);
   uint32_t* cand_cnt = h->ws.take<uint32_t>(P);
   uint32_t* qthr = h->ws.take<uint32_t>(nq);
+  uint32_t* qR = cp.any() ? h->ws.take<uint32_t>(nq) : nullptr;
+  uint32_t* qk = cp.any() ? h->ws.take<uint32_t>(nq) : nullptr;
 
   // 1. partition (K == 1 still goes through it: one centre, token 0)
   h->span_begin(0, s);
   if (!tokens_in) SCANN_TRY(h->part.select(dq, nq, L, tokens, nullptr, scratch, s));
+  if (cp.any()) {  // per-query parameters: the ranks a query does not search leave the batch here
+    query_params_kernel<<<static_cast<unsigned>((P + 255) / 256), 256, 0, s>>>(
+        tokens, P, static_cast<uint32_t>(L), static_cast<uint32_t>(cp.L_call), static_cast<uint32_t>(R),
+        static_cast<uint32_t>(k), cp.L, cp.R, cp.k, qR, qk);
+    SCANN_CUDA(cudaGetLastError());
+    h->prof_launches += 1;
+  }
   h->span_end(s);
   // 2. worklist
   h->span_begin(1, s);
@@ -785,6 +838,7 @@ static scann_status treeah_phase1(scann_treeah* h, const float* dq, size_t nq, s
   a.allow_stride = filt.stride;
   a.qfilt = filt.qfilt;
   a.num_filters = filt.F;
+  a.qR = qR;
   a.sentinel = 255u * static_cast<uint32_t>(h->S) + 1u;
   a.cand = cand;
   a.cand_cnt = cand_cnt;
@@ -812,6 +866,8 @@ static scann_status treeah_phase1(scann_treeah* h, const float* dq, size_t nq, s
   h->ck.cand = cand;
   h->ck.cand_cnt = cand_cnt;
   h->ck.qthr = qthr;
+  h->ck.qR = qR;
+  h->ck.qk = qk;
   h->prof_launches += (tokens_in ? 0 : h->part.launches()) + 7;  // partition + 7 worklist kernels
   if (two_phase) {
     // 3a. probe of the class-A items: the first probe_blocks() blocks of every query's closest leaf prove a bound in
@@ -825,7 +881,8 @@ static scann_status treeah_phase1(scann_treeah* h, const float* dq, size_t nq, s
     h->prof_launches += 1;
     if (h->ck.use_tc) {  // the class-A lists are final: their union bounds the tensor-core pass
       union_bound_kernel<<<static_cast<unsigned>((nq + 7) / 8), 256, 0, s>>>(
-          cand, cand_cnt, nq, static_cast<uint32_t>(L), static_cast<uint32_t>(h->ck.T), static_cast<uint32_t>(R), qthr);
+          cand, cand_cnt, nq, static_cast<uint32_t>(L), static_cast<uint32_t>(h->ck.T), static_cast<uint32_t>(R), qR,
+          qthr);
       h->prof_launches += 1;
     }
     if (tau_out) {
@@ -914,6 +971,8 @@ static scann_status treeah_phase2(scann_treeah* h, bool two_phase, const float* 
   m.qcnt = tco.qcnt;
   m.qflag = tco.qflag;
   m.qcap = h->ck.use_tc ? static_cast<uint32_t>(tc_qcap(R)) : 0u;
+  m.qR = h->ck.qR;
+  m.qk = h->ck.qk;
   m.cand = h->ck.cand;
   m.cand_cnt = h->ck.cand_cnt;
   m.tokens = h->ck.tokens;
@@ -942,15 +1001,13 @@ static scann_status treeah_phase2(scann_treeah* h, bool two_phase, const float* 
   const bool small = h->ck.use_tc;
   size_t msm = merge_smem_bytes(static_cast<int>(R), static_cast<int>(L), static_cast<int>(h->dim),
                                 small ? kMergeChunkSmall : kMergeChunk);
-  if (small) {
-    SCANN_CUDA(cudaFuncSetAttribute(merge_reorder_kernel<kMergeThreads, kMergeChunkSmall>,
-                                    cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(msm)));
-    merge_reorder_kernel<kMergeThreads, kMergeChunkSmall><<<static_cast<unsigned>(nq), kMergeThreads, msm, s>>>(m);
-  } else {
-    SCANN_CUDA(cudaFuncSetAttribute(merge_reorder_kernel<kMergeThreads, kMergeChunk>,
-                                    cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(msm)));
-    merge_reorder_kernel<kMergeThreads, kMergeChunk><<<static_cast<unsigned>(nq), kMergeThreads, msm, s>>>(m);
-  }
+  const bool pq = m.qR != nullptr;
+  auto kern = small ? (pq ? merge_reorder_kernel<kMergeThreads, kMergeChunkSmall, true>
+                          : merge_reorder_kernel<kMergeThreads, kMergeChunkSmall, false>)
+                    : (pq ? merge_reorder_kernel<kMergeThreads, kMergeChunk, true>
+                          : merge_reorder_kernel<kMergeThreads, kMergeChunk, false>);
+  SCANN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(msm)));
+  kern<<<static_cast<unsigned>(nq), kMergeThreads, msm, s>>>(m);
   SCANN_CUDA(cudaGetLastError());
   h->span_end(s);
   h->prof_launches += two_phase && tau_in ? 3 : 2;  // (tau_in) + lut16_scan + merge_reorder
@@ -960,10 +1017,10 @@ static scann_status treeah_phase2(scann_treeah* h, bool two_phase, const float* 
 static scann_status treeah_search_chunk(scann_treeah* h, const float* dq, size_t nq, size_t L, size_t R, size_t k,
                                         uint32_t* d_ids, float* d_dists, uint32_t* d_counts, uint32_t* d_cand_ids,
                                         float* d_cand_dists, uint32_t* d_cand_counts, const ChunkFilter& filt,
-                                        cudaStream_t s) {
+                                        const ChunkParams& cp, cudaStream_t s) {
   // with the tensor-core scan the chunk runs as probe (bounds from every query's closest leaf) + bulk scan
   const bool tc = treeah_use_tc(h, nq, L, R);
-  SCANN_TRY(treeah_phase1(h, dq, nq, L, R, k, tc, nullptr, nullptr, filt, s));
+  SCANN_TRY(treeah_phase1(h, dq, nq, L, R, k, tc, nullptr, nullptr, filt, cp, s));
   return treeah_phase2(h, tc, nullptr, d_ids, d_dists, d_counts, d_cand_ids, d_cand_dists, d_cand_counts, s);
 }
 
@@ -975,10 +1032,17 @@ struct FilterTable {
   const uint32_t* filter_of_query;
 };
 
+// Per-query L / R / k of scann_treeah_search_with_params (the caller's arrays; nullptr = the scalar for every query).
+struct ParamTable {
+  const uint32_t *L, *R, *k;
+};
+
 // Workspace of a chunk, plus (ft != nullptr) what a filtered call takes once for the whole batch of nq_call queries:
-// the filters in block order and, on SCANN_HOST, the uploaded bitmaps and rows.
+// the filters in block order and, on SCANN_HOST, the uploaded bitmaps and rows; (pt != nullptr) the per-query R / k
+// of a chunk and, on SCANN_HOST, the uploaded parameter arrays.
 static size_t treeah_chunk_bytes(const scann_treeah* h, size_t nq, size_t L, size_t R, bool have_tokens = false,
-                                 const FilterTable* ft = nullptr, size_t nq_call = 0, int memspace = SCANN_DEVICE) {
+                                 const FilterTable* ft = nullptr, size_t nq_call = 0, int memspace = SCANN_DEVICE,
+                                 const ParamTable* pt = nullptr) {
   size_t K = h->K, P = nq * L;
   size_t b = 0;
   auto add = [&](size_t bytes) { b += Workspace::padded(bytes); };
@@ -988,6 +1052,13 @@ static size_t treeah_chunk_bytes(const scann_treeah* h, size_t nq, size_t L, siz
       add(ft->F * ((ft->num_ids + 7) / 8));
       add(nq_call * 4);
     }
+  }
+  if (pt) {
+    add(nq * 4);
+    add(nq * 4);
+    if (memspace == SCANN_HOST)
+      for (const uint32_t* a : {pt->L, pt->R, pt->k})
+        if (a) add(nq_call * 4);
   }
   if (!have_tokens) add(h->part.scratch_bytes(nq));
   add(P * 4);
@@ -1007,11 +1078,12 @@ static size_t treeah_chunk_bytes(const scann_treeah* h, size_t nq, size_t L, siz
   return b + 4096;
 }
 
-// scann_treeah_search and scann_treeah_search_filtered (ft != nullptr: per-query filters of this call only)
+// scann_treeah_search, scann_treeah_search_filtered (ft != nullptr: per-query filters of this call only) and
+// scann_treeah_search_with_params (pt != nullptr: per-query L / R / k of this call only)
 static scann_status treeah_search(scann_treeah* h, const float* queries, size_t nq, size_t qdim, size_t L, size_t R,
                                   size_t k, uint32_t* ids, float* dists, uint32_t* counts, uint32_t* cand_ids,
                                   float* cand_dists, uint32_t* cand_counts, int memspace, void* stream,
-                                  const FilterTable* ft) {
+                                  const FilterTable* ft, const ParamTable* pt = nullptr) {
   SCANN_REQUIRE(h != nullptr, SCANN_FAILED_PRECONDITION, "searcher not built");
   if (nq == 0) return SCANN_OK;  // empty batch -> Ok(vec![])
   SCANN_REQUIRE(queries && ids && dists && counts, SCANN_INVALID_ARGUMENT, "NULL buffer");
@@ -1030,12 +1102,23 @@ static scann_status treeah_search(scann_treeah* h, const float* queries, size_t 
         SCANN_REQUIRE(ft->filter_of_query[q] < ft->F, SCANN_INVALID_ARGUMENT,
                       "filter_of_query[%zu] = %u >= num_filters %zu", q, ft->filter_of_query[q], ft->F);
   }
+  // the device path cannot check without a synchronisation: there such a query gets nothing (query_params_kernel)
+  if (pt && memspace == SCANN_HOST) {
+    for (size_t q = 0; q < nq; ++q) {
+      SCANN_REQUIRE(!pt->L || (pt->L[q] >= 1 && pt->L[q] <= L), SCANN_INVALID_ARGUMENT,
+                    "L_of_query[%zu] = %u outside 1..%zu", q, pt->L[q], L);
+      SCANN_REQUIRE(!pt->R || pt->R[q] <= R, SCANN_INVALID_ARGUMENT, "R_of_query[%zu] = %u > R %zu", q, pt->R[q], R);
+      SCANN_REQUIRE(!pt->k || (pt->k[q] >= 1 && pt->k[q] <= k), SCANN_INVALID_ARGUMENT,
+                    "k_of_query[%zu] = %u outside 1..%zu", q, pt->k[q], k);
+    }
+  }
   std::lock_guard<std::mutex> lock(h->mu);
   SCANN_REQUIRE(!h->split_active, SCANN_FAILED_PRECONDITION, "a split search is in flight on this handle");
   SCANN_REQUIRE(!(ft && h->filter_on), SCANN_FAILED_PRECONDITION,
                 "a handle-wide filter is set (scann_treeah_set_filter): clear it before a filtered search");
   CallScope call(h->device, h->order, memspace, stream, h->stream);
   const cudaStream_t s = call.s;
+  const size_t L_call = L;
   if (L > h->K) L = h->K;  // partition() returns min(L, K) tokens (tree_partitioner.rs:214)
   const size_t Reff = R < 1 ? 1 : R;  // R == 0 (k*multiplier < 1) -> no candidates
   // chunk the batch so that the candidate buffer stays <= 1 GiB and the centre-distance scratch <= 512 MiB
@@ -1044,7 +1127,7 @@ static scann_status treeah_search(scann_treeah* h, const float* queries, size_t 
   chunk = std::min(chunk, std::max<size_t>(1, (size_t(512) << 20) / (h->K * 4)));
   const QueryOut outs[] = {{ids, k * 4}, {dists, k * 4}, {counts, 4},
                            {cand_ids, R * 4}, {cand_dists, R * 4}, {cand_counts, 4}};
-  SCANN_TRY(h->ws.reserve(treeah_chunk_bytes(h, chunk, L, Reff, false, ft, nq, memspace) +
+  SCANN_TRY(h->ws.reserve(treeah_chunk_bytes(h, chunk, L, Reff, false, ft, nq, memspace, pt) +
                           staging_bytes(memspace, chunk, h->dim, outs)));
   SCANN_CUDA(cudaMemsetAsync(h->stats.p, 0, 4 * sizeof(unsigned long long), s));
   // the filters of the whole batch, once per call (below the staging of run_query_chunks): every chunk reads its slice
@@ -1073,6 +1156,18 @@ static scann_status treeah_search(scann_treeah* h, const float* queries, size_t 
     filt.F = static_cast<uint32_t>(ft->F);
     filt.qfilt = qf;
   }
+  // the per-query parameters of the whole batch, uploaded once per call on SCANN_HOST: every chunk reads its slice
+  ParamTable dp{nullptr, nullptr, nullptr};
+  if (pt) {
+    dp = *pt;
+    if (memspace == SCANN_HOST)
+      for (const uint32_t** a : {&dp.L, &dp.R, &dp.k})
+        if (*a) {
+          uint32_t* d = h->ws.take<uint32_t>(nq);
+          SCANN_CUDA(cudaMemcpyAsync(d, *a, nq * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
+          *a = d;
+        }
+  }
   return run_query_chunks(h->ws, memspace, s, queries, nq, h->dim, chunk, outs,
                           [&](const float* dq, size_t q0, size_t nqc, void* const* o) -> scann_status {
     uint32_t* d_ids = static_cast<uint32_t*>(o[0]);
@@ -1089,8 +1184,15 @@ static scann_status treeah_search(scann_treeah* h, const float* queries, size_t 
     }
     ChunkFilter cf = filt;
     if (cf.qfilt) cf.qfilt += q0;
+    ChunkParams cp;
+    if (pt) {
+      cp.L = dp.L ? dp.L + q0 : nullptr;
+      cp.R = dp.R ? dp.R + q0 : nullptr;
+      cp.k = dp.k ? dp.k + q0 : nullptr;
+      cp.L_call = L_call;
+    }
     return treeah_search_chunk(h, dq, nqc, L, R, k, d_ids, d_dists, d_counts, static_cast<uint32_t*>(o[3]),
-                               static_cast<float*>(o[4]), d_cc, cf, s);
+                               static_cast<float*>(o[4]), d_cc, cf, cp, s);
   });
 }
 
@@ -1258,6 +1360,16 @@ scann_status scann_treeah_search_filtered(scann_treeah* h, const float* queries,
                               memspace, stream, &ft);
 }
 
+scann_status scann_treeah_search_with_params(scann_treeah* h, const float* queries, size_t nq, size_t qdim, size_t L,
+                                             size_t R, size_t k, const uint32_t* L_of_query, const uint32_t* R_of_query,
+                                             const uint32_t* k_of_query, uint32_t* ids, float* dists, uint32_t* counts,
+                                             uint32_t* cand_ids, float* cand_dists, uint32_t* cand_counts, int memspace,
+                                             void* stream) {
+  const scann::ParamTable pt{L_of_query, R_of_query, k_of_query};
+  return scann::treeah_search(h, queries, nq, qdim, L, R, k, ids, dists, counts, cand_ids, cand_dists, cand_counts,
+                              memspace, stream, nullptr, &pt);
+}
+
 scann_status scann_treeah_last_scan_bytes(scann_treeah* h, uint64_t* bytes, uint64_t* pairs) {
   using namespace scann;
   SCANN_REQUIRE(h != nullptr, SCANN_FAILED_PRECONDITION, "searcher not built");
@@ -1315,7 +1427,7 @@ scann_status scann_treeah_search_begin(scann_treeah* h, const float* queries, si
     CallScope call(h->device, h->order, SCANN_DEVICE, stream, h->stream);
     SCANN_TRY(h->ws.reserve(treeah_chunk_bytes(h, nq, L, R, tokens != nullptr)));
     cudaMemsetAsync(h->stats.p, 0, 4 * sizeof(unsigned long long), call.s);
-    SCANN_TRY(treeah_phase1(h, queries, nq, L, R, k, true, tau_out, tokens, handle_filter(h), call.s));
+    SCANN_TRY(treeah_phase1(h, queries, nq, L, R, k, true, tau_out, tokens, handle_filter(h), ChunkParams(), call.s));
   }
   // The handle is marked busy, not locked: every other entry point answers FAILED_PRECONDITION until _end (or _abort),
   // so nothing can be left locked by a caller that fails between the two calls.

@@ -598,13 +598,77 @@ class TreeXHybridSearcher(_Handle):
                        pre_reorder_k: Optional[int] = None, want_candidates: bool = False):
         return self._search(queries, k, partitions_to_search, pre_reorder_k, want_candidates)
 
+    def search_batched_per_query(self, queries, k, pre_reorder_k=None, partitions_to_search=None,
+                                 want_candidates: bool = False):
+        """search_batched with per-query parameters in one GPU call (scann_treeah_search_with_params).  `k`,
+        `pre_reorder_k` and `partitions_to_search` are each an int or one value per query (numpy, or torch on the
+        device path).  pre_reorder_k None: config.pre_reorder_k(k_q) for every query; partitions_to_search None: the
+        config's.  Row q is bit for bit what search_batched returns for query q alone with its own values.  The
+        outputs have the row length of the largest k (the candidates: of the largest pre_reorder_k), padded beyond
+        counts[q] with id 0xFFFFFFFF and distance +inf.  A per-query torch array is reduced to its maximum on the
+        host, which synchronises with its stream."""
+        return self._search(queries, k, partitions_to_search, pre_reorder_k, want_candidates, per_query=True)
+
+    def search_batched_with_params(self, queries, params, default_k: int = 10):
+        """Searcher::search_batched_with_params (src/searcher.rs:164-169): one SearchParameters per query, the whole
+        batch in one GPU call.  k_q = num_neighbors (default_k when unset); R_q = pre_reordering_num_neighbors
+        (config.pre_reorder_k(k_q) when unset).  The result is one [(index, distance)] list per query, in query order.
+        queries.len() != params.len() → InvalidArgument (brute_force/searcher.rs:233-237)."""
+        q = queries if _is_torch(queries) else np.asarray(queries, np.float32)
+        if len(q) != len(params):
+            raise ScannError(capi.INVALID_ARGUMENT, "Number of queries must match number of parameter sets")
+        if len(params) == 0:
+            return []
+        ks = [p.num_neighbors if p.num_neighbors is not None else default_k for p in params]
+        rs = [p.pre_reordering_num_neighbors if p.pre_reordering_num_neighbors is not None
+              else self.config.pre_reorder_k(kq) for p, kq in zip(params, ks)]
+        ids, dists, counts = self.search_batched_per_query(q, np.array(ks, np.int64), np.array(rs, np.int64))
+        return results_to_lists(ids, dists, counts)
+
+    def _query_params(self, b: "_Batch", k, partitions_to_search, pre_reorder_k):
+        """(batch maximum, per-query u32 array where the batch lives or None) for k, L and R."""
+        torch = _torch() if b.device else None
+
+        def per_query(v, name):
+            if _is_torch(v) and v.dim() == 0 or not _is_torch(v) and np.ndim(v) == 0:
+                return v, None
+            if b.device:
+                a = (v if _is_torch(v) else torch.from_numpy(np.asarray(v))).to(device=b.arr.device, dtype=torch.int64)
+            else:
+                a = np.asarray(v.cpu().numpy() if _is_torch(v) else v).astype(np.int64)
+            if tuple(a.shape) != (b.nq,):
+                raise ScannError(capi.INVALID_ARGUMENT, f"{name} must hold one value per query ({b.nq})")
+            return None, a
+
+        def finish(v, a):
+            if a is None:
+                return int(v), None
+            mx = max(int(a.max()), 0) if b.nq else 0
+            return mx, (a.to(torch.int32).contiguous() if b.device else np.ascontiguousarray(a.astype(np.uint32)))
+
+        k, ka = per_query(k, "k")
+        L, La = per_query(partitions_to_search if partitions_to_search is not None
+                          else self.config.partitions_to_search, "partitions_to_search")
+        if pre_reorder_k is not None:
+            R, Ra = per_query(pre_reorder_k, "pre_reorder_k")
+        elif ka is None:
+            R, Ra = self.config.pre_reorder_k(int(k)), None
+        else:  # (k as f32 * multiplier) as usize, per query
+            mult = np.float32(self.config.pre_reorder_multiplier)
+            R, Ra = None, ((ka.to(torch.float32) * float(mult)).to(torch.int64).clamp(min=0) if b.device
+                           else np.maximum((ka.astype(np.float32) * mult).astype(np.int64), 0))
+        return finish(k, ka), finish(L, La), finish(R, Ra)
+
     def _search(self, queries, k, partitions_to_search, pre_reorder_k, want_candidates, allowed=None,
-                filter_of_query=None):
+                filter_of_query=None, per_query=False):
         if not (self._h and self._h.value):
             raise ScannError(capi.FAILED_PRECONDITION, "searcher not built")
         b = _Batch(queries, self.device)
-        L = int(partitions_to_search if partitions_to_search is not None else self.config.partitions_to_search)
-        R = int(pre_reorder_k if pre_reorder_k is not None else self.config.pre_reorder_k(k))
+        if per_query:
+            (k, ka), (L, La), (R, Ra) = self._query_params(b, k, partitions_to_search, pre_reorder_k)
+        else:
+            L = int(partitions_to_search if partitions_to_search is not None else self.config.partitions_to_search)
+            R = int(pre_reorder_k if pre_reorder_k is not None else self.config.pre_reorder_k(k))
         ids, dists, counts, pi, pd, pc = b.outputs(k)
         cand = None
         pci = pcd = pcc = None
@@ -621,7 +685,12 @@ class TreeXHybridSearcher(_Handle):
                 cc = np.zeros((b.nq,), np.uint32)
                 pci, pcd, pcc = capi.np_ptr(ci), capi.np_ptr(cd), capi.np_ptr(cc)
             cand = (ci, cd, cc)
-        if b.nq and allowed is None:
+        if b.nq and per_query:
+            ptrs = [None if a is None else C.c_void_p(a.data_ptr()) if b.device else capi.np_ptr(a)
+                    for a in (La, Ra, ka)]
+            capi.check(capi.load().scann_treeah_search_with_params(self._h, b.ptr, b.nq, b.dim, L, R, k, *ptrs, pi, pd,
+                                                                   pc, pci, pcd, pcc, b.memspace, b.stream))
+        elif b.nq and allowed is None:
             capi.check(capi.load().scann_treeah_search(self._h, b.ptr, b.nq, b.dim, L, R, k, pi, pd, pc, pci, pcd, pcc,
                                                        b.memspace, b.stream))
         elif b.nq:
@@ -774,6 +843,10 @@ class AsymmetricHasher(TreeXHybridSearcher):
                 raise ScannError(capi.FAILED_PRECONDITION, "Dataset not stored")
             TreeXHybridSearcher.build_from_index(self, centers, cb, packed, ids, off, self._raw if with_raw else None)
             self._have = with_raw
+
+    # pre_reordering_num_neighbors means something else here (search vs search_with_reordering): queries that share
+    # their parameters go to the GPU as one batch
+    search_batched_with_params = _Handle.search_batched_with_params
 
     def search_batched(self, queries, k: int):
         self._ensure(False)
