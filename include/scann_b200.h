@@ -164,6 +164,28 @@ scann_status scann_treeah_create_ex(const float* centers, size_t K, size_t dim, 
                                     size_t n, const float* raw, size_t num_raw, size_t stride, int use_residuals,
                                     int reorder_measure, uint32_t flags, int device, int memspace,
                                     scann_treeah** out);
+/* TreeXHybridSearcher over byte codes with the reference's f32 LookupTable (tree_x_hybrid/mod.rs:297-339,
+ * hashes/lut.rs:47-82): codebook[S*C*ds] f32 (1 <= C <= 256), codes[n*S] u8 = Codebook::encode output, one byte per
+ * subspace, rows GROUPED BY PARTITION like `packed` of scann_treeah_create; everything else as scann_treeah_create_ex
+ * (flags RAW_BY_POSITION / BORROW_RAW included).  K == 1, use_residuals == 0 is the flat AsymmetricHasher
+ * (hasher.rs:162-229).
+ *   The result is an ordinary handle: scann_treeah_search, _search_filtered, _search_with_params, _set_filter,
+ *   _set_reorder, _partition, the profile and the counters take it unchanged.  Per (query, leaf) the scan builds the
+ *   residual f32 table [S][C], sums table[s][code] for s = 0..S-1 in that order (bit for bit the reference's
+ *   compute_distance) and keeps the leaf's top R by (approximate distance, position), exactly as FastTopNeighbors
+ *   outside exact ties of the distance.
+ *   Limits: those of scann_treeah_create_ex except the leaf size, which is < 2^22 points; the scan holds one S x C
+ *   table per query in shared memory, so S*C*4 bytes plus the candidate buffer of R must fit 227 KB.
+ *   Errors: INVALID_ARGUMENT for C outside 1..256 or a code byte >= C (checked on the device); OUT_OF_RANGE for a leaf
+ *   of >= 2^22 points or a geometry whose scan does not fit even with R = 1; at search time RESOURCE_EXHAUSTED for an
+ *   R that does not fit; UNIMPLEMENTED from scann_treeah_search_begin / _end (split search serves LUT16 handles).
+ *   scann_treeah_last_scan_bytes counts S bytes per point; scann_treeah_path_stats counts every chunk of such a
+ *   handle in lut_chunks (tc_chunks stays 0). */
+scann_status scann_treeah_create_lut_f32(const float* centers, size_t K, size_t dim, const float* codebook, size_t S,
+                                         size_t C, const uint8_t* codes, const uint32_t* ids,
+                                         const uint64_t* part_offsets, size_t n, const float* raw, size_t num_raw,
+                                         size_t stride, int use_residuals, int reorder_measure, uint32_t flags,
+                                         int device, int memspace, scann_treeah** out);
 scann_status scann_treeah_search(scann_treeah* h, const float* queries, size_t nq, size_t qdim, size_t L, size_t R,
                                  size_t k, uint32_t* ids, float* dists, uint32_t* counts, uint32_t* cand_ids,
                                  float* cand_dists, uint32_t* cand_counts, int memspace, void* stream);
@@ -234,12 +256,14 @@ scann_status scann_treeah_search_end(scann_treeah* h, const float* tau_in, uint3
                                      uint32_t* counts, void* stream);
 scann_status scann_treeah_search_abort(scann_treeah* h);
 /* introspection used by bench.py for the roofline arithmetic: algorithmic code bytes scanned by the
- * last scann_treeah_search call (Σ over (query, leaf) pairs of leaf_size * ceil(S/2)); host sync. */
+ * last scann_treeah_search call (Σ over (query, leaf) pairs of leaf_size * ceil(S/2); leaf_size * S on a byte-code
+ * handle of scann_treeah_create_lut_f32); host sync. */
 scann_status scann_treeah_last_scan_bytes(scann_treeah* h, uint64_t* bytes, uint64_t* pairs);
 /* which scan kernel served the query chunks of this handle so far: the tensor-core LUT16 scan (tcgen05.mma kind::i8 over
  * one-hot expanded codes, csrc/tcscan.cu; used when the index supports it — S a multiple of 16, S <= 64 — and a leaf is
  * probed by >= 12 queries of the batch on average; SCANN_SCAN_TC=0/1 overrides) or the register-LUT kernel.  Both
- * compute the same u32 sums and return identical results. */
+ * compute the same u32 sums and return identical results.  On a byte-code handle (scann_treeah_create_lut_f32) every
+ * chunk counts in lut_chunks (its f32 scan kernel) and tc_chunks stays 0. */
 scann_status scann_treeah_path_stats(scann_treeah* h, uint64_t* tc_chunks, uint64_t* lut_chunks);
 /* tensor-core scan share of the profile (valid while profiling is enabled, call BEFORE scann_treeah_get_profile, which
  * resets the accumulators): milliseconds of the LUT-tile build kernel and of the tcgen05 scan kernel summed over their

@@ -260,7 +260,7 @@ struct SearchParameters {  // src/searcher.rs:23-77, the fields the GPU path rea
 struct TreeXHybridConfig {  // src/tree_x_hybrid/mod.rs:23-78
   size_t num_partitions = 100;
   size_t partitions_to_search = 10;
-  size_t num_subspaces = 8;       // hash_config.num_subspaces (num_codes is 16 on the LUT16 path)
+  size_t num_subspaces = 8;       // hash_config.num_subspaces (num_codes is 16 on the LUT16 path; build_from_byte_codes takes 1..256)
   bool use_residuals = true;
   float pre_reorder_multiplier = 3.0f;
   DistanceMeasure distance_measure = DistanceMeasure::SquaredL2;  // reorder measure (hard-wired SqL2 in the reference, :124)
@@ -286,6 +286,18 @@ class TreeXHybridSearcher {
     return make_error(scann_treeah_create(centers, K, dim, codebook, S, packed, ids, part_offsets, n, raw, num_raw, stride,
                                           cfg_.use_residuals ? 1 : 0, static_cast<int>(cfg_.distance_measure), device,
                                           SCANN_HOST, &h_));
+  }
+  // the same index over byte codes with the reference's f32 LookupTable (scann_treeah_create_lut_f32): codebook
+  // [S][C][ds] with 1 <= C <= 256, codes [n][S] = Codebook::encode rows grouped by partition
+  ScannError build_from_byte_codes(const float* centers, size_t K, size_t dim, const float* codebook, size_t S,
+                                   size_t C, const uint8_t* codes, const uint32_t* ids, const uint64_t* part_offsets,
+                                   size_t n, const float* raw, size_t num_raw, size_t stride, int device = 0) {
+    scann_treeah_destroy(h_);
+    h_ = nullptr;
+    return make_error(scann_treeah_create_lut_f32(centers, K, dim, codebook, S, C, codes, ids, part_offsets, n, raw,
+                                                  num_raw, stride, cfg_.use_residuals ? 1 : 0,
+                                                  static_cast<int>(cfg_.distance_measure), 0u, device, SCANN_HOST,
+                                                  &h_));
   }
 
   Result<std::vector<NNResultsVector>> search_batched(const std::vector<std::vector<float>>& queries, size_t k) const {

@@ -11,7 +11,7 @@ CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libscann_b200.so")
 SOURCES = ["runtime.cu", "partition.cu", "select.cu", "treeah.cu", "taps.cu", "brute_force.cu", "tc_gemm.cu", "ivf.cu", "tcscan.cu", "build_index.cu", "kmtree.cu"]
-HEADERS = ["common.cuh", "kernels.h", "lut16_device.cuh", "lut16_scan_kernel.cuh", "tcscan.h", os.path.join("..", "..", "include", "scann_b200.h")]
+HEADERS = ["common.cuh", "kernels.h", "lut16_device.cuh", "lut16_scan_kernel.cuh", "lut_f32_device.cuh", "lut_f32_scan_kernel.cuh", "tcscan.h", os.path.join("..", "..", "include", "scann_b200.h")]
 
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = [

@@ -34,7 +34,7 @@ SYMBOLS = [
     "scann_bf_create", "scann_bf_search", "scann_bf_search_radius", "scann_bf_destroy", "scann_bf_path_stats", "scann_sq8_path_stats",
     "scann_sq8_quantize", "scann_sq8_create", "scann_sq8_search", "scann_sq8_destroy",
     "scann_part_create", "scann_part_select", "scann_part_destroy", "scann_part_update",
-    "scann_treeah_create", "scann_treeah_create_ex", "scann_treeah_search", "scann_treeah_search_filtered", "scann_treeah_search_with_params", "scann_treeah_destroy", "scann_treeah_last_scan_bytes",
+    "scann_treeah_create", "scann_treeah_create_ex", "scann_treeah_create_lut_f32", "scann_treeah_search", "scann_treeah_search_filtered", "scann_treeah_search_with_params", "scann_treeah_destroy", "scann_treeah_last_scan_bytes",
     "scann_treeah_set_profiling", "scann_treeah_get_profile", "scann_treeah_search_begin", "scann_treeah_search_end", "scann_treeah_search_abort", "scann_treeah_partition",
     "scann_treeah_set_filter", "scann_treeah_path_stats", "scann_treeah_tc_profile",
     "scann_lut16_build", "scann_lut16_scan", "scann_pq_encode", "scann_merge_topk", "scann_merge_topk_packed", "scann_tc_scores",
@@ -96,6 +96,8 @@ def load():
                                       C.POINTER(vp)]
     L.scann_treeah_create_ex.argtypes = [vp, sz, sz, vp, sz, vp, vp, vp, sz, vp, sz, sz, i32, i32, C.c_uint32, i32, i32,
                                          C.POINTER(vp)]
+    L.scann_treeah_create_lut_f32.argtypes = [vp, sz, sz, vp, sz, sz, vp, vp, vp, sz, vp, sz, sz, i32, i32, C.c_uint32,
+                                              i32, i32, C.POINTER(vp)]
     L.scann_treeah_search.argtypes = [vp, vp, sz, sz, sz, sz, sz, vp, vp, vp, vp, vp, vp, i32, vp]
     L.scann_treeah_search_filtered.argtypes = [vp, vp, sz, sz, sz, sz, sz, vp, sz, sz, vp, vp, vp, vp, vp, vp, vp, i32, vp]
     L.scann_treeah_search_with_params.argtypes = [vp, vp, sz, sz, sz, sz, sz, vp, vp, vp, vp, vp, vp, vp, vp, vp, i32, vp]

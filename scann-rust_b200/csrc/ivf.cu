@@ -21,6 +21,7 @@
 #include <algorithm>
 
 #include "kernels.h"
+#include "lut_f32_device.cuh"
 
 namespace scann {
 
@@ -112,17 +113,7 @@ __global__ void __launch_bounds__(256) ivf_topk_kernel(const IvfArgs a) {
     prefix[0] = 0;
     for (int r = 0; r < a.L; ++r) prefix[r + 1] += prefix[r];
   }
-  if (a.lut_mode) {  // LookupTable::from_query: sequential un-fused squared distance to every centroid
-    for (int e = tid; e < a.S * a.C; e += 256) {
-      const int s = e / a.C;
-      float sum = 0.0f;
-      for (int j = 0; j < a.ds; ++j) {
-        const float d = __fsub_rn(qs[s * a.ds + j], __ldg(a.codebook + static_cast<size_t>(e) * a.ds + j));
-        sum = __fadd_rn(sum, __fmul_rn(d, d));
-      }
-      lut[e] = sum;
-    }
-  }
+  if (a.lut_mode) lut_f32_build(lut, qs, a.codebook, a.S, a.C, a.ds, tid, 256);  // LookupTable::from_query
   __syncthreads();
   const int total = static_cast<int>(prefix[a.L]);
   const bool vec = (a.stride & 3) == 0 && (reinterpret_cast<uintptr_t>(a.raw) & 15) == 0;
@@ -142,27 +133,8 @@ __global__ void __launch_bounds__(256) ivf_topk_kernel(const IvfArgs a) {
     const uint32_t id = a.ids[a.pt_off[a.tokens[q * a.L + cur]] + (static_cast<uint32_t>(i) - prefix[cur])];
     float d;
     if (a.lut_mode) {
-      // LookupTable::compute_distance: sum += distances[s][code_s] for s = 0..S-1, in that order.  The code row is
-      // fetched with the widest aligned loads available (one byte load per subspace made the kernel LSU-bound).
-      const uint8_t* c = a.codes + static_cast<size_t>(id) * a.S;
-      d = 0.0f;
-      auto add4 = [&](uint32_t w, int s0) {
-#pragma unroll
-        for (int j = 0; j < 4; ++j) d = __fadd_rn(d, lut[(s0 + j) * a.C + ((w >> (8 * j)) & 0xFFu)]);
-      };
-      if ((a.S & 15) == 0) {
-        for (int s0 = 0; s0 < a.S; s0 += 16) {
-          const uint4 w = __ldg(reinterpret_cast<const uint4*>(c + s0));
-          add4(w.x, s0);
-          add4(w.y, s0 + 4);
-          add4(w.z, s0 + 8);
-          add4(w.w, s0 + 12);
-        }
-      } else if ((a.S & 3) == 0) {
-        for (int s0 = 0; s0 < a.S; s0 += 4) add4(__ldg(reinterpret_cast<const uint32_t*>(c + s0)), s0);
-      } else {
-        for (int s = 0; s < a.S; ++s) d = __fadd_rn(d, lut[s * a.C + c[s]]);
-      }
+      // LookupTable::compute_distance: sum += distances[s][code_s] for s = 0..S-1, in that order
+      d = lut_f32_row_distance(lut, a.codes + static_cast<size_t>(id) * a.S, a.S, a.C);
     } else {
       d = exact_pair_distance_1t(qs, a.raw + static_cast<size_t>(id) * a.stride, a.dim, a.measure, vec);
     }

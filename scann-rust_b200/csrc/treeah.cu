@@ -24,6 +24,7 @@
 
 #include "kernels.h"
 #include "lut16_scan_kernel.cuh"
+#include "lut_f32_scan_kernel.cuh"
 #include "tcscan.h"
 
 namespace scann {
@@ -59,6 +60,34 @@ __global__ void repack_blocked_kernel(const uint8_t* __restrict__ packed, const 
     }
   }
   out[w] = word;
+}
+
+// Converts byte codes (Codebook::encode rows, row-major [n][S] in leaf order) to the same 256-point blocks, stored
+// subspace-major inside a block: byte s*256 + j of a block is subspace s of its point j, so lane l of a warp reads
+// points l*8 .. l*8+7 of one subspace as 8 contiguous bytes (lut_f32_scan_kernel).  One thread per output u32 (4 points
+// of one subspace); codes >= C are counted into *bad (the scan would read outside the table row).
+__global__ void repack_bytes_kernel(const uint8_t* __restrict__ codes, const uint32_t* __restrict__ blk_leaf,
+                                    const uint32_t* __restrict__ blk_off, const uint64_t* __restrict__ pt_off, int S,
+                                    uint32_t C, size_t total_words, uint32_t* __restrict__ out, uint32_t* __restrict__ bad) {
+  const size_t w = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (w >= total_words) return;
+  const int j4 = static_cast<int>(w & 63);
+  const size_t rest = w >> 6;
+  const int s = static_cast<int>(rest % S);
+  const size_t gb = rest / S;
+  const uint32_t leaf = blk_leaf[gb];
+  const uint64_t p0 = pt_off[leaf] + static_cast<uint64_t>(gb - blk_off[leaf]) * kBlockPts + j4 * 4, pend = pt_off[leaf + 1];
+  uint32_t word = 0, nbad = 0;
+#pragma unroll
+  for (int i = 0; i < 4; ++i) {
+    if (p0 + i < pend) {
+      const uint32_t c = codes[(p0 + i) * S + s];
+      nbad += c >= C ? 1u : 0u;
+      word |= c << (8 * i);
+    }
+  }
+  out[w] = word;
+  if (nbad) atomicAdd(bad, nbad);
 }
 
 // --------------------------------------------------------------------------------------- worklist
@@ -536,6 +565,10 @@ struct scann_treeah {
   size_t K = 0, dim = 0, S = 0, ds = 0, SG = 0, n = 0, num_raw = 0, stride = 0;
   int use_residuals = 1, reorder_measure = SCANN_SQL2, pos_bits = 18;
   uint32_t max_leaf = 0;
+  // code format: false = nibble codes scanned through LUT16 (scann_treeah_create_ex), true = byte codes with C codes per
+  // subspace scanned through the f32 LookupTable (scann_treeah_create_lut_f32, lut_f32_scan_kernel.cuh)
+  bool f32lut = false;
+  size_t C = 16;
   scann::CentreScorer part;  // the partition stage; part.centers() are the f32 centres of the residual LUTs
   scann::DevBuf<float> codebook, raw;
   const float* raw_p = nullptr;  // raw.p, or the caller's device array (SCANN_TREEAH_BORROW_RAW)
@@ -670,6 +703,49 @@ static scann_status launch_scan_g(int G, const ScanArgs& a, int sms, cudaStream_
   }
 }
 
+// the byte-code scan (lut_f32_scan_kernel.cuh); C = codes per subspace
+template <int G, bool FILT>
+static scann_status launch_f32_scan(ScanArgs a, int C, int sms, cudaStream_t s) {
+  a.cap = scan_list_cap(a.R, kScanWarps);
+  const size_t smem = lut_f32_scan_smem_bytes(G, a.S, C, a.dim, a.cap, kScanWarps);
+  SCANN_REQUIRE(smem <= kScanSmemMax, SCANN_RESOURCE_EXHAUSTED, "scan kernel needs %zu B of shared memory (R too large)",
+                smem);
+  auto kern = lut_f32_scan_kernel<G, kScanWarps, FILT>;
+  SCANN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+  int occ = 0;
+  SCANN_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kScanWarps * 32, smem));
+  if (occ < 1) occ = 1;
+  kern<<<sms * occ, kScanWarps * 32, smem, s>>>(a, C);
+  SCANN_CUDA(cudaGetLastError());
+  return SCANN_OK;
+}
+
+template <int G>
+static scann_status launch_f32_scan_filt(const ScanArgs& a, int C, int sms, cudaStream_t s) {
+  if (a.allow != nullptr) return launch_f32_scan<G, true>(a, C, sms, s);
+  return launch_f32_scan<G, false>(a, C, sms, s);
+}
+
+// the scan kernel of the handle's code format, G queries per work item
+static scann_status launch_handle_scan(const scann_treeah* h, int G, const ScanArgs& a, cudaStream_t s) {
+  if (!h->f32lut) return launch_scan_g(G, a, h->sms, s);
+  const int C = static_cast<int>(h->C);
+  switch (G) {
+    case 8: return launch_f32_scan_filt<8>(a, C, h->sms, s);
+    case 4: return launch_f32_scan_filt<4>(a, C, h->sms, s);
+    case 2: return launch_f32_scan_filt<2>(a, C, h->sms, s);
+    default: return launch_f32_scan_filt<1>(a, C, h->sms, s);
+  }
+}
+
+// shared memory of one scan CTA of the handle's code format with G queries per work item
+static size_t scan_cta_bytes(const scann_treeah* h, int G, int cap, bool filt) {
+  if (h->f32lut)
+    return lut_f32_scan_smem_bytes(G, static_cast<int>(h->S), static_cast<int>(h->C), static_cast<int>(h->dim), cap,
+                                   kScanWarps);
+  return scan_smem_bytes(G, static_cast<int>(h->SG) * 4, static_cast<int>(h->dim), cap, kScanWarps, filt);
+}
+
 // Worklist of the register-LUT scan over `tokens` (buffers in h->ck): count -> scans -> scatter -> items.  with_stats:
 // add the batch's algorithmic scan bytes / pairs to h->stats.
 static scann_status treeah_worklist(scann_treeah* h, const uint32_t* tokens, size_t nq, size_t L, bool first,
@@ -688,7 +764,9 @@ static scann_status treeah_worklist(scann_treeah* h, const uint32_t* tokens, siz
   wl_count_kernel<<<pb, 256, 0, s>>>(tokens, P, static_cast<uint32_t>(K), static_cast<uint32_t>(L), T, h->pt_off.p,
                                      pad_cnt);
   wl_unpad_kernel<<<static_cast<unsigned>((2 * K + 255) / 256), 256, 0, s>>>(pad_cnt, static_cast<uint32_t>(2 * K), leaf_cnt);
-  const uint32_t nwb = static_cast<uint32_t>((2 * K + kWlBlock - 1) / kWlBlock), bpp32 = static_cast<uint32_t>((h->S + 1) / 2);
+  // code bytes per point: ceil(S/2) nibble-packed, S as byte codes
+  const uint32_t nwb = static_cast<uint32_t>((2 * K + kWlBlock - 1) / kWlBlock),
+                 bpp32 = static_cast<uint32_t>(h->f32lut ? h->S : (h->S + 1) / 2);
   wl_reduce_kernel<<<nwb, kWlBlock, 0, s>>>(leaf_cnt, static_cast<uint32_t>(K), G, h->leaf_perm.p, h->pt_off.p, bpp32,
                                             h->ck.wl_blk_pair, h->ck.wl_blk_item, h->ck.wl_blk_bytes);
   wl_scan_blocks_kernel<<<1, 1024, 0, s>>>(h->ck.wl_blk_pair, h->ck.wl_blk_item, h->ck.wl_blk_bytes, nwb, h->ck.counters,
@@ -768,9 +846,7 @@ static scann_status treeah_phase1(scann_treeah* h, const float* dq, size_t nq, s
   // the scan CTA holds G queries' residuals, tables and candidate buffers: smaller groups where they do not fit (each
   // pair's per-leaf top-R does not depend on which queries share its item, so results stay the same)
   const int cap = scan_list_cap(static_cast<int>(R), kScanWarps);
-  while (G > 1 && scan_smem_bytes(G, static_cast<int>(h->SG) * 4, static_cast<int>(h->dim), cap, kScanWarps,
-                                  filt.allow != nullptr) > kScanSmemMax)
-    G /= 2;
+  while (G > 1 && scan_cta_bytes(h, G, cap, filt.allow != nullptr) > kScanSmemMax) G /= 2;
   size_t max_items = P / G + 2 * std::min<size_t>(K, P) + 1;
 
   // centre-score scratch of the partition stage (not needed when the caller partitioned)
@@ -962,7 +1038,7 @@ static scann_status treeah_phase2(scann_treeah* h, bool two_phase, const float* 
   }
   a.end_idx = 0;
   a.max_blocks = 0;
-  SCANN_TRY(launch_scan_g(h->ck.G, a, h->sms, s));
+  SCANN_TRY(launch_handle_scan(h, h->ck.G, a, s));
   h->span_end(s);
   // 4. merge + reorder
   h->span_begin(3, s);
@@ -1196,24 +1272,13 @@ static scann_status treeah_search(scann_treeah* h, const float* queries, size_t 
   });
 }
 
-}  // namespace scann
-
-extern "C" {
-
-scann_status scann_treeah_create(const float* centers, size_t K, size_t dim, const float* codebook, size_t S,
-                                 const uint8_t* packed, const uint32_t* ids, const uint64_t* part_offsets,
-                                 size_t n, const float* raw, size_t num_raw, size_t stride, int use_residuals,
-                                 int reorder_measure, int device, int memspace, scann_treeah** out) {
-  return scann_treeah_create_ex(centers, K, dim, codebook, S, packed, ids, part_offsets, n, raw, num_raw, stride,
-                                use_residuals, reorder_measure, 0u, device, memspace, out);
-}
-
-scann_status scann_treeah_create_ex(const float* centers, size_t K, size_t dim, const float* codebook, size_t S,
-                                    const uint8_t* packed, const uint32_t* ids, const uint64_t* part_offsets,
-                                    size_t n, const float* raw, size_t num_raw, size_t stride, int use_residuals,
-                                    int reorder_measure, uint32_t flags, int device, int memspace,
-                                    scann_treeah** out) {
-  using namespace scann;
+// scann_treeah_create_ex (bytes = false: `packed` holds PackedCodes4Bit rows, C = 16) and scann_treeah_create_lut_f32
+// (bytes = true: `packed` holds byte codes [n][S], C codes per subspace)
+static scann_status treeah_create(const float* centers, size_t K, size_t dim, const float* codebook, size_t S,
+                                  size_t C, bool bytes, const uint8_t* packed, const uint32_t* ids,
+                                  const uint64_t* part_offsets, size_t n, const float* raw, size_t num_raw,
+                                  size_t stride, int use_residuals, int reorder_measure, uint32_t flags, int device,
+                                  int memspace, scann_treeah** out) {
   SCANN_REQUIRE((flags & ~(SCANN_TREEAH_RAW_BY_POSITION | SCANN_TREEAH_BORROW_RAW)) == 0, SCANN_INVALID_ARGUMENT,
                 "unknown flags 0x%x", flags);
   SCANN_REQUIRE(!(flags & SCANN_TREEAH_BORROW_RAW) || memspace == SCANN_DEVICE, SCANN_INVALID_ARGUMENT,
@@ -1231,10 +1296,21 @@ scann_status scann_treeah_create_ex(const float* centers, size_t K, size_t dim, 
                 SCANN_INVALID_ARGUMENT, "unsupported reorder measure %d", reorder_measure);
   SCANN_REQUIRE(raw == nullptr || stride >= dim, SCANN_INVALID_ARGUMENT, "stride %zu < dim %zu", stride, dim);
   SCANN_REQUIRE(K < 0xFFFFFFFFull && n < 0xFFFFFFFFull, SCANN_INVALID_ARGUMENT, "index too large for u32 ids");
+  if (bytes) {
+    SCANN_REQUIRE(C >= 1 && C <= 256, SCANN_INVALID_ARGUMENT, "num_codes %zu outside 1..256", C);
+    // the scan CTA holds one query's S x C table: a geometry that does not fit with one query and R = 1 cannot be searched
+    const size_t smem = lut_f32_scan_smem_bytes(1, static_cast<int>(S), static_cast<int>(C), static_cast<int>(dim),
+                                                scan_list_cap(1, kScanWarps), kScanWarps);
+    SCANN_REQUIRE(smem <= kScanSmemMax, SCANN_OUT_OF_RANGE,
+                  "S=%zu x C=%zu f32 lookup table: the scan needs %zu B of shared memory per query (> %zu)", S, C, smem,
+                  kScanSmemMax);
+  }
   SCANN_TRY(check_device(device));
   DeviceGuard g(device);
 
   scann_treeah* h = new scann_treeah();
+  h->f32lut = bytes;
+  h->C = C;
   h->device = device;
   h->K = K;
   h->dim = dim;
@@ -1250,7 +1326,8 @@ scann_status scann_treeah_create_ex(const float* centers, size_t K, size_t dim, 
   int sum_bits = 1;
   while ((1u << sum_bits) <= 255u * S + 1u) ++sum_bits;  // scores 0..255*S plus the filter sentinel 255*S + 1
   h->pos_bits = 32 - sum_bits;
-  if (h->pos_bits > 22) h->pos_bits = 22;
+  // f32 distances carry no integer sum: the position keeps the 22 bits of the merge key (distance, leaf rank, position)
+  if (h->pos_bits > 22 || bytes) h->pos_bits = 22;
 
   scann_status st = SCANN_OK;
   do {
@@ -1296,9 +1373,9 @@ scann_status scann_treeah_create_ex(const float* centers, size_t K, size_t dim, 
     DevBuf<uint8_t> d_packed;
     DevBuf<uint32_t>& d_blk_leaf = h->blk_leaf;
     h->num_blocks = nb;
-    size_t bpp = (S + 1) / 2;
+    size_t bpp = bytes ? S : (S + 1) / 2;
     if ((st = h->part.set(centers, K, dim, memspace, s)) != SCANN_OK) break;
-    if ((st = h->codebook.upload(codebook, S * 16 * h->ds, memspace, s)) != SCANN_OK) break;
+    if ((st = h->codebook.upload(codebook, S * C * h->ds, memspace, s)) != SCANN_OK) break;
     if ((st = h->ids.upload(ids, n, memspace, s)) != SCANN_OK) break;
     if ((st = h->pt_off.upload(off.data(), K + 1, SCANN_HOST, s)) != SCANN_OK) break;
     if ((st = h->blk_off.upload(blk_off.data(), K + 1, SCANN_HOST, s)) != SCANN_OK) break;
@@ -1309,9 +1386,31 @@ scann_status scann_treeah_create_ex(const float* centers, size_t K, size_t dim, 
     if ((st = h->leaf_perm.upload(perm.data(), K, SCANN_HOST, s)) != SCANN_OK) break;
     if ((st = d_blk_leaf.upload(blk_leaf.data(), nb, SCANN_HOST, s)) != SCANN_OK) break;
     if ((st = d_packed.upload(packed, n * bpp, memspace, s)) != SCANN_OK) break;
-    h->tc_ok = tc_scan_supported(S, dim);
-    size_t words = static_cast<size_t>(nb) * h->SG * 128;
-    if ((st = h->codes.alloc(words > 0 ? words : 4)) != SCANN_OK) break;
+    if (bytes) {
+      const size_t words = static_cast<size_t>(nb) * S * (kBlockPts / 4);
+      if ((st = h->codes.alloc(words > 0 ? words : 4)) != SCANN_OK) break;
+      DevBuf<uint32_t> bad;
+      if ((st = bad.alloc(1)) != SCANN_OK) break;
+      cudaMemsetAsync(bad.p, 0, 4, s);
+      if (words > 0)
+        repack_bytes_kernel<<<static_cast<unsigned>((words + 255) / 256), 256, 0, s>>>(
+            d_packed.p, d_blk_leaf.p, h->blk_off.p, h->pt_off.p, static_cast<int>(S), static_cast<uint32_t>(C), words,
+            h->codes.p, bad.p);
+      uint32_t nbad = 0;
+      if (cudaMemcpyAsync(&nbad, bad.p, 4, cudaMemcpyDeviceToHost, s) != cudaSuccess ||
+          cudaStreamSynchronize(s) != cudaSuccess) {
+        st = cuda_fail(cudaGetLastError(), "treeah_create code check", __FILE__, __LINE__);
+        break;
+      }
+      if (nbad != 0) {
+        set_error("%u codes are >= num_codes %zu", nbad, C);
+        st = SCANN_INVALID_ARGUMENT;
+        break;
+      }
+    }
+    h->tc_ok = !bytes && tc_scan_supported(S, dim);
+    size_t words = bytes ? 0 : static_cast<size_t>(nb) * h->SG * 128;
+    if (!bytes && (st = h->codes.alloc(words > 0 ? words : 4)) != SCANN_OK) break;
     if (words > 0) {
       repack_blocked_kernel<<<static_cast<unsigned>((words + 255) / 256), 256, 0, s>>>(
           d_packed.p, d_blk_leaf.p, h->blk_off.p, h->pt_off.p, static_cast<int>(S), static_cast<int>(h->SG), words,
@@ -1341,6 +1440,36 @@ scann_status scann_treeah_create_ex(const float* centers, size_t K, size_t dim, 
   }
   *out = h;
   return SCANN_OK;
+}
+
+}  // namespace scann
+
+extern "C" {
+
+scann_status scann_treeah_create(const float* centers, size_t K, size_t dim, const float* codebook, size_t S,
+                                 const uint8_t* packed, const uint32_t* ids, const uint64_t* part_offsets,
+                                 size_t n, const float* raw, size_t num_raw, size_t stride, int use_residuals,
+                                 int reorder_measure, int device, int memspace, scann_treeah** out) {
+  return scann_treeah_create_ex(centers, K, dim, codebook, S, packed, ids, part_offsets, n, raw, num_raw, stride,
+                                use_residuals, reorder_measure, 0u, device, memspace, out);
+}
+
+scann_status scann_treeah_create_ex(const float* centers, size_t K, size_t dim, const float* codebook, size_t S,
+                                    const uint8_t* packed, const uint32_t* ids, const uint64_t* part_offsets,
+                                    size_t n, const float* raw, size_t num_raw, size_t stride, int use_residuals,
+                                    int reorder_measure, uint32_t flags, int device, int memspace,
+                                    scann_treeah** out) {
+  return scann::treeah_create(centers, K, dim, codebook, S, 16, false, packed, ids, part_offsets, n, raw, num_raw,
+                              stride, use_residuals, reorder_measure, flags, device, memspace, out);
+}
+
+scann_status scann_treeah_create_lut_f32(const float* centers, size_t K, size_t dim, const float* codebook, size_t S,
+                                         size_t C, const uint8_t* codes, const uint32_t* ids,
+                                         const uint64_t* part_offsets, size_t n, const float* raw, size_t num_raw,
+                                         size_t stride, int use_residuals, int reorder_measure, uint32_t flags,
+                                         int device, int memspace, scann_treeah** out) {
+  return scann::treeah_create(centers, K, dim, codebook, S, C, true, codes, ids, part_offsets, n, raw, num_raw, stride,
+                              use_residuals, reorder_measure, flags, device, memspace, out);
 }
 
 scann_status scann_treeah_search(scann_treeah* h, const float* queries, size_t nq, size_t qdim, size_t L, size_t R,
@@ -1412,6 +1541,7 @@ scann_status scann_treeah_search_begin(scann_treeah* h, const float* queries, si
                                        size_t R, size_t k, const uint32_t* tokens, float* tau_out, void* stream) {
   using namespace scann;
   SCANN_REQUIRE(h != nullptr, SCANN_FAILED_PRECONDITION, "searcher not built");
+  SCANN_REQUIRE(!h->f32lut, SCANN_UNIMPLEMENTED, "the split search serves nibble-code (LUT16) handles only");
   SCANN_REQUIRE(!h->split_active, SCANN_FAILED_PRECONDITION, "scann_treeah_search_begin called twice without _end");
   SCANN_REQUIRE(queries && tau_out && nq >= 1, SCANN_INVALID_ARGUMENT, "NULL buffer or empty batch");
   SCANN_REQUIRE(qdim == h->dim, SCANN_INVALID_ARGUMENT, "Query dimensionality mismatch");
@@ -1447,6 +1577,7 @@ scann_status scann_treeah_search_end(scann_treeah* h, const float* tau_in, uint3
                                      uint32_t* counts, void* stream) {
   using namespace scann;
   SCANN_REQUIRE(h != nullptr, SCANN_FAILED_PRECONDITION, "searcher not built");
+  SCANN_REQUIRE(!h->f32lut, SCANN_UNIMPLEMENTED, "the split search serves nibble-code (LUT16) handles only");
   std::lock_guard<std::mutex> lock(h->mu);
   SCANN_REQUIRE(h->split_active, SCANN_FAILED_PRECONDITION, "scann_treeah_search_end without _begin");
   scann_status st = SCANN_OK;

@@ -541,17 +541,37 @@ class TreeXHybridSearcher(_Handle):
         capi.require_gpu()
         if packed.shape[0] == 0:
             raise ScannError(capi.INVALID_ARGUMENT, "Cannot build from empty dataset")
-        K, dim = int(centers.shape[0]), int(centers.shape[1])
-        S = int(codebook.shape[0])
         if int(codebook.shape[1]) != 16:
             raise ScannError(capi.UNIMPLEMENTED, "the GPU AH path is LUT16: num_codes must be 16")
+        return self._create(capi.load().scann_treeah_create_ex, centers, codebook, packed, ids, part_offsets, raw,
+                            raw_by_position, borrow_raw)
+
+    def build_from_byte_codes(self, centers, codebook, codes, ids, part_offsets, raw=None,
+                              raw_by_position: bool = False, borrow_raw: bool = False):
+        """TreeXHybridSearcher over byte codes with the reference's f32 LookupTable (scann_treeah_create_lut_f32):
+        codebook [S, C, ds] f32 with 1 <= C <= 256 codes per subspace, codes [n, S] u8 = Codebook::encode rows grouped
+        by partition; ids, part_offsets, raw, raw_by_position and borrow_raw as in build_from_index.  Every search
+        method then works unchanged; the scan sums the f32 table entries in subspace order, as the reference does."""
+        capi.require_gpu()
+        if codes.shape[0] == 0:
+            raise ScannError(capi.INVALID_ARGUMENT, "Cannot build from empty dataset")
+        if len(codes.shape) != 2 or int(codes.shape[1]) != int(codebook.shape[0]):
+            raise ScannError(capi.INVALID_ARGUMENT, "codes must hold one byte per subspace: [n, S]")
+        num_codes = int(codebook.shape[1])
+        return self._create(lambda p_c, K, dim, p_cb, S, *rest: capi.load().scann_treeah_create_lut_f32(
+            p_c, K, dim, p_cb, S, num_codes, *rest), centers, codebook, codes, ids, part_offsets, raw, raw_by_position,
+            borrow_raw)
+
+    def _create(self, create, centers, codebook, codes, ids, part_offsets, raw, raw_by_position, borrow_raw):
+        K, dim = int(centers.shape[0]), int(centers.shape[1])
+        S = int(codebook.shape[0])
         if dim % S != 0:
             raise ScannError(capi.INVALID_ARGUMENT,
                              f"Dimensionality {dim} must be divisible by num_subspaces {S}")
-        n = int(packed.shape[0])
+        n = int(codes.shape[0])
         p_c, ms_c, k1 = _dataset_ptr(centers, np.float32)
         p_cb, ms_cb, k2 = _dataset_ptr(codebook, np.float32)
-        p_pk, ms_pk, k3 = _dataset_ptr(packed, np.uint8)
+        p_pk, ms_pk, k3 = _dataset_ptr(codes, np.uint8)
         p_id, ms_id, k4 = _dataset_ptr(ids, np.uint32)
         p_off, ms_off, k5 = _dataset_ptr(part_offsets, np.uint64)
         spaces = {ms_c, ms_cb, ms_pk, ms_id, ms_off}
@@ -567,10 +587,9 @@ class TreeXHybridSearcher(_Handle):
         flags = (capi.TREEAH_RAW_BY_POSITION if raw_by_position and raw is not None else 0) | \
                 (capi.TREEAH_BORROW_RAW if borrow_raw and raw is not None and space == capi.DEVICE else 0)
         self._raw_keep = k6 if flags & capi.TREEAH_BORROW_RAW else None
-        capi.check(capi.load().scann_treeah_create_ex(p_c, K, dim, p_cb, S, p_pk, p_id, p_off, n, p_raw, num_raw, stride,
-                                                      int(self.config.use_residuals),
-                                                      int(self.config.distance_measure), flags, self.device, space,
-                                                      C.byref(self._h)))
+        capi.check(create(p_c, K, dim, p_cb, S, p_pk, p_id, p_off, n, p_raw, num_raw, stride,
+                          int(self.config.use_residuals), int(self.config.distance_measure), flags, self.device, space,
+                          C.byref(self._h)))
         self.num_datapoints, self.dimensionality, self.num_partitions, self.num_subspaces = n, dim, K, S
         return self
 
