@@ -364,15 +364,24 @@ struct BfCore {
 
   // ---- legacy CUDA-core chunk (dim > 256, list overflow, SCANN_BF_NO_TC=1): steps 1-3 of the file header ----
   // qsrc: device queries [nqc][dim]; writes device outputs oid/od [nqc][k], oc [nqc]
+  // its carve: padded queries and norms of a query tile, the tile's scores against a row tile, the running top-kc
+  struct LegacyBufs {
+    float *Apad, *qn, *scores;
+    uint64_t* state;
+    uint32_t* cand;
+  };
+  size_t legacy_qtile(size_t nqc) const { return std::min<size_t>(kQTile, (nqc + kBM - 1) / kBM * kBM); }
+  LegacyBufs take_legacy(Workspace& w, size_t nqc, size_t kc) const {
+    const size_t qt = legacy_qtile(nqc), nt = std::min<size_t>(kNTile, n_pad);
+    return {w.take<float>(qt * dim_pad), w.take<float>(qt), w.take<float>(qt * nt), w.take<uint64_t>(qt * kc),
+            w.take<uint32_t>(qt * kc)};
+  }
   scann_status legacy_chunk(const float* qsrc, size_t nqc, size_t k, size_t kc, uint32_t* oid, float* od, uint32_t* oc,
                             cudaStream_t s) {
-    const size_t qt = std::min<size_t>(kQTile, (nqc + kBM - 1) / kBM * kBM);
+    const size_t qt = legacy_qtile(nqc);
     const size_t nt = std::min<size_t>(kNTile, n_pad);
-    float* Apad = ws.take<float>(qt * dim_pad);
-    float* qn = ws.take<float>(qt);
-    float* scores = ws.take<float>(qt * nt);
-    uint64_t* state = ws.take<uint64_t>(qt * kc);
-    uint32_t* cand = ws.take<uint32_t>(qt * kc);
+    const auto [Apad, qn, scores, state, cand] = take_legacy(ws, nqc, kc);
+    SCANN_TRY(ws.check("brute-force CUDA-core chunk"));
     const int p2 = next_pow2(static_cast<int>(kc));
     const size_t sel_smem = (kc + kBfChunk + p2) * 8 + 264 * 4;
     SCANN_CUDA(cudaFuncSetAttribute(bf_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -406,12 +415,6 @@ struct BfCore {
     ++stat_legacy_chunks;
     return SCANN_OK;
   }
-  size_t legacy_need(size_t nqc, size_t kc) const {
-    const size_t qt = std::min<size_t>(kQTile, (nqc + kBM - 1) / kBM * kBM);
-    const size_t nt = std::min<size_t>(kNTile, n_pad);
-    return Workspace::padded(qt * dim_pad * 4) + Workspace::padded(qt * 4) + Workspace::padded(qt * nt * 4) +
-           Workspace::padded(qt * kc * 8) + Workspace::padded(qt * kc * 4);
-  }
 
   RescoreParams rescore_params(const float* q) const {
     RescoreParams rp;
@@ -437,22 +440,25 @@ struct BfCore {
     const size_t tiles = tc_rows_pad(n) / 128, stride = tc_sample_stride();
     return (tiles + stride - 1) / stride;  // <= kTcSampleTiles; tile (tc_sample_tiles() - 1) * stride is the last one hit
   }
-  size_t tc_need(size_t nqc, size_t kk) const {
+  // the tensor-core carve: bf16 queries, norms, (sample) the threshold sample's scores, thresholds, lists and counts
+  struct TcBufs {
+    uint16_t* qbf;
+    float *qn, *dense, *thr;
+    uint32_t* cnt;
+    unsigned long long* lists;
+  };
+  TcBufs take_tc(Workspace& w, size_t nqc, bool sample) const {
     const size_t qpad = tc_queries_pad(nqc, dim);
-    return Workspace::padded(qpad * tc_kpad(dim) * 2) + Workspace::padded(qpad * 4) +
-           Workspace::padded(nqc * tc_sample_tiles() * 128 * 4) +
-           Workspace::padded(nqc * 4) * 2 + Workspace::padded(nqc * kTcCap * 8);
+    return {w.take<uint16_t>(qpad * tc_kpad(dim)), w.take<float>(qpad),
+            sample ? w.take<float>(nqc * tc_sample_tiles() * 128) : nullptr, w.take<float>(nqc), w.take<uint32_t>(nqc),
+            w.take<unsigned long long>(nqc * kTcCap)};
   }
   scann_status tc_chunk(const float* qsrc, size_t nqc, size_t k, size_t kk, uint32_t* oid, float* od, uint32_t* oc,
                         cudaStream_t s, bool* overflow) {
-    const size_t kpad = tc_kpad(dim), qpad = tc_queries_pad(nqc, dim), rpad = tc_rows_pad(n);
+    const size_t rpad = tc_rows_pad(n);
     const size_t tiles = rpad / 128, stiles = tc_sample_tiles(), scols = stiles * 128;
-    uint16_t* qbf = ws.take<uint16_t>(qpad * kpad);
-    float* qn = ws.take<float>(qpad);
-    float* dense = ws.take<float>(nqc * scols);
-    float* thr = ws.take<float>(nqc);
-    uint32_t* cnt = ws.take<uint32_t>(nqc);
-    unsigned long long* lists = ws.take<unsigned long long>(nqc * kTcCap);
+    const auto [qbf, qn, dense, thr, cnt, lists] = take_tc(ws, nqc, true);
+    SCANN_TRY(ws.check("brute-force tensor-core chunk"));
     uint32_t* flag = reinterpret_cast<uint32_t*>(d_small.p + 1);
     SCANN_TRY(tc_prepare_queries(qsrc, nqc, dim, i8 ? scale : 1.0f, qbf, qn, s));
     TcScoreParams p;
@@ -541,22 +547,20 @@ struct BfCore {
     SCANN_REQUIRE(tc, SCANN_UNIMPLEMENTED, "radius search runs on the tensor-core path (dim <= 256)");
     const size_t k = max_results;
     const size_t chunk = std::min<size_t>(kTcQTile, nq);
-    const size_t kpad = tc_kpad(dim), rpad = tc_rows_pad(n);
+    const size_t rpad = tc_rows_pad(n);
     const QueryOut outs[] = {{ids, k * 4}, {dists, k * 4}, {counts, 4}};
-    SCANN_TRY(ws.reserve(Workspace::padded(tc_queries_pad(chunk, dim) * kpad * 2) +
-                         Workspace::padded(tc_queries_pad(chunk, dim) * 4) + Workspace::padded(chunk * 4) * 2 +
-                         Workspace::padded(chunk * kTcCap * 8) + 4096 + staging_bytes(memspace, chunk, dim, outs)));
+    SCANN_TRY(ws.reserve(Workspace::count([&](Workspace& w) {
+      take_staging(w, memspace, chunk, dim, outs);
+      take_tc(w, chunk, false);
+    })));
     // the flag collects every chunk's truncation (the kernels only set bits); every chunk is finished before the
     // truncation is reported: all outputs are written
     uint32_t* flag = reinterpret_cast<uint32_t*>(d_small.p + 1);
     SCANN_CUDA(cudaMemsetAsync(flag, 0, 4, s));
     SCANN_TRY(run_query_chunks(ws, memspace, s, queries, nq, dim, chunk, outs,
                                [&](const float* qsrc, size_t, size_t nqc, void* const* o) -> scann_status {
-      uint16_t* qbf = ws.take<uint16_t>(tc_queries_pad(chunk, dim) * kpad);
-      float* qn = ws.take<float>(tc_queries_pad(chunk, dim));
-      float* thr = ws.take<float>(chunk);
-      uint32_t* cnt = ws.take<uint32_t>(chunk);
-      unsigned long long* lists = ws.take<unsigned long long>(chunk * kTcCap);
+      const auto [qbf, qn, dense, thr, cnt, lists] = take_tc(ws, nqc, false);
+      SCANN_TRY(ws.check("brute-force radius chunk"));
       SCANN_TRY(tc_prepare_queries(qsrc, nqc, dim, i8 ? scale : 1.0f, qbf, qn, s));
       bf_radius_thr_kernel<<<static_cast<unsigned>((nqc + 255) / 256), 256, 0, s>>>(qn, xmax2, radius, measure, nqc, i8 ? 1 : 0, thr);
       SCANN_CUDA(cudaMemsetAsync(cnt, 0, nqc * 4, s));
@@ -613,10 +617,12 @@ struct BfCore {
     const bool use_tc = tc && static_cast<double>(kk) * static_cast<double>(tc_rows_pad(n)) /
                                       static_cast<double>(tc_sample_tiles() * 128) <= kTcCap / 2;
     const size_t chunk = std::min<size_t>(use_tc ? kTcQTile : kQTile, nq);
-    size_t need = legacy_need(chunk, kc);
-    if (use_tc) need = std::max(need, tc_need(chunk, kk));
     const QueryOut outs[] = {{ids, k * 4}, {dists, k * 4}, {counts, 4}};
-    SCANN_TRY(ws.reserve(need + staging_bytes(memspace, chunk, dim, outs) + 4096));
+    // an overflowing tensor-core chunk is re-done by the legacy chunk in the same space
+    const size_t legacy = Workspace::count([&](Workspace& w) { take_legacy(w, chunk, kc); });
+    const size_t tcb = use_tc ? Workspace::count([&](Workspace& w) { take_tc(w, chunk, true); }) : 0;
+    SCANN_TRY(ws.reserve(Workspace::count([&](Workspace& w) { take_staging(w, memspace, chunk, dim, outs); }) +
+                         std::max(legacy, tcb)));
     return run_query_chunks(ws, memspace, s, queries, nq, dim, chunk, outs,
                             [&](const float* qsrc, size_t, size_t nqc, void* const* o) -> scann_status {
       uint32_t* oid = static_cast<uint32_t*>(o[0]);

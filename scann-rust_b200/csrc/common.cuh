@@ -82,25 +82,40 @@ struct CallScope {
   ~CallScope() { order.leave(s); }
 };
 
-// grow-only device arena; one per handle, guarded by the handle's mutex
+// Grow-only device arena; one per handle, guarded by the handle's mutex.  A list of buffers is one carve (a function
+// that only calls take), run by count() in counting mode (take returns nullptr) to size the reservation, then for real:
+// a take past the reservation returns nullptr, and check() after the carve reports it before any kernel runs.
 struct Workspace {
   char* base = nullptr;
   size_t cap = 0;
   size_t used = 0;
+  bool counting = false;
+  bool overflow = false;
   Workspace() = default;
   Workspace(const Workspace&) = delete;
   Workspace& operator=(const Workspace&) = delete;
   ~Workspace() { release(); }
   scann_status reserve(size_t bytes);
-  void reset() { used = 0; }
+  // bytes carve(Workspace&) takes
+  template <class Carve>
+  static size_t count(Carve carve) {
+    Workspace w;
+    w.counting = true;
+    carve(w);
+    return w.used;
+  }
   template <class T>
   T* take(size_t count) {
-    size_t bytes = (count * sizeof(T) + 255) & ~size_t(255);
-    T* p = reinterpret_cast<T*>(base + used);
+    const size_t bytes = (count * sizeof(T) + 255) & ~size_t(255);
+    if (!counting && bytes > cap - used) {
+      overflow = true;
+      return nullptr;
+    }
+    T* p = counting ? nullptr : reinterpret_cast<T*>(base + used);
     used += bytes;
     return p;
   }
-  static size_t padded(size_t bytes) { return (bytes + 255) & ~size_t(255); }
+  scann_status check(const char* carve) const;
   void release();
 };
 
@@ -165,29 +180,35 @@ struct QueryOut {
   size_t bytes;
 };
 
-// Workspace bytes run_query_chunks takes for staging: on SCANN_HOST the chunk's queries and every requested output.
+// The staging carve of run_query_chunks: on SCANN_HOST the chunk's queries and every requested output.
 template <size_t N>
-size_t staging_bytes(int memspace, size_t chunk, size_t dim, const QueryOut (&outs)[N]) {
-  if (memspace != SCANN_HOST) return 0;
-  size_t b = Workspace::padded(chunk * dim * sizeof(float));
-  for (const QueryOut& o : outs)
-    if (o.p) b += Workspace::padded(chunk * o.bytes);
-  return b;
+struct Staging {
+  float* q = nullptr;
+  void* out[N] = {};
+};
+template <size_t N>
+Staging<N> take_staging(Workspace& ws, int memspace, size_t chunk, size_t dim, const QueryOut (&outs)[N]) {
+  Staging<N> st;
+  if (memspace != SCANN_HOST) return st;
+  st.q = ws.take<float>(chunk * dim);
+  for (size_t i = 0; i < N; ++i)
+    if (outs[i].p) st.out[i] = ws.take<uint8_t>(chunk * outs[i].bytes);
+  return st;
 }
 
 // Runs a batch of nq queries [nq][dim] in chunks of at most `chunk` queries as
 //   run(const float* device_queries, size_t q0, size_t nqc, void* const* device_outs)  -> scann_status
 // where device_outs[i] is outs[i] of the chunk (NULL when not requested).  SCANN_DEVICE: the caller's arrays at q0;
-// nothing is copied or synchronised.  SCANN_HOST: staging buffers taken from `ws` once (reserve staging_bytes() for
-// them); per chunk one copy of the queries in, one copy of every requested output out, one stream synchronisation.
-// The workspace is reset to the mark above the staging before every chunk: run takes its scratch from there.
+// nothing is copied or synchronised.  SCANN_HOST: staging buffers taken from `ws` once (the reservation counts
+// take_staging); per chunk one copy of the queries in, one copy of every requested output out, one stream
+// synchronisation.  The workspace is reset to the mark above the staging before every chunk: run takes its scratch
+// from there.
 template <size_t N, class Run>
 scann_status run_query_chunks(Workspace& ws, int memspace, cudaStream_t s, const float* queries, size_t nq, size_t dim,
                               size_t chunk, const QueryOut (&outs)[N], Run run) {
   const bool host = memspace == SCANN_HOST;
-  float* hq = host ? ws.take<float>(chunk * dim) : nullptr;
-  void* stage[N];
-  for (size_t i = 0; i < N; ++i) stage[i] = host && outs[i].p ? ws.take<uint8_t>(chunk * outs[i].bytes) : nullptr;
+  const Staging<N> st = take_staging(ws, memspace, chunk, dim, outs);
+  SCANN_TRY(ws.check("query staging"));
   const size_t mark = ws.used;
   for (size_t q0 = 0; q0 < nq; q0 += chunk) {
     const size_t nqc = nq - q0 < chunk ? nq - q0 : chunk;
@@ -198,11 +219,11 @@ scann_status run_query_chunks(Workspace& ws, int memspace, cudaStream_t s, const
       SCANN_TRY(run(queries + q0 * dim, q0, nqc, dout));
       continue;
     }
-    SCANN_CUDA(cudaMemcpyAsync(hq, queries + q0 * dim, nqc * dim * sizeof(float), cudaMemcpyHostToDevice, s));
-    SCANN_TRY(run(static_cast<const float*>(hq), q0, nqc, stage));
+    SCANN_CUDA(cudaMemcpyAsync(st.q, queries + q0 * dim, nqc * dim * sizeof(float), cudaMemcpyHostToDevice, s));
+    SCANN_TRY(run(static_cast<const float*>(st.q), q0, nqc, st.out));
     for (size_t i = 0; i < N; ++i)
       if (outs[i].p)
-        SCANN_CUDA(cudaMemcpyAsync(static_cast<char*>(outs[i].p) + q0 * outs[i].bytes, stage[i], nqc * outs[i].bytes,
+        SCANN_CUDA(cudaMemcpyAsync(static_cast<char*>(outs[i].p) + q0 * outs[i].bytes, st.out[i], nqc * outs[i].bytes,
                                    cudaMemcpyDeviceToHost, s));
     SCANN_CUDA(cudaStreamSynchronize(s));
   }

@@ -335,10 +335,13 @@ scann_status scann_ivf_search(scann_ivf* h, int mode, const float* queries, size
   const size_t K = h->K;
   if (L > K) L = K;
   size_t chunk = std::min(nq, std::max<size_t>(1, (size_t(256) << 20) / (K * 4)));
-  const size_t scr = h->part.scratch_bytes(chunk);
   const QueryOut outs[] = {{ids, k * 4}, {dists, k * 4}, {counts, 4}};
-  SCANN_TRY(h->ws.reserve(Workspace::padded(scr) + Workspace::padded(chunk * L * 4) + 4096 +
-                          staging_bytes(memspace, chunk, h->dim, outs)));
+  auto take_tokens = [&](Workspace& w) { return w.take<uint32_t>(chunk * L); };
+  SCANN_TRY(h->ws.reserve(Workspace::count([&](Workspace& w) {
+    take_staging(w, memspace, chunk, h->dim, outs);
+    take_tokens(w);
+    h->part.take_scratch(w, chunk);
+  })));
   const int p2 = next_pow2(static_cast<int>(k));
   const size_t smem = (k + kIvfChunk + p2) * 8 + 264 * 4 + (L + 1) * 4 + ((h->dim + 3) & ~size_t(3)) * 4 +
                       (mode == 1 ? h->S * h->C * 4 : 0) + 16;
@@ -346,9 +349,9 @@ scann_status scann_ivf_search(scann_ivf* h, int mode, const float* queries, size
   SCANN_CUDA(cudaFuncSetAttribute(ivf_topk_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
   return run_query_chunks(h->ws, memspace, call.s, queries, nq, h->dim, chunk, outs,
                           [&](const float* dq, size_t, size_t nqc, void* const* o) -> scann_status {
-                            void* scratch = h->ws.take<uint8_t>(scr);
-                            uint32_t* tokens = h->ws.take<uint32_t>(chunk * L);
-                            SCANN_TRY(h->part.select(dq, nqc, L, tokens, nullptr, scratch, call.s));
+                            uint32_t* tokens = take_tokens(h->ws);
+                            SCANN_TRY(h->ws.check("IVF tokens"));
+                            SCANN_TRY(h->part.select(dq, nqc, L, tokens, nullptr, h->ws, call.s));
                             IvfArgs a;
                             a.tokens = tokens;
                             a.pt_off = h->pt_off.p;

@@ -19,10 +19,14 @@ class CentreScorer {
  public:
   // (re)loads the centres [K][dim] and derives the scoring operands; synchronises s
   scann_status set(const float* centers, size_t K, size_t dim, int memspace, cudaStream_t s);
-  // device scratch select() needs for a batch of nq queries
-  size_t scratch_bytes(size_t nq) const;
-  // tokens [nq][L] (0xFFFFFFFF past min(L, K)), dists [nq][L] or null; all device pointers
-  scann_status select(const float* queries, size_t nq, size_t L, uint32_t* tokens, float* dists, void* scratch,
+  // the scratch select() takes for nq queries: (tensor cores) bf16 queries and norms, the score of every centre
+  struct Scratch {
+    uint16_t* qbf = nullptr;
+    float *qn = nullptr, *scores = nullptr;
+  };
+  Scratch take_scratch(Workspace& ws, size_t nq) const;
+  // tokens [nq][L] (0xFFFFFFFF past min(L, K)), dists [nq][L] or null; all device pointers.  Takes its scratch from ws.
+  scann_status select(const float* queries, size_t nq, size_t L, uint32_t* tokens, float* dists, Workspace& ws,
                       cudaStream_t s) const;
   const float* centers() const { return centers_.p; }  // device [K][dim] f32
   int launches() const { return tc_.ready ? 3 : 2; }    // kernels one select() enqueues

@@ -455,7 +455,11 @@ scann_status scann_kmtree_search_leaves(scann_kmtree* h, const float* queries, s
   const size_t per_q = static_cast<size_t>(h->levels) * h->max_children * 8;
   size_t chunk = std::min(nq, std::max<size_t>(1, (size_t(256) << 20) / per_q));
   const QueryOut outs[] = {{leaf_nodes, k * 4}, {dists, k * 4}, {depths, k * 4}, {counts, 4}};
-  SCANN_TRY(h->ws.reserve(Workspace::padded(chunk * per_q) + staging_bytes(memspace, chunk, h->dim, outs)));
+  auto take_scratch = [&](Workspace& w) { return w.take<unsigned long long>(chunk * per_q / 8); };
+  SCANN_TRY(h->ws.reserve(Workspace::count([&](Workspace& w) {
+    take_staging(w, memspace, chunk, h->dim, outs);
+    take_scratch(w);
+  })));
   TreeArgs t{h->centers.p, h->depth.p, h->child_begin.p, h->child_count.p, h->children.p, static_cast<int>(h->dim),
              h->max_children, h->levels};
   int mc2 = 1;
@@ -469,7 +473,8 @@ scann_status scann_kmtree_search_leaves(scann_kmtree* h, const float* queries, s
     SCANN_CUDA(cudaFuncSetAttribute(kmtree_search_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
   return run_query_chunks(h->ws, memspace, call.s, queries, nq, h->dim, chunk, outs,
                           [&](const float* q, size_t, size_t nqc, void* const* o) -> scann_status {
-                            unsigned long long* scratch = h->ws.take<unsigned long long>(chunk * per_q / 8);
+                            unsigned long long* scratch = take_scratch(h->ws);
+                            SCANN_TRY(h->ws.check("k-means tree search"));
                             kmtree_search_kernel<<<static_cast<unsigned>(nqc), 32, smem, call.s>>>(
                                 t, q, static_cast<int>(nqc), static_cast<int>(k), scratch, static_cast<uint32_t*>(o[0]),
                                 static_cast<float*>(o[1]), static_cast<uint32_t*>(o[2]), static_cast<uint32_t*>(o[3]));

@@ -236,11 +236,6 @@ static bool part_tc_usable(size_t K, size_t dim) {
   return tc_supported(dim) && K >= 256;  // small K: the exact kernel alone is cheaper than the extra launches
 }
 
-static size_t part_tc_scratch_bytes(size_t K, size_t dim, size_t nq) {
-  return Workspace::padded(tc_queries_pad(nq, dim) * tc_kpad(dim) * 2) + Workspace::padded(tc_queries_pad(nq, dim) * 4) +
-         Workspace::padded(nq * tc_rows_pad(K) * 4) + 1024;
-}
-
 static scann_status part_tc_prepare(const float* centers, size_t K, size_t dim, PartTc* out, cudaStream_t s) {
   const size_t kpad = tc_kpad(dim), rpad = tc_rows_pad(K);
   if (out->cbf.n != rpad * kpad) SCANN_TRY(out->cbf.alloc(rpad * kpad));  // kept across CentreScorer::set
@@ -253,18 +248,13 @@ static scann_status part_tc_prepare(const float* centers, size_t K, size_t dim, 
   return SCANN_OK;
 }
 
+// scratch (CentreScorer::take_scratch): the bf16 queries, their norms and the dense scores [nq][rpad]
 static scann_status launch_partition_tc(const PartTc& tc, const float* centers, size_t K, size_t dim,
                                         const float* queries, size_t nq, size_t L, uint32_t* tokens, float* dists,
-                                        void* scratch, int sms, cudaStream_t s) {
+                                        uint16_t* qbf, float* qn, float* dense, int sms, cudaStream_t s) {
   if (nq == 0 || L == 0) return SCANN_OK;
   SCANN_REQUIRE(L <= 1024, SCANN_INVALID_ARGUMENT, "partitions_to_search %zu > 1024 unsupported", L);
-  const size_t kpad = tc_kpad(dim), rpad = tc_rows_pad(K), qpad = tc_queries_pad(nq, dim);
-  uint8_t* p = static_cast<uint8_t*>(scratch);
-  uint16_t* qbf = reinterpret_cast<uint16_t*>(p);
-  p += Workspace::padded(qpad * kpad * 2);
-  float* qn = reinterpret_cast<float*>(p);
-  p += Workspace::padded(qpad * 4);
-  float* dense = reinterpret_cast<float*>(p);
+  const size_t rpad = tc_rows_pad(K);
   SCANN_TRY(tc_prepare_queries(queries, nq, dim, 1.0f, qbf, qn, s));
   TcScoreParams sp;
   sp.q_bf16 = qbf;
@@ -371,14 +361,25 @@ scann_status CentreScorer::set(const float* centers, size_t K, size_t dim, int m
   return SCANN_OK;
 }
 
-size_t CentreScorer::scratch_bytes(size_t nq) const {
-  return std::max(nq * K_ * sizeof(float), tc_.ready ? part_tc_scratch_bytes(K_, dim_, nq) : size_t(0));
+CentreScorer::Scratch CentreScorer::take_scratch(Workspace& ws, size_t nq) const {
+  Scratch sc;
+  if (tc_.ready) {
+    const size_t qpad = tc_queries_pad(nq, dim_);
+    sc.qbf = ws.take<uint16_t>(qpad * tc_kpad(dim_));
+    sc.qn = ws.take<float>(qpad);
+  }
+  sc.scores = ws.take<float>(nq * (tc_.ready ? tc_rows_pad(K_) : K_));
+  return sc;
 }
 
 scann_status CentreScorer::select(const float* queries, size_t nq, size_t L, uint32_t* tokens, float* dists,
-                                  void* scratch, cudaStream_t s) const {
-  if (tc_.ready) return launch_partition_tc(tc_, centers_.p, K_, dim_, queries, nq, L, tokens, dists, scratch, sms_, s);
-  return launch_partition(centersT_.p, K_, dim_, queries, nq, L, tokens, dists, static_cast<float*>(scratch), s);
+                                  Workspace& ws, cudaStream_t s) const {
+  const Scratch sc = take_scratch(ws, nq);
+  SCANN_TRY(ws.check("partition"));
+  if (tc_.ready)
+    return launch_partition_tc(tc_, centers_.p, K_, dim_, queries, nq, L, tokens, dists, sc.qbf, sc.qn, sc.scores, sms_,
+                               s);
+  return launch_partition(centersT_.p, K_, dim_, queries, nq, L, tokens, dists, sc.scores, s);
 }
 
 }  // namespace scann
@@ -450,13 +451,15 @@ scann_status scann_part_select(scann_part* h, const float* queries, size_t nq, s
   size_t chunk = (size_t(2) << 30) / (h->K * sizeof(float));  // dense score scratch: 2 GiB keeps >= 8192 rows per pass at K = 65,536
   if (chunk < 1) chunk = 1;
   if (chunk > nq) chunk = nq;
-  const size_t scratch_bytes = h->scorer.scratch_bytes(chunk);
   const QueryOut outs[] = {{tokens, L * sizeof(uint32_t)}, {dists, L * sizeof(float)}};
-  SCANN_TRY(h->ws.reserve(Workspace::padded(scratch_bytes) + staging_bytes(memspace, chunk, h->dim, outs)));
+  SCANN_TRY(h->ws.reserve(Workspace::count([&](Workspace& w) {
+    take_staging(w, memspace, chunk, h->dim, outs);
+    h->scorer.take_scratch(w, chunk);
+  })));
   return run_query_chunks(h->ws, memspace, call.s, queries, nq, h->dim, chunk, outs,
                           [&](const float* q, size_t, size_t nqc, void* const* o) {
                             return h->scorer.select(q, nqc, L, static_cast<uint32_t*>(o[0]), static_cast<float*>(o[1]),
-                                                    h->ws.take<uint8_t>(scratch_bytes), call.s);
+                                                    h->ws, call.s);
                           });
 }
 

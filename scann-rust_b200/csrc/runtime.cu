@@ -61,22 +61,22 @@ int scan_acc_mode(int S) {
 
 scann_status Workspace::reserve(size_t bytes) {
   used = 0;
+  overflow = false;
   if (bytes <= cap) return SCANN_OK;
   if (base) cudaFree(base);
   base = nullptr;
   cap = 0;
-  size_t want = bytes + bytes / 8 + (1u << 20);
-  cudaError_t e = cudaMalloc(reinterpret_cast<void**>(&base), want);
-  if (e != cudaSuccess) {
-    cudaGetLastError();
-    want = bytes;
-    e = cudaMalloc(reinterpret_cast<void**>(&base), want);
-  }
+  cudaError_t e = cudaMalloc(reinterpret_cast<void**>(&base), bytes);
   if (e != cudaSuccess) {
     base = nullptr;
     return cuda_fail(e, "workspace cudaMalloc", __FILE__, __LINE__);
   }
-  cap = want;
+  cap = bytes;
+  return SCANN_OK;
+}
+
+scann_status Workspace::check(const char* carve) const {
+  SCANN_REQUIRE(!overflow, SCANN_INTERNAL, "workspace: the %s carve exceeds its reservation of %zu bytes", carve, cap);
   return SCANN_OK;
 }
 

@@ -9,8 +9,9 @@
 // the tensor pipe idle; here a 128-point x 128-query tile costs 24 (S = 48) tcgen05.mma instructions of 64 cycles.
 //
 // Per batch (launch_tc_scan, after the probe of every query's closest leaf has produced the bounds tau_q):
-//   tcwl_*           pairs (query, rank) grouped BY LEAF; a group = one leaf + up to 128 of its pairs; an item = one
-//                    group x a run of <= 32 point tiles (128 points each) of the leaf
+//   tcwl_*           the caller's class-B lists (pairs (query, rank >= T) grouped BY LEAF, treeah.cu) cut into groups and
+//                    items: a group = one leaf + up to 128 of its pairs; an item = one group x a run of <= 32 point tiles
+//                    (128 points each) of the leaf
 //   tc_lut_kernel    one warp per (group, pair): residual LUT16 table (bit-exact quantiser, lut16_device.cuh) written as
 //                    one K-major u8 row of the group's LUT tile, followed by two "threshold digits" (below)
 //   tc_scan_kernel   persistent, one CTA per SM, warp-specialised:
@@ -219,15 +220,6 @@ __device__ __forceinline__ int score_bound_from_tau(float tau, float mult, float
 }
 
 // ------------------------------------------------------------------------------------------------ worklist
-// pairs of rank < T (the query's T closest leaves) are not part of this scan: the register-LUT kernel has scanned them
-__global__ void tcwl_count_kernel(const uint32_t* __restrict__ tokens, size_t P, uint32_t K, uint32_t L, uint32_t T,
-                                  const uint64_t* __restrict__ pt_off, uint32_t* __restrict__ leaf_cnt) {
-  const size_t p = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (p >= P || static_cast<uint32_t>(p) % L < T) return;  // 32-bit: see wl_virtual_leaf (treeah.cu)
-  const uint32_t leaf = tokens[p];
-  if (leaf < K && pt_off[leaf + 1] > pt_off[leaf]) atomicAdd(&leaf_cnt[leaf], 1u);
-}
-
 __device__ __forceinline__ void tcwl_entry(uint32_t leaf, const uint32_t* __restrict__ leaf_cnt,
                                            const uint64_t* __restrict__ pt_off, uint32_t& pc, uint32_t& groups,
                                            uint32_t& chunks) {
@@ -295,16 +287,6 @@ __global__ void __launch_bounds__(1024) tcwl_scan_kernel(const uint32_t* __restr
     counters[1] = s_g[1023];
     counters[2] = 0;  // protocol-error counter of the scan
   }
-}
-
-__global__ void tcwl_scatter_kernel(const uint32_t* __restrict__ tokens, size_t P, uint32_t K, uint32_t L, uint32_t T,
-                                    const uint64_t* __restrict__ pt_off, const uint32_t* __restrict__ pair_start,
-                                    uint32_t* __restrict__ cursor, uint32_t* __restrict__ sorted_pairs) {
-  const size_t p = static_cast<size_t>(blockIdx.x) * blockDim.x + threadIdx.x;
-  if (p >= P || static_cast<uint32_t>(p) % L < T) return;  // 32-bit: see wl_virtual_leaf (treeah.cu)
-  const uint32_t leaf = tokens[p];
-  if (leaf < K && pt_off[leaf + 1] > pt_off[leaf])
-    sorted_pairs[pair_start[leaf] + atomicAdd(&cursor[leaf], 1u)] = static_cast<uint32_t>(p);
 }
 
 // groups[g] = {leaf, first sorted pair, pairs in the group, 0}; items[i] = {group, first tile, end tile, leaf}
@@ -845,43 +827,30 @@ size_t tc_scan_max_items(size_t P, size_t K, size_t max_leaf) {
   return tc_scan_max_groups(P, K) * std::max<size_t>(1, (tiles + kTcsItemTiles - 1) / kTcsItemTiles);
 }
 
-size_t tc_scan_workspace_bytes(size_t nq, size_t L, size_t K, size_t S, size_t max_leaf, size_t qcap) {
+TcScanBufs take_tc_scan(Workspace& ws, size_t nq, size_t L, size_t K, size_t S, size_t max_leaf, size_t qcap) {
   const size_t P = nq * L, G = tc_scan_max_groups(P, K);
-  size_t b = 0;
-  auto add = [&](size_t bytes) { b += Workspace::padded(bytes); };
-  add(2 * K * 4);                       // leaf_cnt + cursor
-  add(3 * (K + 1) * 4);                 // pair / group / item starts
-  add(16);                              // counters
-  add(P * 4);                           // sorted pairs
-  add(G * 16);                          // groups
-  add(tc_scan_max_items(P, K, max_leaf) * 16);
-  add(G * kTcsGroup * (S * 16 + 32));   // LUT tiles
-  add(G * kTcsGroup * 16);              // meta
-  add(nq * qcap * 8);                   // candidate lists
-  add(nq * 4);                          // counts
-  add(nq * 4);                          // flags
-  add(P * 4);                           // masked tokens
-  return b + 4096;
+  TcScanBufs b;
+  b.starts = ws.take<uint32_t>(3 * (K + 1));
+  b.counters = ws.take<uint32_t>(4);
+  b.groups = ws.take<uint4>(G);
+  b.items = ws.take<uint4>(tc_scan_max_items(P, K, max_leaf));
+  b.lut = ws.take<uint8_t>(G * kTcsGroup * (S * 16 + 32));
+  b.meta = ws.take<uint4>(G * kTcsGroup);
+  b.qcand = ws.take<unsigned long long>(nq * qcap);
+  b.qcnt = ws.take<uint32_t>(nq);
+  b.qflag = ws.take<uint32_t>(nq);
+  b.fb_tokens = ws.take<uint32_t>(P);
+  return b;
 }
 
 scann_status launch_tc_scan(const TcScanParams& p, Workspace& ws, TcScanOut* out, cudaStream_t s) {
   const size_t K = p.K, P = p.nq * p.L, S = p.S;
-  const size_t G = tc_scan_max_groups(P, K), I = tc_scan_max_items(P, K, p.max_leaf);
+  const size_t G = tc_scan_max_groups(P, K);
   const int row_bytes = static_cast<int>(S * 16 + 32);
-  uint32_t* leaf_cnt = ws.take<uint32_t>(2 * K);
-  uint32_t* cursor = leaf_cnt + K;
-  uint32_t* starts = ws.take<uint32_t>(3 * (K + 1));
+  const auto [starts, counters, groups, items, meta, lut, qcand, qcnt, qflag, fb_tokens] =
+      take_tc_scan(ws, p.nq, p.L, K, S, p.max_leaf, p.qcap);
+  SCANN_TRY(ws.check("tensor-core scan"));
   uint32_t *pair_start = starts, *group_start = starts + (K + 1), *item_start = starts + 2 * (K + 1);
-  uint32_t* counters = ws.take<uint32_t>(4);
-  uint32_t* sorted_pairs = ws.take<uint32_t>(P);
-  uint4* groups = ws.take<uint4>(G);
-  uint4* items = ws.take<uint4>(I);
-  uint8_t* lut = ws.take<uint8_t>(G * kTcsGroup * row_bytes);
-  uint4* meta = ws.take<uint4>(G * kTcsGroup);
-  unsigned long long* qcand = ws.take<unsigned long long>(p.nq * p.qcap);
-  uint32_t* qcnt = ws.take<uint32_t>(p.nq);
-  uint32_t* qflag = ws.take<uint32_t>(p.nq);
-  uint32_t* fb_tokens = ws.take<uint32_t>(P);
 
   const char* dbg_env = getenv("SCANN_TC_DEBUG");
   const bool dbg = dbg_env && dbg_env[0] == '1';
@@ -892,34 +861,19 @@ scann_status launch_tc_scan(const TcScanParams& p, Workspace& ws, TcScanOut* out
   SCANN_CUDA(cudaMemsetAsync(qcnt, 0, p.nq * 4, s));
   SCANN_CUDA(cudaMemsetAsync(qflag, 0, p.nq * 4, s));
   const unsigned pb = static_cast<unsigned>((P + 255) / 256);
-  // The count and scatter passes are atomics on 4-byte counters (8 per 32-byte sector: ~1300 serialised updates per
-  // sector at C3, 0.09 ms each).  The caller's worklist has usually grouped the same pairs already (class B of
-  // treeah.cu's build_worklist): then only the group / item tables are built here.
-  const bool reuse = p.wl_cnt != nullptr && p.wl_pair_start != nullptr && p.wl_sorted_pairs != nullptr;
-  const uint32_t* cnt_in = leaf_cnt;
-  const uint32_t* pairs_in = sorted_pairs;
-  if (reuse) {
-    cnt_in = p.wl_cnt;
-    pairs_in = p.wl_sorted_pairs;
-  } else {
-    SCANN_CUDA(cudaMemsetAsync(leaf_cnt, 0, 2 * K * 4, s));
-    tcwl_count_kernel<<<pb, 256, 0, s>>>(p.tokens, P, static_cast<uint32_t>(K), static_cast<uint32_t>(p.L),
-                                         static_cast<uint32_t>(p.T), p.pt_off, leaf_cnt);
-  }
-  tcwl_scan_kernel<<<1, 1024, 0, s>>>(cnt_in, static_cast<uint32_t>(K), p.leaf_perm, p.pt_off, pair_start, group_start,
-                                      item_start, counters, p.pair_points);
-  if (!reuse)
-    tcwl_scatter_kernel<<<pb, 256, 0, s>>>(p.tokens, P, static_cast<uint32_t>(K), static_cast<uint32_t>(p.L),
-                                           static_cast<uint32_t>(p.T), p.pt_off, pair_start, cursor, sorted_pairs);
-  tcwl_items_kernel<<<static_cast<unsigned>((K + 127) / 128), 128, 0, s>>>(cnt_in, static_cast<uint32_t>(K), p.pt_off,
-                                                                          reuse ? p.wl_pair_start : pair_start,
-                                                                          group_start, item_start, groups, items);
+  // the pairs come grouped by leaf from the caller's worklist (class B of treeah.cu's treeah_worklist): only the group
+  // and item tables are built here (tcwl_scan_kernel also writes pair starts of its own, which nothing reads)
+  tcwl_scan_kernel<<<1, 1024, 0, s>>>(p.wl_cnt, static_cast<uint32_t>(K), p.leaf_perm, p.pt_off, pair_start,
+                                      group_start, item_start, counters, p.pair_points);
+  tcwl_items_kernel<<<static_cast<unsigned>((K + 127) / 128), 128, 0, s>>>(p.wl_cnt, static_cast<uint32_t>(K), p.pt_off,
+                                                                          p.wl_pair_start, group_start, item_start,
+                                                                          groups, items);
   if (dbg) cudaEventRecord(ev[1], s);
   if (p.ev[0]) cudaEventRecord(p.ev[0], s);
   LutArgs la;
   la.groups = groups;
   la.counters = counters;
-  la.sorted_pairs = pairs_in;
+  la.sorted_pairs = p.wl_sorted_pairs;
   la.queries = p.queries;
   la.centers = p.centers;
   la.codebook = p.codebook;
@@ -1029,7 +983,6 @@ scann_status launch_tc_scan(const TcScanParams& p, Workspace& ws, TcScanOut* out
   out->qcnt = qcnt;
   out->qflag = qflag;
   out->fb_tokens = fb_tokens;
-  out->launches = reuse ? 5 : 7;  // kernels of this function (memsets are not counted)
   return SCANN_OK;
 }
 

@@ -26,11 +26,10 @@ struct TcScanParams {
   int sms;
   cudaEvent_t ev[3] = {nullptr, nullptr, nullptr};  // optional: recorded before the LUT kernel, before and after the scan
   unsigned long long* pair_points = nullptr;        // optional: += Σ over scanned (pair, leaf) of leaf size
-  // optional: the per-leaf lists of the pairs of rank >= T that the caller's own worklist has already built
-  // (treeah.cu build_worklist counts and scatters them as class B): saves this scan its count + scatter passes
-  const uint32_t* wl_cnt = nullptr;          // [K] pairs of rank >= T per leaf
-  const uint32_t* wl_pair_start = nullptr;   // [K] first entry of the leaf's list in wl_sorted_pairs
-  const uint32_t* wl_sorted_pairs = nullptr; // pair indices (q * L + rank), grouped by leaf
+  // the per-leaf lists of the pairs of rank >= T, class B of the caller's worklist (treeah.cu treeah_worklist)
+  const uint32_t* wl_cnt;                    // [K] pairs of rank >= T per leaf
+  const uint32_t* wl_pair_start;             // [K] first entry of the leaf's list in wl_sorted_pairs
+  const uint32_t* wl_sorted_pairs;           // pair indices (q * L + rank), grouped by leaf
   // optional restrict filters (ScanArgs::allow of lut16_scan_kernel.cuh): a survivor its query's filter row does not
   // allow is dropped before it takes a list slot
   const uint8_t* allow = nullptr;            // [num_filters][allow_stride] one byte per (256-point block, lane)
@@ -45,11 +44,22 @@ struct TcScanOut {
   const uint32_t* qcnt;             // [nq] appended (may exceed qcap)
   const uint32_t* qflag;            // [nq] 1 = no bound or overflow: the register-LUT kernel re-does the query
   const uint32_t* fb_tokens;        // [nq][L] tokens of the flagged queries, 0xFFFFFFFF elsewhere
-  int launches;
+};
+constexpr int kTcScanLaunches = 5;  // kernels one launch_tc_scan enqueues (memsets are not counted)
+
+// The workspace carve of launch_tc_scan for nq queries x L ranks (qcap = TcScanParams::qcap): group / item tables, LUT
+// tiles and the outputs of TcScanOut
+struct TcScanBufs {
+  uint32_t* starts;  // pair / group / item start of every leaf
+  uint32_t* counters;
+  uint4 *groups, *items, *meta;
+  uint8_t* lut;
+  unsigned long long* qcand;
+  uint32_t *qcnt, *qflag, *fb_tokens;
 };
 
 bool tc_scan_supported(size_t S, size_t dim);
-size_t tc_scan_workspace_bytes(size_t nq, size_t L, size_t K, size_t S, size_t max_leaf, size_t qcap);
+TcScanBufs take_tc_scan(Workspace& ws, size_t nq, size_t L, size_t K, size_t S, size_t max_leaf, size_t qcap);
 scann_status launch_tc_scan(const TcScanParams& p, Workspace& ws, TcScanOut* out, cudaStream_t s);
 scann_status tc_make_map_u8(void* map, const void* base, size_t rows, size_t row_bytes);  // tc_gemm.cu
 

@@ -589,11 +589,15 @@ struct scann_treeah {
   scann::StreamOrder order;  // device work of successive calls, across streams
   cudaStream_t stream = nullptr;
   int sms = 148;
-  // the chunk being searched, between its two phases (treeah_phase1 / treeah_phase2)
+  // the chunk being searched, between its two phases (treeah_phase1 / treeah_phase2): treeah_plan, treeah_take_chunk
   struct Chunk {
     const float* dq = nullptr;
     size_t nq = 0, L = 0, R = 0, k = 0;
-    int G = 8;
+    int G = 8;              // queries per register-LUT work item
+    bool use_tc = false;    // probe + tensor-core scan of the other ranks
+    int T = 1;              // ranks in class A of the worklist
+    bool partition = true;  // the chunk partitions its queries (else the caller passed the tokens)
+    bool params = false;    // per-query R / k (scann_treeah_search_with_params)
     uint32_t *tokens = nullptr, *counters = nullptr, *cand_cnt = nullptr, *qthr = nullptr;
     uint2* cand = nullptr;
     // worklist buffers (rebuilt over the flagged queries' tokens after a tensor-core scan)
@@ -601,9 +605,7 @@ struct scann_treeah {
              *wl_blk_item = nullptr, *sorted_pairs = nullptr;
     unsigned long long* wl_blk_bytes = nullptr;
     uint4* items = nullptr;
-    bool use_tc = false;
-    int T = 1;  // ranks in class A of the worklist
-    const uint32_t *qR = nullptr, *qk = nullptr;  // per-query R / k (scann_treeah_search_with_params), else nullptr
+    uint32_t *qR = nullptr, *qk = nullptr;  // per-query R / k when params, else nullptr
     scann::ScanArgs a;
   } ck;
   bool split_active = false;  // between scann_treeah_search_begin and _end / _abort: other entry points are refused
@@ -786,13 +788,12 @@ static scann_status treeah_worklist(scann_treeah* h, const uint32_t* tokens, siz
 // candidate list capacity per query of the tensor-core scan
 static size_t tc_qcap(size_t R) { return std::min<size_t>(16384, std::max<size_t>(2048, 64 * R)); }
 
-// tensor-core scan for this chunk?  SCANN_SCAN_TC=0 never, =1 whenever the index supports it, default: when a leaf is
-// probed by enough queries of the batch to fill the 128-wide query tiles
-static bool treeah_use_tc(const scann_treeah* h, size_t nq, size_t L, size_t R) {
+// tensor-core scan for this chunk?  tc_env = SCANN_SCAN_TC, read once per call: 0 never, 1 whenever the index supports
+// it, default: when a leaf is probed by enough queries of the batch to fill the 128-wide query tiles
+static bool treeah_use_tc(const scann_treeah* h, size_t nq, size_t L, size_t R, const char* tc_env) {
   if (!h->tc_ok || h->packed_rm.p == nullptr || L > 1024 || R < 1) return false;
-  const char* e = getenv("SCANN_SCAN_TC");
-  if (e && e[0] == '0') return false;
-  if (e && e[0] == '1') return true;
+  if (tc_env && tc_env[0] == '0') return false;
+  if (tc_env && tc_env[0] == '1') return true;
   const size_t P = nq * L;
   return static_cast<double>(P) / static_cast<double>(std::min<size_t>(h->K, P)) >= 12.0;
 }
@@ -831,94 +832,113 @@ static ChunkFilter handle_filter(const scann_treeah* h) {
 struct ChunkParams {
   const uint32_t *L = nullptr, *R = nullptr, *k = nullptr;
   size_t L_call = 0;
-  bool any() const { return L || R || k; }
 };
 
-// Phase 1 of a chunk: partition -> worklist -> (two_phase: scan of the class-A items, i.e. every query's closest leaf
-// on this shard; tau_out receives the bounds they prove).  State for phase 2 stays in h->ck / the workspace.
-static scann_status treeah_phase1(scann_treeah* h, const float* dq, size_t nq, size_t L, size_t R, size_t k,
-                                  bool two_phase, float* tau_out, const uint32_t* tokens_in, const ChunkFilter& filt,
-                                  const ChunkParams& cp, cudaStream_t s) {
-  const size_t K = h->K, P = nq * L;
+// The decisions a chunk of nq queries runs with, written into ck; the counting pass of the reservation and the run
+// both take them from here.  partition: the chunk partitions its queries (else the caller passed tokens); filtered: a
+// restrict filter applies; params: per-query R / k.
+static void treeah_plan(const scann_treeah* h, size_t nq, size_t L, size_t R, const char* tc_env, bool partition,
+                        bool filtered, bool params, scann_treeah::Chunk& ck) {
+  const size_t P = nq * L;
   // group size: how many queries share a leaf on average
-  double avg = static_cast<double>(P) / static_cast<double>(std::min<size_t>(K, P));
+  const double avg = static_cast<double>(P) / static_cast<double>(std::min<size_t>(h->K, P));
   int G = avg >= 6.0 ? 8 : (avg >= 3.0 ? 4 : (avg >= 1.5 ? 2 : 1));
   // the scan CTA holds G queries' residuals, tables and candidate buffers: smaller groups where they do not fit (each
   // pair's per-leaf top-R does not depend on which queries share its item, so results stay the same)
   const int cap = scan_list_cap(static_cast<int>(R), kScanWarps);
-  while (G > 1 && scan_cta_bytes(h, G, cap, filt.allow != nullptr) > kScanSmemMax) G /= 2;
-  size_t max_items = P / G + 2 * std::min<size_t>(K, P) + 1;
+  while (G > 1 && scan_cta_bytes(h, G, cap, filtered) > kScanSmemMax) G /= 2;
+  ck.nq = nq;
+  ck.L = L;
+  ck.R = R;
+  ck.G = G;
+  ck.use_tc = treeah_use_tc(h, nq, L, R, tc_env);  // then the chunk runs in two phases: the probe gives the bounds
+  ck.T = ck.use_tc ? static_cast<int>(tc_ranks(L)) : 1;
+  ck.partition = partition;
+  ck.params = params;
+}
 
-  // centre-score scratch of the partition stage (not needed when the caller partitioned)
-  void* scratch = tokens_in ? nullptr : h->ws.take<uint8_t>(h->part.scratch_bytes(nq));
-  uint32_t* tokens = h->ws.take<uint32_t>(P);
-  if (tokens_in) tokens = const_cast<uint32_t*>(tokens_in);  // the caller partitioned (and keeps the array alive)
-  uint32_t* leaf_cnt = h->ws.take<uint32_t>(2 * K + 4 * K * kWlPad);  // counts of the 2K virtual leaves + padded counters / cursors
-  uint32_t* pair_start = h->ws.take<uint32_t>(2 * K + 1);
-  uint32_t* item_start = h->ws.take<uint32_t>(2 * K + 1);
-  uint32_t* counters = h->ws.take<uint32_t>(4);
+// The buffers of a chunk planned into ck, written there.  The partition's scratch is taken by CentreScorer::select.
+static void treeah_take_chunk(const scann_treeah* h, Workspace& ws, scann_treeah::Chunk& ck) {
+  const size_t K = h->K, nq = ck.nq, P = nq * ck.L;
+  if (ck.partition) ck.tokens = ws.take<uint32_t>(P);
+  ck.leaf_cnt = ws.take<uint32_t>(2 * K + 4 * K * kWlPad);  // counts of the 2K virtual leaves + padded counters / cursors
+  ck.pair_start = ws.take<uint32_t>(2 * K + 1);
+  ck.item_start = ws.take<uint32_t>(2 * K + 1);
+  ck.counters = ws.take<uint32_t>(4);
   const size_t nwl = (2 * K + kWlBlock - 1) / kWlBlock;
-  uint32_t* wl_blk_pair = h->ws.take<uint32_t>(nwl);
-  uint32_t* wl_blk_item = h->ws.take<uint32_t>(nwl);
-  unsigned long long* wl_blk_bytes = h->ws.take<unsigned long long>(nwl);
-  uint32_t* sorted_pairs = h->ws.take<uint32_t>(P);
-  uint4* items = h->ws.take<uint4>(max_items);
-  uint2* cand = h->ws.take<uint2>(P * R);
-  uint32_t* cand_cnt = h->ws.take<uint32_t>(P);
-  uint32_t* qthr = h->ws.take<uint32_t>(nq);
-  uint32_t* qR = cp.any() ? h->ws.take<uint32_t>(nq) : nullptr;
-  uint32_t* qk = cp.any() ? h->ws.take<uint32_t>(nq) : nullptr;
+  ck.wl_blk_pair = ws.take<uint32_t>(nwl);
+  ck.wl_blk_item = ws.take<uint32_t>(nwl);
+  ck.wl_blk_bytes = ws.take<unsigned long long>(nwl);
+  ck.sorted_pairs = ws.take<uint32_t>(P);
+  ck.items = ws.take<uint4>(P / ck.G + 2 * std::min<size_t>(K, P) + 1);
+  ck.cand = ws.take<uint2>(P * ck.R);
+  ck.cand_cnt = ws.take<uint32_t>(P);
+  ck.qthr = ws.take<uint32_t>(nq);
+  ck.qR = ck.params ? ws.take<uint32_t>(nq) : nullptr;
+  ck.qk = ck.params ? ws.take<uint32_t>(nq) : nullptr;
+}
+
+// Workspace bytes of a chunk planned into `plan`: treeah_take_chunk in phase 1, the partition's scratch and, in
+// phase 2, the tensor-core scan
+static size_t treeah_count_chunk(const scann_treeah* h, scann_treeah::Chunk plan) {
+  return Workspace::count([&](Workspace& w) {
+    treeah_take_chunk(h, w, plan);
+    if (plan.partition) h->part.take_scratch(w, plan.nq);
+    if (plan.use_tc) take_tc_scan(w, plan.nq, plan.L, h->K, h->S, h->max_leaf, tc_qcap(plan.R));
+  });
+}
+
+// Phase 1 of a chunk planned into h->ck: partition -> worklist -> (two_phase: scan of the class-A items, i.e. every
+// query's closest leaf on this shard; tau_out receives the bounds they prove).  State for phase 2 stays in h->ck / the
+// workspace.
+static scann_status treeah_phase1(scann_treeah* h, const float* dq, size_t k, bool two_phase, float* tau_out,
+                                  const uint32_t* tokens_in, const ChunkFilter& filt, const ChunkParams& cp,
+                                  cudaStream_t s) {
+  scann_treeah::Chunk& ck = h->ck;
+  const size_t nq = ck.nq, L = ck.L, R = ck.R, P = nq * L;
+  treeah_take_chunk(h, h->ws, ck);
+  SCANN_TRY(h->ws.check("Tree-AH chunk"));
+  if (!ck.partition) ck.tokens = const_cast<uint32_t*>(tokens_in);  // the caller keeps the array alive
+  ck.dq = dq;
+  ck.k = k;
 
   // 1. partition (K == 1 still goes through it: one centre, token 0)
   h->span_begin(0, s);
-  if (!tokens_in) SCANN_TRY(h->part.select(dq, nq, L, tokens, nullptr, scratch, s));
-  if (cp.any()) {  // per-query parameters: the ranks a query does not search leave the batch here
+  if (ck.partition) SCANN_TRY(h->part.select(dq, nq, L, ck.tokens, nullptr, h->ws, s));
+  if (ck.params) {  // per-query parameters: the ranks a query does not search leave the batch here
     query_params_kernel<<<static_cast<unsigned>((P + 255) / 256), 256, 0, s>>>(
-        tokens, P, static_cast<uint32_t>(L), static_cast<uint32_t>(cp.L_call), static_cast<uint32_t>(R),
-        static_cast<uint32_t>(k), cp.L, cp.R, cp.k, qR, qk);
+        ck.tokens, P, static_cast<uint32_t>(L), static_cast<uint32_t>(cp.L_call), static_cast<uint32_t>(R),
+        static_cast<uint32_t>(k), cp.L, cp.R, cp.k, ck.qR, ck.qk);
     SCANN_CUDA(cudaGetLastError());
     h->prof_launches += 1;
   }
   h->span_end(s);
   // 2. worklist
   h->span_begin(1, s);
-  h->ck.use_tc = two_phase && treeah_use_tc(h, nq, L, R);  // the tensor-core scan needs the bounds of phase 1
-  h->ck.T = h->ck.use_tc ? static_cast<int>(tc_ranks(L)) : 1;
-  h->ck.G = G;
-  h->ck.leaf_cnt = leaf_cnt;
-  h->ck.pair_start = pair_start;
-  h->ck.item_start = item_start;
-  h->ck.wl_blk_pair = wl_blk_pair;
-  h->ck.wl_blk_item = wl_blk_item;
-  h->ck.wl_blk_bytes = wl_blk_bytes;
-  h->ck.sorted_pairs = sorted_pairs;
-  h->ck.items = items;
-  h->ck.counters = counters;
-  h->ck.cand_cnt = cand_cnt;
-  SCANN_CUDA(cudaMemsetAsync(qthr, 0xFF, nq * sizeof(uint32_t), s));
-  SCANN_TRY(treeah_worklist(h, tokens, nq, L, true, s));
+  SCANN_CUDA(cudaMemsetAsync(ck.qthr, 0xFF, nq * sizeof(uint32_t), s));
+  SCANN_TRY(treeah_worklist(h, ck.tokens, nq, L, true, s));
   h->span_end(s);
-  ScanArgs& a = h->ck.a;
+  ScanArgs& a = ck.a;
   a.codes = reinterpret_cast<const uint4*>(h->codes.p);
   a.blk_off = h->blk_off.p;
   a.pt_off = h->pt_off.p;
   a.centers = h->part.centers();
   a.codebook = h->codebook.p;
   a.queries = dq;
-  a.items = items;
-  a.sorted_pairs = sorted_pairs;
-  a.counters = counters;
+  a.items = ck.items;
+  a.sorted_pairs = ck.sorted_pairs;
+  a.counters = ck.counters;
   a.end_idx = 0;
   a.max_blocks = 0;
   a.allow = filt.allow;
   a.allow_stride = filt.stride;
   a.qfilt = filt.qfilt;
   a.num_filters = filt.F;
-  a.qR = qR;
+  a.qR = ck.qR;
   a.sentinel = 255u * static_cast<uint32_t>(h->S) + 1u;
-  a.cand = cand;
-  a.cand_cnt = cand_cnt;
-  a.qthr = qthr;
+  a.cand = ck.cand;
+  a.cand_cnt = ck.cand_cnt;
+  a.qthr = ck.qthr;
   a.mul.one = 1u;
   a.mul.sh24 = 1u << 24;
   a.mul.w15 = 0x80000001u;
@@ -931,20 +951,7 @@ static scann_status treeah_phase1(scann_treeah* h, const float* dq, size_t nq, s
   a.cap = 0;  // set per CTA shape in launch_scan_mode
   a.pos_bits = h->pos_bits;
   a.use_residuals = h->use_residuals;
-  h->ck.dq = dq;
-  h->ck.nq = nq;
-  h->ck.L = L;
-  h->ck.R = R;
-  h->ck.k = k;
-  h->ck.G = G;
-  h->ck.tokens = tokens;
-  h->ck.counters = counters;
-  h->ck.cand = cand;
-  h->ck.cand_cnt = cand_cnt;
-  h->ck.qthr = qthr;
-  h->ck.qR = qR;
-  h->ck.qk = qk;
-  h->prof_launches += (tokens_in ? 0 : h->part.launches()) + 7;  // partition + 7 worklist kernels
+  h->prof_launches += (ck.partition ? h->part.launches() : 0) + 7;  // partition + 7 worklist kernels
   if (two_phase) {
     // 3a. probe of the class-A items: the first probe_blocks() blocks of every query's closest leaf prove a bound in
     // bounded time (a full scan of the largest leaves would serialise on a few CTAs); phase 2 scans them in full
@@ -952,17 +959,17 @@ static scann_status treeah_phase1(scann_treeah* h, const float* dq, size_t nq, s
     a.end_idx = 2;
     // tensor-core mode: the class-A ranks are scanned in full here (their per-leaf lists are final, phase 2 does not
     // come back to them); otherwise a bounded probe of the closest leaf
-    a.max_blocks = h->ck.use_tc ? 0 : probe_blocks();
-    SCANN_TRY(launch_scan_g(h->ck.G, a, h->sms, s));
+    a.max_blocks = ck.use_tc ? 0 : probe_blocks();
+    SCANN_TRY(launch_scan_g(ck.G, a, h->sms, s));
     h->prof_launches += 1;
-    if (h->ck.use_tc) {  // the class-A lists are final: their union bounds the tensor-core pass
+    if (ck.use_tc) {  // the class-A lists are final: their union bounds the tensor-core pass
       union_bound_kernel<<<static_cast<unsigned>((nq + 7) / 8), 256, 0, s>>>(
-          cand, cand_cnt, nq, static_cast<uint32_t>(L), static_cast<uint32_t>(h->ck.T), static_cast<uint32_t>(R), qR,
-          qthr);
+          ck.cand, ck.cand_cnt, nq, static_cast<uint32_t>(L), static_cast<uint32_t>(ck.T), static_cast<uint32_t>(R),
+          ck.qR, ck.qthr);
       h->prof_launches += 1;
     }
     if (tau_out) {
-      tau_out_kernel<<<static_cast<unsigned>((nq + 255) / 256), 256, 0, s>>>(qthr, nq, tau_out);
+      tau_out_kernel<<<static_cast<unsigned>((nq + 255) / 256), 256, 0, s>>>(ck.qthr, nq, tau_out);
       h->prof_launches += 1;
     }
     SCANN_CUDA(cudaGetLastError());
@@ -983,12 +990,7 @@ static scann_status treeah_phase2(scann_treeah* h, bool two_phase, const float* 
     SCANN_CUDA(cudaMemsetAsync(h->ck.counters + 1, 0, sizeof(uint32_t), s));  // restart the item counter
     if (tau_in) tau_in_kernel<<<static_cast<unsigned>((nq + 255) / 256), 256, 0, s>>>(tau_in, nq, h->ck.qthr);
   }
-  TcScanOut tco;
-  tco.qcand = nullptr;
-  tco.qcnt = nullptr;
-  tco.qflag = nullptr;
-  tco.fb_tokens = nullptr;
-  tco.launches = 0;
+  TcScanOut tco{nullptr, nullptr, nullptr, nullptr};
   (h->ck.use_tc ? h->stat_tc : h->stat_lut) += 1;
   if (h->ck.use_tc) {
     // 3b. tensor-core scan (tcscan.cu) under the bounds of the probe: per-query candidate lists; the queries it flags
@@ -1034,7 +1036,7 @@ static scann_status treeah_phase2(scann_treeah* h, bool two_phase, const float* 
     }
     SCANN_TRY(launch_tc_scan(tp, h->ws, &tco, s));
     SCANN_TRY(treeah_worklist(h, tco.fb_tokens, nq, L, false, s));
-    h->prof_launches += tco.launches + 7;
+    h->prof_launches += kTcScanLaunches + 7;
   }
   a.end_idx = 0;
   a.max_blocks = 0;
@@ -1090,16 +1092,6 @@ static scann_status treeah_phase2(scann_treeah* h, bool two_phase, const float* 
   return SCANN_OK;
 }
 
-static scann_status treeah_search_chunk(scann_treeah* h, const float* dq, size_t nq, size_t L, size_t R, size_t k,
-                                        uint32_t* d_ids, float* d_dists, uint32_t* d_counts, uint32_t* d_cand_ids,
-                                        float* d_cand_dists, uint32_t* d_cand_counts, const ChunkFilter& filt,
-                                        const ChunkParams& cp, cudaStream_t s) {
-  // with the tensor-core scan the chunk runs as probe (bounds from every query's closest leaf) + bulk scan
-  const bool tc = treeah_use_tc(h, nq, L, R);
-  SCANN_TRY(treeah_phase1(h, dq, nq, L, R, k, tc, nullptr, nullptr, filt, cp, s));
-  return treeah_phase2(h, tc, nullptr, d_ids, d_dists, d_counts, d_cand_ids, d_cand_dists, d_cand_counts, s);
-}
-
 // Per-call restrict filters of scann_treeah_search_filtered (the caller's arrays): F = num_filters rows of
 // ceil(num_ids / 8) bytes, the row of every query.
 struct FilterTable {
@@ -1113,45 +1105,31 @@ struct ParamTable {
   const uint32_t *L, *R, *k;
 };
 
-// Workspace of a chunk, plus (ft != nullptr) what a filtered call takes once for the whole batch of nq_call queries:
-// the filters in block order and, on SCANN_HOST, the uploaded bitmaps and rows; (pt != nullptr) the per-query R / k
-// of a chunk and, on SCANN_HOST, the uploaded parameter arrays.
-static size_t treeah_chunk_bytes(const scann_treeah* h, size_t nq, size_t L, size_t R, bool have_tokens = false,
-                                 const FilterTable* ft = nullptr, size_t nq_call = 0, int memspace = SCANN_DEVICE,
-                                 const ParamTable* pt = nullptr) {
-  size_t K = h->K, P = nq * L;
-  size_t b = 0;
-  auto add = [&](size_t bytes) { b += Workspace::padded(bytes); };
+// What a call takes once for its whole batch of nq queries: (ft) the filters in block order and, on SCANN_HOST, the
+// uploaded bitmaps and rows; (pt, SCANN_HOST) the uploaded per-query L / R / k.  Every chunk reads its slice.
+struct CallBufs {
+  uint8_t* table = nullptr;
+  uint8_t* allow = nullptr;
+  uint32_t* qf = nullptr;
+  uint32_t* params[3] = {};  // L, R, k
+};
+static CallBufs treeah_take_call(const scann_treeah* h, Workspace& ws, size_t nq, int memspace, const FilterTable* ft,
+                                 const ParamTable* pt) {
+  CallBufs b;
+  const bool host = memspace == SCANN_HOST;
   if (ft) {
-    add(ft->F * h->num_blocks * 32);
-    if (memspace == SCANN_HOST) {
-      add(ft->F * ((ft->num_ids + 7) / 8));
-      add(nq_call * 4);
+    b.table = ws.take<uint8_t>(ft->F * h->num_blocks * 32);
+    if (host) {
+      b.allow = ws.take<uint8_t>(ft->F * ((ft->num_ids + 7) / 8));
+      b.qf = ws.take<uint32_t>(nq);
     }
   }
-  if (pt) {
-    add(nq * 4);
-    add(nq * 4);
-    if (memspace == SCANN_HOST)
-      for (const uint32_t* a : {pt->L, pt->R, pt->k})
-        if (a) add(nq_call * 4);
+  if (pt && host) {
+    const uint32_t* src[3] = {pt->L, pt->R, pt->k};
+    for (int i = 0; i < 3; ++i)
+      if (src[i]) b.params[i] = ws.take<uint32_t>(nq);
   }
-  if (!have_tokens) add(h->part.scratch_bytes(nq));
-  add(P * 4);
-  add((2 * K + 4 * K * kWlPad) * 4);
-  add((2 * K + 1) * 4);
-  add((2 * K + 1) * 4);
-  add(16);
-  add(((2 * K + 255) / 256) * 4);
-  add(((2 * K + 255) / 256) * 4);
-  add(((2 * K + 255) / 256) * 8);
-  add(P * 4);
-  add((P + 2 * K + 2) * 16);
-  add(P * R * 8);
-  add(P * 4);
-  add(nq * 4);
-  if (treeah_use_tc(h, nq, L, R)) b += tc_scan_workspace_bytes(nq, L, K, h->S, h->max_leaf, tc_qcap(R));
-  return b + 4096;
+  return b;
 }
 
 // scann_treeah_search, scann_treeah_search_filtered (ft != nullptr: per-query filters of this call only) and
@@ -1203,46 +1181,56 @@ static scann_status treeah_search(scann_treeah* h, const float* queries, size_t 
   chunk = std::min(chunk, std::max<size_t>(1, (size_t(512) << 20) / (h->K * 4)));
   const QueryOut outs[] = {{ids, k * 4}, {dists, k * 4}, {counts, 4},
                            {cand_ids, R * 4}, {cand_dists, R * 4}, {cand_counts, 4}};
-  SCANN_TRY(h->ws.reserve(treeah_chunk_bytes(h, chunk, L, Reff, false, ft, nq, memspace, pt) +
-                          staging_bytes(memspace, chunk, h->dim, outs)));
+  const char* tc_env = getenv("SCANN_SCAN_TC");
+  const bool filtered = ft != nullptr || h->filter_on, params = pt && (pt->L || pt->R || pt->k);
+  // One chunk's carve is reserved for the largest of the distinct chunk sizes (a full chunk and the last one): G grows
+  // with a chunk's queries, so the items P / G + ... of a short last chunk can outnumber those of a full chunk.
+  size_t chunk_bytes = 0;
+  for (const size_t nqc : {chunk, nq % chunk}) {
+    if (nqc == 0) continue;
+    scann_treeah::Chunk plan;
+    treeah_plan(h, nqc, L, R, tc_env, true, filtered, params, plan);
+    chunk_bytes = std::max(chunk_bytes, treeah_count_chunk(h, plan));
+  }
+  SCANN_TRY(h->ws.reserve(chunk_bytes + Workspace::count([&](Workspace& w) {
+                            treeah_take_call(h, w, nq, memspace, ft, pt);
+                            take_staging(w, memspace, chunk, h->dim, outs);
+                          })));
   SCANN_CUDA(cudaMemsetAsync(h->stats.p, 0, 4 * sizeof(unsigned long long), s));
-  // the filters of the whole batch, once per call (below the staging of run_query_chunks): every chunk reads its slice
+  // below the staging of run_query_chunks
+  const CallBufs cb = treeah_take_call(h, h->ws, nq, memspace, ft, pt);
+  SCANN_TRY(h->ws.check("Tree-AH call"));
   ChunkFilter filt = handle_filter(h);
   if (ft) {
     const size_t total = h->num_blocks * 32, row_bytes = (ft->num_ids + 7) / 8;
-    uint8_t* table = h->ws.take<uint8_t>(ft->F * total);
     const uint8_t* src = ft->allow;
     const uint32_t* qf = ft->filter_of_query;
     if (memspace == SCANN_HOST) {
-      uint8_t* d_src = h->ws.take<uint8_t>(ft->F * row_bytes);
-      uint32_t* d_qf = h->ws.take<uint32_t>(nq);
       if (ft->F * row_bytes > 0)
-        SCANN_CUDA(cudaMemcpyAsync(d_src, src, ft->F * row_bytes, cudaMemcpyHostToDevice, s));
-      SCANN_CUDA(cudaMemcpyAsync(d_qf, qf, nq * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
-      src = d_src;
-      qf = d_qf;
+        SCANN_CUDA(cudaMemcpyAsync(cb.allow, src, ft->F * row_bytes, cudaMemcpyHostToDevice, s));
+      SCANN_CUDA(cudaMemcpyAsync(cb.qf, qf, nq * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
+      src = cb.allow;
+      qf = cb.qf;
     }
     if (total > 0) {
       build_allow_kernel<<<static_cast<unsigned>((total + 255) / 256), 256, 0, s>>>(
-          src, row_bytes, ft->F, ft->num_ids, h->blk_leaf.p, h->blk_off.p, h->pt_off.p, h->ids.p, total, table);
+          src, row_bytes, ft->F, ft->num_ids, h->blk_leaf.p, h->blk_off.p, h->pt_off.p, h->ids.p, total, cb.table);
       SCANN_CUDA(cudaGetLastError());
     }
-    filt.allow = table;
+    filt.allow = cb.table;
     filt.stride = total;
     filt.F = static_cast<uint32_t>(ft->F);
     filt.qfilt = qf;
   }
-  // the per-query parameters of the whole batch, uploaded once per call on SCANN_HOST: every chunk reads its slice
   ParamTable dp{nullptr, nullptr, nullptr};
   if (pt) {
     dp = *pt;
-    if (memspace == SCANN_HOST)
-      for (const uint32_t** a : {&dp.L, &dp.R, &dp.k})
-        if (*a) {
-          uint32_t* d = h->ws.take<uint32_t>(nq);
-          SCANN_CUDA(cudaMemcpyAsync(d, *a, nq * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
-          *a = d;
-        }
+    const uint32_t** a[3] = {&dp.L, &dp.R, &dp.k};
+    for (int i = 0; i < 3; ++i)
+      if (cb.params[i]) {
+        SCANN_CUDA(cudaMemcpyAsync(cb.params[i], *a[i], nq * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
+        *a[i] = cb.params[i];
+      }
   }
   return run_query_chunks(h->ws, memspace, s, queries, nq, h->dim, chunk, outs,
                           [&](const float* dq, size_t q0, size_t nqc, void* const* o) -> scann_status {
@@ -1267,8 +1255,12 @@ static scann_status treeah_search(scann_treeah* h, const float* queries, size_t 
       cp.k = dp.k ? dp.k + q0 : nullptr;
       cp.L_call = L_call;
     }
-    return treeah_search_chunk(h, dq, nqc, L, R, k, d_ids, d_dists, d_counts, static_cast<uint32_t*>(o[3]),
-                               static_cast<float*>(o[4]), d_cc, cf, cp, s);
+    treeah_plan(h, nqc, L, R, tc_env, true, filtered, params, h->ck);
+    // with the tensor-core scan the chunk runs as probe (bounds from every query's closest leaf) + bulk scan
+    const bool two_phase = h->ck.use_tc;
+    SCANN_TRY(treeah_phase1(h, dq, k, two_phase, nullptr, nullptr, cf, cp, s));
+    return treeah_phase2(h, two_phase, nullptr, d_ids, d_dists, d_counts, static_cast<uint32_t*>(o[3]),
+                         static_cast<float*>(o[4]), d_cc, s);
   });
 }
 
@@ -1531,10 +1523,9 @@ scann_status scann_treeah_partition(scann_treeah* h, const float* queries, size_
   const size_t K = h->K;
   const size_t Leff = std::min(L, K);
   SCANN_REQUIRE(Leff == L, SCANN_INVALID_ARGUMENT, "partitions_to_search %zu > %zu partitions", L, K);
-  const size_t scratch_bytes = h->part.scratch_bytes(nq);
-  SCANN_TRY(h->ws.reserve(scratch_bytes + 4096));
+  SCANN_TRY(h->ws.reserve(Workspace::count([&](Workspace& w) { h->part.take_scratch(w, nq); })));
   h->prof_launches += h->part.launches();
-  return h->part.select(queries, nq, L, tokens, nullptr, h->ws.take<uint8_t>(scratch_bytes), call.s);
+  return h->part.select(queries, nq, L, tokens, nullptr, h->ws, call.s);
 }
 
 scann_status scann_treeah_search_begin(scann_treeah* h, const float* queries, size_t nq, size_t qdim, size_t L,
@@ -1555,9 +1546,11 @@ scann_status scann_treeah_search_begin(scann_treeah* h, const float* queries, si
   SCANN_REQUIRE(!h->split_active, SCANN_FAILED_PRECONDITION, "scann_treeah_search_begin called twice without _end");
   {
     CallScope call(h->device, h->order, SCANN_DEVICE, stream, h->stream);
-    SCANN_TRY(h->ws.reserve(treeah_chunk_bytes(h, nq, L, R, tokens != nullptr)));
+    // the reservation covers _end's tensor-core scan too: _end takes it from above phase 1's buffers
+    treeah_plan(h, nq, L, R, getenv("SCANN_SCAN_TC"), tokens == nullptr, h->filter_on, false, h->ck);
+    SCANN_TRY(h->ws.reserve(treeah_count_chunk(h, h->ck)));
     cudaMemsetAsync(h->stats.p, 0, 4 * sizeof(unsigned long long), call.s);
-    SCANN_TRY(treeah_phase1(h, queries, nq, L, R, k, true, tau_out, tokens, handle_filter(h), ChunkParams(), call.s));
+    SCANN_TRY(treeah_phase1(h, queries, k, true, tau_out, tokens, handle_filter(h), ChunkParams(), call.s));
   }
   // The handle is marked busy, not locked: every other entry point answers FAILED_PRECONDITION until _end (or _abort),
   // so nothing can be left locked by a caller that fails between the two calls.
