@@ -6,7 +6,17 @@
 //
 // u8 x u8 products accumulated in s32 are exact, so the accumulators are bit-identical to the reference's u32 sums.
 // The register-LUT kernel spends ~1.25 ALU instructions per (query, point, subspace) lookup and is ALU-pipe bound with
-// the tensor pipe idle; here a 128-point x 128-query tile costs 24 (S = 48) tcgen05.mma instructions of 64 cycles.
+// the tensor pipe idle; here a 128-point x 128-query tile costs 12 (S = 48) 2:4-sparse tcgen05.mma instructions of
+// K = 64 plus one dense K = 32 instruction for the threshold bytes.
+//
+// The one-hot operand is 2:4 sparse by construction (one 1 among a subspace's 16 bytes), so A is stored compressed:
+// per subspace 8 value bytes (2 per group of 4 K-bytes) and 16 bits of metadata (a nibble per group: the positions of
+// the two kept bytes); expand_sparse gives the encoding.  TMEM map (512 columns, lane = point row):
+//   0..255    two s32 accumulators of 128 query columns
+//   256..447  A ring, 6 slots x 32 columns of values: a slot is 16 subspaces (four K = 64 MMAs of 8 columns each)
+//   448..495  the slots' metadata, 8 columns each (two per MMA: groups 0-7 / 8-15 of its 64 K-bytes, nibble g % 8)
+//   496..503  the threshold constants (1, 255, 0, ...): written once per CTA, read by the dense MMA of every tile
+// Each pipeline owns 3 slots, a whole S = 48 tile.
 //
 // Per batch (launch_tc_scan, after the probe of every query's closest leaf has produced the bounds tau_q):
 //   tcwl_*           the caller's class-B lists (pairs (query, rank >= T) grouped BY LEAF, treeah.cu) cut into groups and
@@ -16,11 +26,13 @@
 //                    one K-major u8 row of the group's LUT tile, followed by two "threshold digits" (below)
 //   tc_scan_kernel   persistent, one CTA per SM, warp-specialised:
 //       warp 0       TMA: the item's LUT tile (128 rows x (S*16 + 32) bytes, 128-byte swizzle) -> shared memory (B operand)
-//       warp 1       one lane issues tcgen05.mma.kind::i8, M = 128 points, N = 16..128 queries, K = 32 bytes; the A
-//                    operand is read from TENSOR MEMORY, the accumulator (s32) is double-buffered in TMEM
-//       warps 2-9    expanders: thread = one point; turn its packed 4-bit codes into one-hot bytes in registers, 8
-//                    subspaces (128 K-bytes) at a time, and tcgen05.st them into a ring of A slots in TMEM
-//       warps 10-13  epilogue: tcgen05.ld the accumulator (thread = one point, columns = queries), threshold, append the
+//       warps 1-2    one lane each (one per accumulator) issues tcgen05.mma.sp.kind::i8, M = 128 points, N = 16..128
+//                    queries, K = 64 bytes; the compressed A operand and its metadata are read from TENSOR MEMORY, the
+//                    accumulator (s32) is double-buffered in TMEM
+//       warps 4-11   expanders (warps 4-19 with SCANN_TC_EXP=4): thread = one point; turn its packed 4-bit codes into
+//                    compressed one-hot values and metadata in registers, 16 subspaces (256 K-bytes) at a time, and
+//                    tcgen05.st them into a ring of A slots in TMEM
+//       last 8 warps epilogue: tcgen05.ld the accumulator (thread = one point, columns = queries), threshold, append the
 //                    survivors (approx distance key | leaf rank | position) to per-query candidate lists
 //   Threshold without a per-column compare: the LUT row of (query, leaf) carries two extra bytes (d0, d1) with
 //   d0 + 255 d1 = BIG - smax, smax = the largest integer score whose dequantised distance is <= tau_q, and every point
@@ -48,10 +60,13 @@ namespace {
 
 // warp 0 TMA, 1-2 MMA issuers, 3 TMEM owner, then 4 * EG expander warps, then 8 epilogue warps
 constexpr int ts_threads(int EG) { return 32 * (4 + 4 * EG + 8); }
-constexpr int kTsRing = 8;            // A slots of 32 TMEM columns (128 K-bytes per point row)
-constexpr int kTsHalf = kTsRing / 2;  // each expander group owns half of the ring: every use of a slot is by the same
-                                      // group, so a waiter is never more than one mbarrier phase ahead
-constexpr int kTsAcol = 256;          // first TMEM column of the A ring (accumulators: 2 x 128 columns before it)
+constexpr int kTsRing = 6;            // A slots: 16 subspaces (256 dense K-bytes) of a point row each
+constexpr int kTsHalf = kTsRing / 2;  // each pipeline owns half of the ring: 48 subspaces, a whole S = 48 tile
+constexpr int kTsAcol = 256;          // TMEM columns of the slots' compressed values, 32 per slot (accumulators: 2 x 128
+                                      // columns before them)
+constexpr int kTsMcol = kTsAcol + 32 * kTsRing;  // the slots' sparsity metadata, 8 columns per slot
+constexpr int kTsTcol = kTsMcol + 8 * kTsRing;   // the threshold constants (1, 255, 0, ...): a dense K = 32 A operand
+static_assert(kTsTcol + 8 <= 512, "TMEM map");
 constexpr int kTsAtom = 128 * 128;    // bytes of one (128 rows x 128 B) swizzle atom tile
 constexpr uint32_t kTsBig = 32768;    // > 255 * 64: accumulator threshold
 constexpr uint32_t kNoKey = 0xFFFFFFFFu;
@@ -117,6 +132,16 @@ __device__ __forceinline__ void mma_i8_ts(uint32_t d, uint32_t a_tmem, uint64_t 
       "r"(a_tmem), "l"(bdesc), "r"(idesc), "r"(acc)
       : "memory");
 }
+// D[tmem] (+)= A[tmem] * B[smem desc] with A 2:4-sparse: 32 compressed bytes per row stand for K = 64, the metadata
+// (4 bits per 4 K-bytes: the positions of the two kept bytes) is read from TMEM at m_tmem
+__device__ __forceinline__ void mma_i8_sp(uint32_t d, uint32_t a_tmem, uint64_t bdesc, uint32_t m_tmem, uint32_t idesc,
+                                          uint32_t acc) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %5, 0;\n\t"
+      "tcgen05.mma.sp.cta_group::1.kind::i8 [%0], [%1], %2, [%3], %4, p;\n\t}" ::"r"(d),
+      "r"(a_tmem), "l"(bdesc), "r"(m_tmem), "r"(idesc), "r"(acc)
+      : "memory");
+}
 __device__ __forceinline__ void tc_ld32(uint32_t taddr, uint32_t (&v)[32]) {
   asm volatile(
       "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
@@ -154,10 +179,9 @@ __device__ __forceinline__ void tc_st32(uint32_t taddr, const uint32_t (&v)[32])
       "r"(v[28]), "r"(v[29]), "r"(v[30]), "r"(v[31])
       : "memory");
 }
-__device__ __forceinline__ void tc_st8(uint32_t taddr, uint32_t v0) {
-  const uint32_t z = 0;
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr), "r"(v0),
-               "r"(z), "r"(z), "r"(z), "r"(z), "r"(z), "r"(z), "r"(z)
+__device__ __forceinline__ void tc_st8(uint32_t taddr, const uint32_t (&v)[8]) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr), "r"(v[0]),
+               "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7])
                : "memory");
 }
 __device__ __forceinline__ void tc_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
@@ -176,29 +200,47 @@ __device__ __forceinline__ uint32_t shl_clamp(uint32_t v, uint32_t sh) {  // PTX
   return r;
 }
 
-// One word of packed codes = the 4-bit codes of 8 consecutive subspaces of one point -> 8 x 16 one-hot bytes (K order:
-// subspace-major, code-minor = the byte order of a LUT row).  Byte (s, c) is 1 iff code_s == c.
-// Pipe balance: the expansion is the ALU-pipe load of the kernel (~5 nibbles per clock per SM at full tensor rate), so
-// the nibble extraction and the three "- 32 k" run as integer multiply-adds on the FMA pipe; the multipliers come from
-// kernel parameters (xm.sh[i] = 1 << (28 - 4 i), xm.eight = 8) so that the compiler cannot turn them back into shifts.
+// Two words of packed codes = the 4-bit codes of 16 consecutive subspaces of one point -> their one-hot rows (K order:
+// subspace-major, code-minor = the byte order of a LUT row; byte (s, c) is 1 iff code_s == c) in the 2:4-compressed form
+// of the sparse MMA.  A subspace's 16 bytes are 4 groups of 4, each kept as 2 value bytes plus a 4-bit metadata nibble
+// (bits 0-1: position of the first kept byte, bits 2-3: of the second).  Code c = 4 g + j is the value byte c >> 1 of
+// the subspace's 8 (group g, kept byte j >> 1); every group of the subspace gets the nibble (0,2) when c is even and
+// (1,3) when c is odd, which puts the 1 at position j and is a valid (increasing) pair for the groups whose values are 0.
+// So the values depend on c >> 1 only and the metadata on c & 1 only:
+//   r[2 s], r[2 s + 1]  value bytes 0-3, 4-7 of subspace s: 1 << 8 (c >> 1), 1 << (8 (c >> 1) - 32) (0 when >= 32)
+//   mt[s / 2]           metadata of subspaces s (bits 0-15) and s + 1 (bits 16-31): 0x8888 or 0xDDDD each
+// Pipe balance: the expansion is the ALU-pipe load of the kernel, so the nibble extraction and "8 p - 32" run as integer
+// multiply-adds on the FMA pipe; the multipliers come from kernel parameters (xm.sh[i] = 1 << (28 - 4 i), xm.eight = 8)
+// so that the compiler cannot turn them back into shifts.  The metadata is one PRMT (the sign-replicating byte select
+// turns bit 0 of a code into 0x00 / 0xFF bytes) and one LOP3 per two subspaces.
 struct ExpandMul {
   uint32_t sh[8];
   uint32_t eight;
 };
-__device__ __forceinline__ void expand_onehot(uint32_t C, uint32_t (&r)[32], const ExpandMul& xm) {
+__device__ __forceinline__ void expand_sparse(uint32_t C0, uint32_t C1, uint32_t (&r)[32], uint32_t (&mt)[8],
+                                              const ExpandMul& xm) {
 #pragma unroll
-  for (int i = 0; i < 8; ++i) {
-    uint32_t x, t, t1, t2, t3;
-    asm("mul.lo.u32 %0, %1, %2;" : "=r"(x) : "r"(C), "r"(xm.sh[i]));  // nibble i -> bits 28..31 (lower nibbles below it)
-    const uint32_t nib = x >> 28;                                         // the code, 0..15
-    asm("mul.lo.u32 %0, %1, %2;" : "=r"(t) : "r"(nib), "r"(xm.eight));                // 8 * code: bit position of the 1
-    asm("mad.lo.u32 %0, %1, %2, 0xFFFFFFE0;" : "=r"(t1) : "r"(nib), "r"(xm.eight));  // - 32
-    asm("mad.lo.u32 %0, %1, %2, 0xFFFFFFC0;" : "=r"(t2) : "r"(nib), "r"(xm.eight));  // - 64
-    asm("mad.lo.u32 %0, %1, %2, 0xFFFFFFA0;" : "=r"(t3) : "r"(nib), "r"(xm.eight));  // - 96
-    r[4 * i + 0] = shl_clamp(1u, t);
-    r[4 * i + 1] = shl_clamp(1u, t1);
-    r[4 * i + 2] = shl_clamp(1u, t2);
-    r[4 * i + 3] = shl_clamp(1u, t3);
+  for (int h = 0; h < 2; ++h) {
+    const uint32_t C = h ? C1 : C0;
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      uint32_t x, t, t1;
+      asm("mul.lo.u32 %0, %1, %2;" : "=r"(x) : "r"(C), "r"(xm.sh[i]));  // nibble i -> bits 28..31 (lower nibbles below it)
+      const uint32_t p = x >> 29;                                          // value byte of the code: c >> 1
+      asm("mul.lo.u32 %0, %1, %2;" : "=r"(t) : "r"(p), "r"(xm.eight));                // 8 p: bit position of the 1
+      asm("mad.lo.u32 %0, %1, %2, 0xFFFFFFE0;" : "=r"(t1) : "r"(p), "r"(xm.eight));  // - 32
+      r[16 * h + 2 * i] = shl_clamp(1u, t);
+      r[16 * h + 2 * i + 1] = shl_clamp(1u, t1);
+    }
+    uint32_t y, z;
+    asm("mul.lo.u32 %0, %1, %2;" : "=r"(z) : "r"(C), "r"(xm.eight));   // bit 0 of code 2k + 1 -> bit 8k + 7
+    asm("mul.lo.u32 %0, %1, %2;" : "=r"(y) : "r"(z), "r"(xm.sh[6]));   // bit 0 of code 2k -> bit 8k + 7
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {  // bytes 0-1: sign of y's byte k, bytes 2-3: sign of z's byte k
+      uint32_t s;
+      asm("prmt.b32 %0, %1, %2, %3;" : "=r"(s) : "r"(y), "r"(z), "r"(0xCC88u + 0x1111u * k));
+      mt[4 * h + k] = (s & 0x55555555u) | 0x88888888u;
+    }
   }
 }
 
@@ -509,7 +551,7 @@ __device__ __forceinline__ void tcs_emit(const TcsArgs& a, const TcsFilter& f, u
 constexpr int kWqCap = 320;    // entries of one epilogue warp's survivor queue (uint4 {lut_row, acc, pos, leaf (FILT)})
 constexpr int kWqStep = 256;   // most entries one filter step (32 lanes x 8 columns) can add
 
-// EG: expander groups, 2 (one per pipeline) or 4 (two per pipeline, alternate chunks); FILT: restrict filters (a template
+// EG: expander groups, 2 (one per pipeline) or 4 (two per pipeline, alternate slots); FILT: restrict filters (a template
 // flag, so the unfiltered kernel carries none of it)
 template <int EG, bool FILT>
 __global__ void __launch_bounds__(ts_threads(EG), 1) tc_scan_kernel(const __grid_constant__ CUtensorMap tmB, const TcsArgs a,
@@ -550,8 +592,18 @@ __global__ void __launch_bounds__(ts_threads(EG), 1) tc_scan_kernel(const __grid
   __syncthreads();
   tc_fence_after();
   const uint32_t tmem = *tmem_slot;
+  if (warp >= 4 && warp < 8) {  // the threshold constants are the same for every point row: written once (one warp per
+                                // TMEM lane quadrant)
+    const uint32_t c[8] = {0x0000FF01u, 0, 0, 0, 0, 0, 0, 0};
+    tc_st8(tmem + ((static_cast<uint32_t>(warp & 3) * 32) << 16) + kTsTcol, c);
+    tc_wait_st();
+  }
+  tc_fence_before();
+  __syncthreads();
+  tc_fence_after();
   const uint32_t n_items = a.counters[0];
-  const int nchunk = a.KA + 1;  // A chunks per point tile (the last one carries the threshold constants)
+  const int nslot = a.KA / 2;   // A slots (16 subspaces each) per point tile
+  const int nchunk = a.KA + 1;  // B atoms per item: the table bytes, then the threshold digits
 
   if (warp == 0) {
     // ================================================================= TMA producer: the item's LUT tile
@@ -577,46 +629,46 @@ __global__ void __launch_bounds__(ts_threads(EG), 1) tc_scan_kernel(const __grid
       const uint64_t bd0 = umma_desc(smem_u32(sB));
       const uint32_t d = tmem + pp * kTcsGroup;
       const uint32_t a0 = tmem + kTsAcol + pp * kTsHalf * 32;
+      const uint32_t mt0 = tmem + kTsMcol + pp * kTsHalf * 8;
       for (uint32_t item = blockIdx.x; item < n_items; item += gridDim.x, ++it) {
         const uint4 I = a.items[item];
         const uint32_t ncol = (a.groups[I.x].z + 15u) & ~15u;
         const uint32_t idesc = (2u << 4) | ((ncol >> 3) << 17) | ((128u >> 4) << 24);  // s32 += u8 x u8, K-major both
+        const uint32_t idesc_sp = idesc | (1u << 2);                                    // the same, A 2:4-sparse
         mbar_wait(bar(kBFull), it & 1u, 0x200u + it);
         for (uint32_t t = I.y; t < I.z; ++t, ++ts) {
           if ((ts & 1u) != pp) continue;
           const uint32_t k = ts >> 1;  // tiles of this pipeline so far
           mbar_wait(bar(kTEmpty + pp), (k & 1u) ^ 1u, 0x300000u + ts);  // the epilogue has drained this accumulator
           tc_fence_after();
-          uint32_t m = k * static_cast<uint32_t>(nchunk);  // chunks of this pipeline so far
-          for (int c = 0; c < a.KA; ++c, ++m) {
+          uint32_t m = k * static_cast<uint32_t>(nslot);  // slots of this pipeline so far
+          for (int c = 0; c < nslot; ++c, ++m) {
             const uint32_t sl = m % kTsHalf;
             mbar_wait(bar(kAFull + pp * kTsHalf + sl), (m / kTsHalf) & 1u, 0x400000u + m);
             tc_fence_after();
-            const uint64_t bd = bd0 + static_cast<uint64_t>(c) * (kTsAtom >> 4);
-            const uint32_t at = a0 + sl * 32;
-            mma_i8_ts(d, at, bd, idesc, c != 0 ? 1u : 0u);
-            mma_i8_ts(d, at + 8, bd + 2u, idesc, 1u);
-            mma_i8_ts(d, at + 16, bd + 4u, idesc, 1u);
-            mma_i8_ts(d, at + 24, bd + 6u, idesc, 1u);
+            // four K = 64 MMAs: B advances by half a swizzle atom each, the metadata by two columns
+            const uint64_t bd = bd0 + static_cast<uint64_t>(2 * c) * (kTsAtom >> 4);
+            const uint32_t at = a0 + sl * 32, mt = mt0 + sl * 8;
+            mma_i8_sp(d, at, bd, mt, idesc_sp, c != 0 ? 1u : 0u);
+            mma_i8_sp(d, at + 8, bd + 4u, mt + 2, idesc_sp, 1u);
+            mma_i8_sp(d, at + 16, bd + (kTsAtom >> 4), mt + 4, idesc_sp, 1u);
+            mma_i8_sp(d, at + 24, bd + (kTsAtom >> 4) + 4u, mt + 6, idesc_sp, 1u);
             tc_commit(bar(kAEmpty + pp * kTsHalf + sl));  // the slot may be refilled once these MMAs retire
           }
-          {  // the threshold atom holds 32 K-bytes
-            const uint32_t sl = m % kTsHalf;
-            mbar_wait(bar(kAFull + pp * kTsHalf + sl), (m / kTsHalf) & 1u, 0x400000u + m);
-            tc_fence_after();
-            mma_i8_ts(d, a0 + sl * 32, bd0 + static_cast<uint64_t>(a.KA) * (kTsAtom >> 4), idesc, 1u);
-            tc_commit(bar(kAEmpty + pp * kTsHalf + sl));
-            tc_commit(bar(kTFull + pp));
-          }
+          // the threshold atom holds 32 K-bytes, against the constant A rows
+          mma_i8_ts(d, tmem + kTsTcol, bd0 + static_cast<uint64_t>(a.KA) * (kTsAtom >> 4), idesc, 1u);
+          tc_commit(bar(kTFull + pp));
         }
         tc_commit(bar(kBEmpty));  // this pipeline's MMAs on the B tile have retired
       }
     }
   } else if (warp >= 4 && warp < 4 + 4 * EG) {
-    // ================================================================= expanders: codes -> one-hot A chunks in TMEM
-    // Four groups of four warps (one warp per TMEM lane quadrant): pipeline pp = group / 2 takes the tiles of parity
-    // pp, and inside a pipeline the two groups take alternate chunks (by the parity of the pipeline's running chunk
-    // count m), so each A slot (m % 4) is always filled by the same group.
+    // ================================================================= expanders: codes -> sparse one-hot A slots in TMEM
+    // Groups of four warps (one warp per TMEM lane quadrant): pipeline pp takes the tiles of parity pp.  With EG = 4
+    // the two groups of a pipeline take alternate slots (by the parity of the pipeline's running slot count m), so the
+    // uses of one A slot (m % 3) alternate between them.  A parity wait needs the barrier at most one phase behind: the
+    // group's previous slot m - 2 waited for the release of m - 5, and one pipeline's commits complete in order, so
+    // m - 6 (the use before last of this slot) has been released.
     const uint32_t gi = static_cast<uint32_t>(warp - 4) >> 2;
     const uint32_t pp = EG == 4 ? gi >> 1 : gi, sg = gi & 1u;
     const uint32_t quad = warp & 3;
@@ -643,8 +695,8 @@ __global__ void __launch_bounds__(ts_threads(EG), 1) tc_scan_kernel(const __grid
               w[2 * c2 + 1] = v.y;
             }
         }
-        const uint32_t m0 = (ts >> 1) * static_cast<uint32_t>(nchunk);  // chunks of this pipeline before this tile
-        // software pipeline: the tcgen05.st of a chunk is left in flight while this group's next chunk is expanded; its
+        const uint32_t m0 = (ts >> 1) * static_cast<uint32_t>(nslot);  // slots of this pipeline before this tile
+        // software pipeline: the tcgen05.st of a slot is left in flight while this group's next slot is expanded; its
         // completion (wait::st) and the hand-over to the MMA warp come right before the next store
         int prev_slot = -1;
         auto publish = [&]() {
@@ -656,31 +708,22 @@ __global__ void __launch_bounds__(ts_threads(EG), 1) tc_scan_kernel(const __grid
           }
         };
 #pragma unroll
-        for (int c = 0; c < 8; ++c) {
+        for (int c = 0; c < 4; ++c) {
           const uint32_t m = m0 + c;
-          if (c < a.KA && (EG == 2 || (m & 1u) == sg)) {
+          if (c < nslot && (EG == 2 || (m & 1u) == sg)) {
             const uint32_t slot = pp * kTsHalf + (m % kTsHalf);
-            uint32_t r[32];
-            expand_onehot(w[c], r, a.xm);  // rows past the end of the leaf expand code 0: the epilogue ignores them
+            uint32_t r[32], mt[8];
+            // rows past the end of the leaf expand code 0: the epilogue ignores them
+            expand_sparse(w[2 * c], w[2 * c + 1], r, mt, a.xm);
             publish();
             mbar_wait(bar(kAEmpty + slot), ((m / kTsHalf) & 1u) ^ 1u, 0x500000u + m);
             tc_fence_after();
             tc_st32(tmem + lane_addr + kTsAcol + slot * 32, r);
+            tc_st8(tmem + lane_addr + kTsMcol + slot * 8, mt);
             prev_slot = static_cast<int>(slot);
           }
         }
-        {  // threshold chunk: K bytes (1, 255, 0, ...) against the LUT row's digits (d0, d1)
-          const uint32_t m = m0 + static_cast<uint32_t>(a.KA);
-          if (EG == 2 || (m & 1u) == sg) {
-            const uint32_t slot = pp * kTsHalf + (m % kTsHalf);
-            publish();
-            mbar_wait(bar(kAEmpty + slot), ((m / kTsHalf) & 1u) ^ 1u, 0x600000u + m);
-            tc_fence_after();
-            tc_st8(tmem + lane_addr + kTsAcol + slot * 32, 0x0000FF01u);
-            prev_slot = static_cast<int>(slot);
-          }
-          publish();
-        }
+        publish();
       }
     }
   } else if (warp >= 4 + 4 * EG) {
