@@ -87,8 +87,4 @@ scann_status launch_tc_scores(const TcScoreParams& p, cudaStream_t s);
 scann_status kmeans_rows_device(const float* x, size_t n, size_t dim, size_t K, int iters, uint64_t seed,
                                 float balance_ratio, float* centers, uint32_t* assign_out, int device);
 
-// runtime.cu — accumulation mode of the LUT16 scan for a table of S subspaces (lut16_device.cuh scan_block):
-// default 3 (IDP.2A, needs S <= 128) else 2; SCANN_ACC_MODE=0|1|2|3 overrides (tuning / parity tests)
-int scan_acc_mode(int S);
-
 }  // namespace scann

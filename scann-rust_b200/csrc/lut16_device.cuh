@@ -24,7 +24,10 @@
 namespace scann {
 
 constexpr int kBlockPts = 256;   // points per code block (32 lanes x 8 nibbles)
-constexpr int kAccMode = 3;      // default accumulation mode, see scan_block() (measured best on B200)
+
+// Accumulation mode of scan_block() for a table of S subspaces: 3 (IDP.2A, measured best on B200) where the per-point
+// sums fit its 15-bit fields (S <= 128: 128 * 255 = 32640 < 2^15), else 2.
+constexpr int scan_acc_mode(int S) { return S <= 128 ? 3 : 2; }
 
 #ifdef __CUDACC__
 
@@ -137,31 +140,22 @@ __device__ __forceinline__ uint32_t min_sum(const PackedSums& p) {
 }
 
 // Pipe balancing: the PRMT/LOP3 lookups saturate the ALU pipe, so the accumulation is issued on the
-// FMA pipe as integer multiply-adds.  `one` (== 1) and `sh24` (== 1 << 24) are kernel parameters so the
-// compiler cannot strength-reduce them back into ALU-pipe adds/shifts:
-//   acc_e = (r & 0x00FF00FF) * one + acc_e            IMAD
-//   acc_x = hi32(r * sh24) + acc_x  (= (r >> 8) + acc_x)   IMAD.HI
+// FMA pipe as integer multiply-adds.  The multipliers are kernel parameters so the compiler cannot
+// strength-reduce them back into ALU-pipe adds.
 struct AccMul {
-  uint32_t one, sh24, w15;  // 1, 1 << 24, (1 | 2^15 << 16): the IDP.2A weight pair of MODE 3
+  uint32_t one, w15;  // 1 (MODE 2), (1 | 2^15 << 16): the IDP.2A weight pair of MODE 3
 };
-template <int MODE>
+// MODE 2: masked add on the FMA pipe (acc_e = (r & 0x00FF00FF) * one + acc_e, IMAD), shifted add on the ALU pipe
 __device__ __forceinline__ void acc_add(uint32_t& acc_e, uint32_t& acc_x, uint32_t r, const AccMul& m) {
   const uint32_t e = r & 0x00FF00FFu;
-  if (MODE == 0) {  // everything on the ALU pipe (IADD3 / LEA.HI)
-    acc_e += e;
-    acc_x += r >> 8;
-  } else if (MODE == 1) {  // both adds on the FMA pipe
-    asm("mad.lo.u32 %0, %1, %2, %0;" : "+r"(acc_e) : "r"(e), "r"(m.one));
-    asm("mad.hi.u32 %0, %1, %2, %0;" : "+r"(acc_x) : "r"(r), "r"(m.sh24));
-  } else {  // masked add on the FMA pipe, shifted add on the ALU pipe
-    asm("mad.lo.u32 %0, %1, %2, %0;" : "+r"(acc_e) : "r"(e), "r"(m.one));
-    acc_x += r >> 8;
-  }
+  asm("mad.lo.u32 %0, %1, %2, %0;" : "+r"(acc_e) : "r"(e), "r"(m.one));
+  acc_x += r >> 8;
 }
 
 // Scan one 256-point block for G queries.  lut: shared memory, [G][S4] uint4 (one 16-entry u8
 // table per (query, subspace)).  On return out[g] holds the eight u32 accumulators of points
 // lane*8+0..7 in packed form — the same integers src/simd/dispatch.rs:259-295 computes.
+// MODE = scan_acc_mode(S).
 //
 // MODE 3 (S <= 128): the four bytes of a lookup result r are accumulated by two IDP.2A instructions on
 // the FMA pipe with the constant weight pair w = (1, 2^15):
@@ -172,6 +166,7 @@ __device__ __forceinline__ void acc_add(uint32_t& acc_e, uint32_t& acc_x, uint32
 template <int G, int MODE>
 __device__ __forceinline__ void scan_block(const uint4* __restrict__ blk, int SG, const uint4* __restrict__ lut,
                                            int S4, int lane, const AccMul mul, PackedSums (&out)[G]) {
+  static_assert(MODE == 2 || MODE == 3, "accumulation mode");
   uint32_t accEA[G], accXA[G], accEB[G], accXB[G];
 #pragma unroll
   for (int g = 0; g < G; ++g) accEA[g] = accXA[g] = accEB[g] = accXB[g] = 0;
@@ -205,8 +200,8 @@ __device__ __forceinline__ void scan_block(const uint4* __restrict__ blk, int SG
           asm("dp2a.lo.u32.u32 %0, %1, %2, %0;" : "+r"(accEB[g]) : "r"(mul.w15), "r"(rB));
           asm("dp2a.hi.u32.u32 %0, %1, %2, %0;" : "+r"(accXB[g]) : "r"(mul.w15), "r"(rB));
         } else {
-          acc_add<MODE>(accEA[g], accXA[g], rA, mul);
-          acc_add<MODE>(accEB[g], accXB[g], rB, mul);
+          acc_add(accEA[g], accXA[g], rA, mul);
+          acc_add(accEB[g], accXB[g], rB, mul);
         }
       }
     }

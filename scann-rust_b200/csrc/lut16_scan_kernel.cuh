@@ -1,6 +1,6 @@
 // The Tree-AH hot kernel: persistent LUT16 scan over (leaf, <=G queries) work items.
 //
-// Per work item a CTA of NW = 8 warps
+// Per work item a CTA of kScanWarps = 8 warps
 //   (1) stages the G query residuals q - centroid(leaf) in shared memory,
 //   (2) builds the G residual LUT16 tables (warp g builds table g; bit-exact quantiser, lut16_device.cuh),
 //   (3) turns the batch-wide upper bound tau_q of every query (see below) into an integer score bound
@@ -72,15 +72,21 @@ __device__ __forceinline__ uint32_t key_bound_from_tau(float tau, float mult, fl
   return static_cast<uint32_t>(s + 1) << pos_bits;
 }
 
-template <int G, int MODE, int NW, bool FILT>
-__global__ void __launch_bounds__(NW * 32, 16 / NW) lut16_scan_kernel(const ScanArgs a) {
+// 8 warps per scan CTA (2 CTAs/SM), for this kernel and lut_f32_scan_kernel.  Measured on B200 at C3: 8 warps 35.6 ms,
+// 4 warps 35.8 ms, 2 warps 44.7 ms (profiles/r1_scan_kernel.md).
+constexpr int kScanWarps = 8;
+
+// MODE = scan_acc_mode(S) (lut16_device.cuh); FILT: restrict filters (a template flag, so the unfiltered kernel carries
+// none of it)
+template <int G, int MODE, bool FILT>
+__global__ void __launch_bounds__(kScanWarps * 32, 16 / kScanWarps) lut16_scan_kernel(const ScanArgs a) {
   extern __shared__ __align__(16) uint8_t smem[];
   const int S4 = a.SG * 4;
   uint4* lut = reinterpret_cast<uint4*>(smem);                                  // [G][S4]
   float* qres = reinterpret_cast<float*>(lut + G * S4);                         // [G][dim]
   uint32_t* buf = reinterpret_cast<uint32_t*>(qres + ((G * a.dim + 3) & ~3));   // [G][cap], 16-B aligned
-  uint32_t* hist = buf + static_cast<size_t>(G) * a.cap;                        // [NW][256]
-  float* s_mult = reinterpret_cast<float*>(hist + NW * 256);
+  uint32_t* hist = buf + static_cast<size_t>(G) * a.cap;                        // [kScanWarps][256]
+  float* s_mult = reinterpret_cast<float*>(hist + kScanWarps * 256);
   float* s_bias = s_mult + G;
   uint32_t* s_thr = reinterpret_cast<uint32_t*>(s_bias + G);   // exclusive key bound per query
   uint32_t* s_cnt = s_thr + G;                                 // candidates buffered per query
@@ -111,7 +117,7 @@ __global__ void __launch_bounds__(NW * 32, 16 / NW) lut16_scan_kernel(const Scan
     }
 
     // (1) query residuals: q - centroid (src/tree_x_hybrid/mod.rs:309-316)
-    for (int idx = tid; idx < G * a.dim; idx += NW * 32) {
+    for (int idx = tid; idx < G * a.dim; idx += kScanWarps * 32) {
       int g = idx / a.dim, d = idx - g * a.dim;
       float v = 0.0f;
       if (g < ng) {
@@ -130,8 +136,8 @@ __global__ void __launch_bounds__(NW * 32, 16 / NW) lut16_scan_kernel(const Scan
     __syncthreads();
 
     // (2) LUT16 build (warp g builds query g's table) and (3) the bound for this leaf
-    const int nfull0 = min(NW, static_cast<int>(leaf_n / kBlockPts));  // full blocks of tile 0
-    for (int g = warp; g < G; g += NW) {
+    const int nfull0 = min(kScanWarps, static_cast<int>(leaf_n / kBlockPts));  // full blocks of tile 0
+    for (int g = warp; g < G; g += kScanWarps) {
       uint8_t* l8 = reinterpret_cast<uint8_t*>(lut + g * S4);
       if (g < ng) {
         float mult, bias;
@@ -160,9 +166,9 @@ __global__ void __launch_bounds__(NW * 32, 16 / NW) lut16_scan_kernel(const Scan
     __syncthreads();
 
     // (4)+(5) stream the leaf, one 256-point block per warp per tile
-    const int ntiles = (nblk + NW - 1) / NW;
+    const int ntiles = (nblk + kScanWarps - 1) / kScanWarps;
     for (int t = 0; t < ntiles; ++t) {
-      const int b = t * NW + warp;
+      const int b = t * kScanWarps + warp;
       if (b < nblk) {
         PackedSums ps[G];
         {
@@ -237,7 +243,7 @@ __global__ void __launch_bounds__(NW * 32, 16 / NW) lut16_scan_kernel(const Scan
       }
       __syncthreads();
       // exact compaction to the R best when the buffer could overflow in the next tile; refresh tau
-      for (int g = warp; g < ng; g += NW) {
+      for (int g = warp; g < ng; g += kScanWarps) {
         int c = static_cast<int>(min(s_cnt[g], static_cast<uint32_t>(a.cap)));
         const uint32_t q = s_pair[g] / static_cast<uint32_t>(a.L);
         const int R = a.qR ? static_cast<int>(__ldg(a.qR + q)) : a.R;
@@ -272,7 +278,7 @@ __global__ void __launch_bounds__(NW * 32, 16 / NW) lut16_scan_kernel(const Scan
 
     // (6) write this item's candidates: approx distance = sum*multiplier + bias*S (lut16_simd.rs:136-140)
     if (a.max_blocks > 0) continue;  // probe launch: only the bounds matter
-    for (int g = warp; g < ng; g += NW) {
+    for (int g = warp; g < ng; g += kScanWarps) {
       const uint32_t R = a.qR ? __ldg(a.qR + s_pair[g] / static_cast<uint32_t>(a.L)) : static_cast<uint32_t>(a.R);
       const int c = static_cast<int>(min(s_cnt[g], R));
       const uint32_t pair = s_pair[g];
@@ -306,11 +312,11 @@ __global__ void __launch_bounds__(NW * 32, 16 / NW) lut16_scan_kernel(const Scan
 }
 
 // entries of a query's shared-memory candidate buffer: one tile of unfiltered points + 2R carried, in 32-entry rows
-inline int scan_list_cap(int R, int NW) { return (NW * kBlockPts + 2 * R + 31) / 32 * 32; }
+inline int scan_list_cap(int R) { return (kScanWarps * kBlockPts + 2 * R + 31) / 32 * 32; }
 
-inline size_t scan_smem_bytes(int G, int S4, int dim, int cap, int NW, bool filt) {
+inline size_t scan_smem_bytes(int G, int S4, int dim, int cap, bool filt) {
   return static_cast<size_t>(G) * S4 * 16 + static_cast<size_t>((G * dim + 3) & ~3) * 4 +
-         static_cast<size_t>(G) * cap * 4 + NW * 256 * 4 + static_cast<size_t>(G) * (filt ? 7 : 6) * 4 + 16;
+         static_cast<size_t>(G) * cap * 4 + kScanWarps * 256 * 4 + static_cast<size_t>(G) * (filt ? 7 : 6) * 4 + 16;
 }
 
 }  // namespace scann

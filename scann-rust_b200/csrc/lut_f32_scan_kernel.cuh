@@ -1,7 +1,7 @@
 // The Tree-X-Hybrid scan over byte codes with the reference's f32 LookupTable (tree_x_hybrid/mod.rs:297-339,
 // hashes/lut.rs:47-82): persistent kernel over the same (leaf, <= G queries) work items as lut16_scan_kernel.
 //
-// Per work item a CTA of NW warps
+// Per work item a CTA of kScanWarps warps
 //   (1) stages the G query residuals q - centroid(leaf) in shared memory (skipped without residuals),
 //   (2) builds the G f32 tables [S][C] in shared memory with LookupTable::from_query arithmetic (lut_f32_device.cuh),
 //   (3) streams the leaf's blocked byte codes once for all G queries — one 256-point block per warp per tile, lane l
@@ -63,16 +63,16 @@ __device__ __forceinline__ uint64_t f32_bound_key(uint32_t tk) {
 
 // a.codes: the byte codes in 256-point blocks, block b at byte b * S * 256, subspace-major inside (byte s*256 + j =
 // subspace s of point j).  C: codes per subspace (the table row length).  a.max_blocks / probe launches are not used.
-template <int G, int NW, bool FILT>
-__global__ void __launch_bounds__(NW * 32, 1) lut_f32_scan_kernel(const ScanArgs a, const int C) {
+template <int G, bool FILT>
+__global__ void __launch_bounds__(kScanWarps * 32, 1) lut_f32_scan_kernel(const ScanArgs a, const int C) {
   extern __shared__ __align__(16) uint8_t smem[];
   const int SC = a.S * C;
   uint64_t* buf = reinterpret_cast<uint64_t*>(smem);                  // [G][cap] keys
   uint64_t* s_thr = buf + static_cast<size_t>(G) * a.cap;             // [G] inclusive key bound per query
   float* lut = reinterpret_cast<float*>(s_thr + G);                   // [G][S][C]
   float* qres = lut + static_cast<size_t>(G) * SC;                    // [G][dim]
-  uint32_t* hist = reinterpret_cast<uint32_t*>(qres + G * a.dim);     // [NW][256]
-  uint32_t* s_cnt = hist + NW * 256;                                  // candidates buffered per query
+  uint32_t* hist = reinterpret_cast<uint32_t*>(qres + G * a.dim);     // [kScanWarps][256]
+  uint32_t* s_cnt = hist + kScanWarps * 256;                          // candidates buffered per query
   uint32_t* s_pair = s_cnt + G;                                       // pair id (q * L + rank)
   uint32_t* s_tau = s_pair + G;                                       // last qthr key seen per query
   uint32_t* s_row = s_tau + G;                                        // FILT: filter row (0xFFFFFFFF = none allowed)
@@ -96,7 +96,7 @@ __global__ void __launch_bounds__(NW * 32, 1) lut_f32_scan_kernel(const ScanArgs
     const uint32_t leaf_n = static_cast<uint32_t>(a.pt_off[leaf + 1] - a.pt_off[leaf]);
 
     // (1) query residuals: q - centroid (src/tree_x_hybrid/mod.rs:309-316)
-    for (int idx = tid; idx < ng * a.dim; idx += NW * 32) {
+    for (int idx = tid; idx < ng * a.dim; idx += kScanWarps * 32) {
       const int g = idx / a.dim, d = idx - g * a.dim;
       const uint32_t q = a.sorted_pairs[pbeg + g] / static_cast<uint32_t>(a.L);
       float v = a.queries[static_cast<size_t>(q) * a.dim + d];
@@ -120,13 +120,14 @@ __global__ void __launch_bounds__(NW * 32, 1) lut_f32_scan_kernel(const ScanArgs
 
     // (2) the G tables
     for (int g = 0; g < ng; ++g)
-      lut_f32_build(lut + static_cast<size_t>(g) * SC, qres + g * a.dim, a.codebook, a.S, C, a.ds, tid, NW * 32);
+      lut_f32_build(lut + static_cast<size_t>(g) * SC, qres + g * a.dim, a.codebook, a.S, C, a.ds, tid,
+                    kScanWarps * 32);
     __syncthreads();
 
     // (3)+(4) stream the leaf, one 256-point block per warp per tile
-    const int ntiles = (nblk + NW - 1) / NW;
+    const int ntiles = (nblk + kScanWarps - 1) / kScanWarps;
     for (int t = 0; t < ntiles; ++t) {
-      const int b = t * NW + warp;
+      const int b = t * kScanWarps + warp;
       if (b < nblk) {
         float acc[G][8];
 #pragma unroll
@@ -179,7 +180,7 @@ __global__ void __launch_bounds__(NW * 32, 1) lut_f32_scan_kernel(const ScanArgs
       }
       __syncthreads();
       // exact compaction to the R best when the buffer could overflow in the next tile; refresh the bound
-      for (int g = warp; g < ng; g += NW) {
+      for (int g = warp; g < ng; g += kScanWarps) {
         int c = static_cast<int>(min(s_cnt[g], static_cast<uint32_t>(a.cap)));
         const uint32_t q = s_pair[g] / static_cast<uint32_t>(a.L);
         const int R = a.qR ? static_cast<int>(__ldg(a.qR + q)) : a.R;
@@ -208,7 +209,7 @@ __global__ void __launch_bounds__(NW * 32, 1) lut_f32_scan_kernel(const ScanArgs
     }
 
     // (5) this item's candidates
-    for (int g = warp; g < ng; g += NW) {
+    for (int g = warp; g < ng; g += kScanWarps) {
       const uint32_t pair = s_pair[g];
       const uint32_t R = a.qR ? __ldg(a.qR + pair / static_cast<uint32_t>(a.L)) : static_cast<uint32_t>(a.R);
       const int c = static_cast<int>(min(s_cnt[g], R));
@@ -224,9 +225,10 @@ __global__ void __launch_bounds__(NW * 32, 1) lut_f32_scan_kernel(const ScanArgs
 }
 
 // Shared memory of one CTA: G tables of S*C floats dominate (48 KB per query at S = 48, C = 256).
-inline size_t lut_f32_scan_smem_bytes(int G, int S, int C, int dim, int cap, int NW) {
+inline size_t lut_f32_scan_smem_bytes(int G, int S, int C, int dim, int cap) {
   return static_cast<size_t>(G) * cap * 8 + static_cast<size_t>(G) * 8 + static_cast<size_t>(G) * S * C * 4 +
-         static_cast<size_t>(G) * dim * 4 + static_cast<size_t>(NW) * 256 * 4 + static_cast<size_t>(G) * 4 * 4 + 4 + 16;
+         static_cast<size_t>(G) * dim * 4 + static_cast<size_t>(kScanWarps) * 256 * 4 + static_cast<size_t>(G) * 4 * 4 +
+         4 + 16;
 }
 
 }  // namespace scann

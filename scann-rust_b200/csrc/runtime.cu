@@ -1,6 +1,5 @@
 // Host runtime pieces shared by every entry point: thread-local error text, CUDA error mapping,
 // device checks, the grow-only workspace arena.
-#include <stdlib.h>
 #include <stdarg.h>
 #include <string.h>
 
@@ -48,15 +47,6 @@ int sm_count(int device) {
   int v = 0;
   if (cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, device) != cudaSuccess || v <= 0) v = 148;
   return v;
-}
-
-int scan_acc_mode(int S) {
-  // read each call (cheap) so tests can flip SCANN_ACC_MODE between searches
-  const char* e = getenv("SCANN_ACC_MODE");
-  int m = e ? atoi(e) : 3;
-  if (m < 0 || m > 3) m = 3;
-  if (m == 3 && S > 128) m = 2;  // IDP.2A packing needs per-point sums < 2^15 (128 * 255 = 32640)
-  return m;
 }
 
 scann_status Workspace::reserve(size_t bytes) {

@@ -3,7 +3,6 @@
 // table build / integer accumulation is bit-exact.
 #include <algorithm>
 
-#include "kernels.h"
 #include "lut16_device.cuh"
 
 namespace scann {
@@ -69,8 +68,7 @@ __global__ void repack_flat_kernel(const uint8_t* __restrict__ packed, size_t n,
 template <int MODE>
 __global__ void __launch_bounds__(256) lut16_scan_all_kernel(const uint4* __restrict__ codes, size_t nblocks, int S,
                                                              int SG, const uint8_t* __restrict__ lut8, size_t n,
-                                                             uint32_t* __restrict__ sums, uint32_t one,
-                                                             uint32_t sh24) {
+                                                             uint32_t* __restrict__ sums, uint32_t one) {
   extern __shared__ __align__(16) uint8_t sm[];
   const int S4 = SG * 4;
   for (int e = threadIdx.x; e < S4 * 16; e += blockDim.x) sm[e] = e < S * 16 ? lut8[e] : 0;
@@ -81,7 +79,6 @@ __global__ void __launch_bounds__(256) lut16_scan_all_kernel(const uint4* __rest
     PackedSums ps[1];
     AccMul mul;
     mul.one = one;
-    mul.sh24 = sh24;
     mul.w15 = 0x80000001u;
     scan_block<1, MODE>(codes + b * SG * 32, SG, lut, S4, lane, mul, ps);
     uint32_t s1[8];
@@ -211,18 +208,10 @@ scann_status scann_lut16_scan(const uint8_t* packed, size_t n, size_t S, const u
                                                                           static_cast<int>(SG), words, d_codes.p);
   SCANN_CUDA(cudaGetLastError());
   unsigned grid = static_cast<unsigned>(std::min<size_t>((nblocks + 7) / 8, 148 * 8));
-  // same accumulation mode as the product path would pick for this S (treeah.cu launch_scan)
-  const int mode = scan_acc_mode(static_cast<int>(S));
-  auto launch = [&](auto kern) {
-    kern<<<grid, 256, SG * 4 * 16>>>(reinterpret_cast<const uint4*>(d_codes.p), nblocks, static_cast<int>(S),
-                                     static_cast<int>(SG), pl, n, ps, 1u, 1u << 24);
-  };
-  switch (mode) {
-    case 0: launch(lut16_scan_all_kernel<0>); break;
-    case 1: launch(lut16_scan_all_kernel<1>); break;
-    case 3: launch(lut16_scan_all_kernel<3>); break;
-    default: launch(lut16_scan_all_kernel<2>); break;
-  }
+  // same accumulation mode as the product path picks for this S (treeah.cu launch_scan_g)
+  auto kern = scan_acc_mode(static_cast<int>(S)) == 3 ? lut16_scan_all_kernel<3> : lut16_scan_all_kernel<2>;
+  kern<<<grid, 256, SG * 4 * 16>>>(reinterpret_cast<const uint4*>(d_codes.p), nblocks, static_cast<int>(S),
+                                   static_cast<int>(SG), pl, n, ps, 1u);
   SCANN_CUDA(cudaGetLastError());
   if (host) SCANN_CUDA(cudaMemcpy(sums, ps, n * 4, cudaMemcpyDeviceToHost));
   SCANN_CUDA(cudaDeviceSynchronize());

@@ -29,9 +29,9 @@
 //       warps 1-2    one lane each (one per accumulator) issues tcgen05.mma.sp.kind::i8, M = 128 points, N = 16..128
 //                    queries, K = 64 bytes; the compressed A operand and its metadata are read from TENSOR MEMORY, the
 //                    accumulator (s32) is double-buffered in TMEM
-//       warps 4-11   expanders (warps 4-19 with SCANN_TC_EXP=4): thread = one point; turn its packed 4-bit codes into
-//                    compressed one-hot values and metadata in registers, 16 subspaces (256 K-bytes) at a time, and
-//                    tcgen05.st them into a ring of A slots in TMEM
+//       warps 4-11   expanders: thread = one point; turn its packed 4-bit codes into compressed one-hot values and
+//                    metadata in registers, 16 subspaces (256 K-bytes) at a time, and tcgen05.st them into a ring of A
+//                    slots in TMEM
 //       last 8 warps epilogue: tcgen05.ld the accumulator (thread = one point, columns = queries), threshold, append the
 //                    survivors (approx distance key | leaf rank | position) to per-query candidate lists
 //   Threshold without a per-column compare: the LUT row of (query, leaf) carries two extra bytes (d0, d1) with
@@ -58,8 +58,8 @@ namespace scann {
 
 namespace {
 
-// warp 0 TMA, 1-2 MMA issuers, 3 TMEM owner, then 4 * EG expander warps, then 8 epilogue warps
-constexpr int ts_threads(int EG) { return 32 * (4 + 4 * EG + 8); }
+// warp 0 TMA, 1-2 MMA issuers, 3 TMEM owner, 4-11 expanders (two groups of four), 12-19 epilogue
+constexpr int kTsThreads = 32 * (4 + 8 + 8);
 constexpr int kTsRing = 6;            // A slots: 16 subspaces (256 dense K-bytes) of a point row each
 constexpr int kTsHalf = kTsRing / 2;  // each pipeline owns half of the ring: 48 subspaces, a whole S = 48 tile
 constexpr int kTsAcol = 256;          // TMEM columns of the slots' compressed values, 32 per slot (accumulators: 2 x 128
@@ -87,10 +87,6 @@ __device__ __forceinline__ void mbar_arrive(uint32_t bar) {
 // Bounded wait: a protocol error becomes a trap (reported as a CUDA error by the next API call) instead of a hang.
 // g_tcs_dbg (host-mapped, optional): where the wait that timed out was — {1, barrier smem address, parity, tag}.
 __device__ volatile uint32_t* g_tcs_dbg = nullptr;
-__device__ __forceinline__ void dbg_mark(int idx, uint32_t v) {
-  volatile uint32_t* d = g_tcs_dbg;
-  if (d != nullptr && blockIdx.x == 0) d[8 + idx] = v;
-}
 __device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity, uint32_t tag = 0) {
   uint32_t ok = 0;
   for (uint32_t it = 0; !ok; ++it) {
@@ -272,55 +268,48 @@ __device__ __forceinline__ void tcwl_entry(uint32_t leaf, const uint32_t* __rest
 }
 
 // One CTA: exclusive scans over the leaves in `perm` order (largest leaves first, so the statically dealt items end on
-// the small ones) of pairs / groups / items.  counters: [0] items, [1] groups.
+// the small ones) of groups / items.  counters: [0] items, [1] groups.
 __global__ void __launch_bounds__(1024) tcwl_scan_kernel(const uint32_t* __restrict__ leaf_cnt, uint32_t K,
                                                          const uint32_t* __restrict__ perm,
                                                          const uint64_t* __restrict__ pt_off,
-                                                         uint32_t* __restrict__ pair_start,
                                                          uint32_t* __restrict__ group_start,
                                                          uint32_t* __restrict__ item_start,
                                                          uint32_t* __restrict__ counters,
                                                          unsigned long long* __restrict__ pair_points) {
-  __shared__ uint32_t s_p[1024], s_g[1024], s_i[1024];
+  __shared__ uint32_t s_g[1024], s_i[1024];
   unsigned long long pp_local = 0;
   const uint32_t per = (K + 1023) / 1024;
   const uint32_t b = threadIdx.x * per, e = min(K, b + per);
-  uint32_t sp = 0, sg = 0, si = 0;
+  uint32_t sg = 0, si = 0;
   for (uint32_t i = b; i < e; ++i) {
     uint32_t pc, g, c;
     tcwl_entry(perm[i], leaf_cnt, pt_off, pc, g, c);
-    sp += pc;
     sg += g;
     si += g * c;
     pp_local += static_cast<unsigned long long>(pc) * (pt_off[perm[i] + 1] - pt_off[perm[i]]);
   }
   if (pair_points && pp_local) atomicAdd(pair_points, pp_local);
-  s_p[threadIdx.x] = sp;
   s_g[threadIdx.x] = sg;
   s_i[threadIdx.x] = si;
   __syncthreads();
   for (int o = 1; o < 1024; o <<= 1) {
-    uint32_t vp = 0, vg = 0, vi = 0;
+    uint32_t vg = 0, vi = 0;
     if (threadIdx.x >= o) {
-      vp = s_p[threadIdx.x - o];
       vg = s_g[threadIdx.x - o];
       vi = s_i[threadIdx.x - o];
     }
     __syncthreads();
-    s_p[threadIdx.x] += vp;
     s_g[threadIdx.x] += vg;
     s_i[threadIdx.x] += vi;
     __syncthreads();
   }
-  uint32_t rp = s_p[threadIdx.x] - sp, rg = s_g[threadIdx.x] - sg, ri = s_i[threadIdx.x] - si;
+  uint32_t rg = s_g[threadIdx.x] - sg, ri = s_i[threadIdx.x] - si;
   for (uint32_t i = b; i < e; ++i) {
     const uint32_t leaf = perm[i];
     uint32_t pc, g, c;
     tcwl_entry(leaf, leaf_cnt, pt_off, pc, g, c);
-    pair_start[leaf] = rp;
     group_start[leaf] = rg;
     item_start[leaf] = ri;
-    rp += pc;
     rg += g;
     ri += g * c;
   }
@@ -512,8 +501,8 @@ struct TcsArgs {
   int L;
 };
 
-// restrict filters of the filtered instantiation (TcScanParams).  A kernel parameter of its own: widening TcsArgs alone
-// made ptxas spill in the unfiltered EG = 4 kernel.
+// restrict filters of the filtered instantiation (TcScanParams).  A kernel parameter of its own, so that TcsArgs and
+// the unfiltered kernel do not carry them.
 struct TcsFilter {
   const uint8_t* allow;
   size_t allow_stride;
@@ -551,11 +540,10 @@ __device__ __forceinline__ void tcs_emit(const TcsArgs& a, const TcsFilter& f, u
 constexpr int kWqCap = 320;    // entries of one epilogue warp's survivor queue (uint4 {lut_row, acc, pos, leaf (FILT)})
 constexpr int kWqStep = 256;   // most entries one filter step (32 lanes x 8 columns) can add
 
-// EG: expander groups, 2 (one per pipeline) or 4 (two per pipeline, alternate slots); FILT: restrict filters (a template
-// flag, so the unfiltered kernel carries none of it)
-template <int EG, bool FILT>
-__global__ void __launch_bounds__(ts_threads(EG), 1) tc_scan_kernel(const __grid_constant__ CUtensorMap tmB, const TcsArgs a,
-                                                                    const TcsFilter filt) {
+// FILT: restrict filters (a template flag, so the unfiltered kernel carries none of it)
+template <bool FILT>
+__global__ void __launch_bounds__(kTsThreads, 1) tc_scan_kernel(const __grid_constant__ CUtensorMap tmB,
+                                                                const TcsArgs a, const TcsFilter filt) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* sB = smem;  // [KA + 1] atom tiles
@@ -662,15 +650,10 @@ __global__ void __launch_bounds__(ts_threads(EG), 1) tc_scan_kernel(const __grid
         tc_commit(bar(kBEmpty));  // this pipeline's MMAs on the B tile have retired
       }
     }
-  } else if (warp >= 4 && warp < 4 + 4 * EG) {
+  } else if (warp >= 4 && warp < 12) {
     // ================================================================= expanders: codes -> sparse one-hot A slots in TMEM
-    // Groups of four warps (one warp per TMEM lane quadrant): pipeline pp takes the tiles of parity pp.  With EG = 4
-    // the two groups of a pipeline take alternate slots (by the parity of the pipeline's running slot count m), so the
-    // uses of one A slot (m % 3) alternate between them.  A parity wait needs the barrier at most one phase behind: the
-    // group's previous slot m - 2 waited for the release of m - 5, and one pipeline's commits complete in order, so
-    // m - 6 (the use before last of this slot) has been released.
-    const uint32_t gi = static_cast<uint32_t>(warp - 4) >> 2;
-    const uint32_t pp = EG == 4 ? gi >> 1 : gi, sg = gi & 1u;
+    // Two groups of four warps (one warp per TMEM lane quadrant): group pp takes the tiles of parity pp.
+    const uint32_t pp = static_cast<uint32_t>(warp - 4) >> 2;
     const uint32_t quad = warp & 3;
     const uint32_t row = quad * 32 + lane;
     const uint32_t lane_addr = (quad * 32) << 16;
@@ -710,7 +693,7 @@ __global__ void __launch_bounds__(ts_threads(EG), 1) tc_scan_kernel(const __grid
 #pragma unroll
         for (int c = 0; c < 4; ++c) {
           const uint32_t m = m0 + c;
-          if (c < nslot && (EG == 2 || (m & 1u) == sg)) {
+          if (c < nslot) {
             const uint32_t slot = pp * kTsHalf + (m % kTsHalf);
             uint32_t r[32], mt[8];
             // rows past the end of the leaf expand code 0: the epilogue ignores them
@@ -726,12 +709,12 @@ __global__ void __launch_bounds__(ts_threads(EG), 1) tc_scan_kernel(const __grid
         publish();
       }
     }
-  } else if (warp >= 4 + 4 * EG) {
+  } else if (warp >= 12) {
     // ================================================================= epilogue: threshold + candidate append
     // Eight warps: two per TMEM lane quadrant, one for accumulator columns 0..63 and one for 64..127, so the
     // accumulator goes back to its MMA warp after ONE round of TMEM loads (a pipeline cannot start its next tile
     // before that).
-    const uint32_t ew = static_cast<uint32_t>(warp - (4 + 4 * EG));  // 0..7
+    const uint32_t ew = static_cast<uint32_t>(warp - 12);  // 0..7
     const uint32_t half_id = ew >> 2;
     const uint32_t quad = warp & 3;
     const uint32_t row = quad * 32 + lane;
@@ -873,7 +856,7 @@ size_t tc_scan_max_items(size_t P, size_t K, size_t max_leaf) {
 TcScanBufs take_tc_scan(Workspace& ws, size_t nq, size_t L, size_t K, size_t S, size_t max_leaf, size_t qcap) {
   const size_t P = nq * L, G = tc_scan_max_groups(P, K);
   TcScanBufs b;
-  b.starts = ws.take<uint32_t>(3 * (K + 1));
+  b.starts = ws.take<uint32_t>(2 * (K + 1));
   b.counters = ws.take<uint32_t>(4);
   b.groups = ws.take<uint4>(G);
   b.items = ws.take<uint4>(tc_scan_max_items(P, K, max_leaf));
@@ -893,7 +876,7 @@ scann_status launch_tc_scan(const TcScanParams& p, Workspace& ws, TcScanOut* out
   const auto [starts, counters, groups, items, meta, lut, qcand, qcnt, qflag, fb_tokens] =
       take_tc_scan(ws, p.nq, p.L, K, S, p.max_leaf, p.qcap);
   SCANN_TRY(ws.check("tensor-core scan"));
-  uint32_t *pair_start = starts, *group_start = starts + (K + 1), *item_start = starts + 2 * (K + 1);
+  uint32_t *group_start = starts, *item_start = starts + (K + 1);
 
   const char* dbg_env = getenv("SCANN_TC_DEBUG");
   const bool dbg = dbg_env && dbg_env[0] == '1';
@@ -905,9 +888,9 @@ scann_status launch_tc_scan(const TcScanParams& p, Workspace& ws, TcScanOut* out
   SCANN_CUDA(cudaMemsetAsync(qflag, 0, p.nq * 4, s));
   const unsigned pb = static_cast<unsigned>((P + 255) / 256);
   // the pairs come grouped by leaf from the caller's worklist (class B of treeah.cu's treeah_worklist): only the group
-  // and item tables are built here (tcwl_scan_kernel also writes pair starts of its own, which nothing reads)
-  tcwl_scan_kernel<<<1, 1024, 0, s>>>(p.wl_cnt, static_cast<uint32_t>(K), p.leaf_perm, p.pt_off, pair_start,
-                                      group_start, item_start, counters, p.pair_points);
+  // and item tables are built here
+  tcwl_scan_kernel<<<1, 1024, 0, s>>>(p.wl_cnt, static_cast<uint32_t>(K), p.leaf_perm, p.pt_off, group_start,
+                                      item_start, counters, p.pair_points);
   tcwl_items_kernel<<<static_cast<unsigned>((K + 127) / 128), 128, 0, s>>>(p.wl_cnt, static_cast<uint32_t>(K), p.pt_off,
                                                                           p.wl_pair_start, group_start, item_start,
                                                                           groups, items);
@@ -968,10 +951,7 @@ scann_status launch_tc_scan(const TcScanParams& p, Workspace& ws, TcScanOut* out
   // >= 120 KB keeps it at one CTA per SM for every S (a second resident CTA would block in tcgen05.alloc)
   const size_t smem = std::max<size_t>(120 * 1024, 1024 + static_cast<size_t>(a.KA + 1) * kTsAtom + 32 * 8 + 64 +
                                                        8 * kWqCap * 16 + 64);
-  const char* eg_env = getenv("SCANN_TC_EXP");
-  const bool eg4 = eg_env && eg_env[0] == '4';
-  auto kern = eg4 ? (filt ? tc_scan_kernel<4, true> : tc_scan_kernel<4, false>)
-                  : (filt ? tc_scan_kernel<2, true> : tc_scan_kernel<2, false>);
+  auto kern = filt ? tc_scan_kernel<true> : tc_scan_kernel<false>;
   SCANN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
   static uint32_t* h_dbg = nullptr;
   if (dbg && h_dbg == nullptr) {
@@ -982,7 +962,7 @@ scann_status launch_tc_scan(const TcScanParams& p, Workspace& ws, TcScanOut* out
       cudaMemcpyToSymbol(g_tcs_dbg, &d_dbg, sizeof(d_dbg));
     }
   }
-  kern<<<p.sms, ts_threads(eg4 ? 4 : 2), smem, s>>>(tmB, a, tf);
+  kern<<<p.sms, kTsThreads, smem, s>>>(tmB, a, tf);
   SCANN_CUDA(cudaGetLastError());
   if (dbg) {
     cudaError_t e = cudaStreamSynchronize(s);
@@ -990,9 +970,6 @@ scann_status launch_tc_scan(const TcScanParams& p, Workspace& ws, TcScanOut* out
     {
       fprintf(stderr, "[tcscan] scan kernel failed (%s): timed-out wait = %u, barrier smem 0x%x, parity %u, tag 0x%x, cta %u, thread %u\n",
               cudaGetErrorString(e), h_dbg[0], h_dbg[1], h_dbg[2], h_dbg[3], h_dbg[4], h_dbg[5]);
-      fprintf(stderr, "[tcscan] cta 0 progress marks (warp: value):");
-      for (int w = 0; w < 14; ++w) fprintf(stderr, " %d:0x%x", w, h_dbg[8 + w]);
-      fprintf(stderr, "\n");
     }
   }
   if (dbg) cudaEventRecord(ev[3], s);

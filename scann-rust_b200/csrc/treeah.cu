@@ -651,101 +651,57 @@ struct scann_treeah {
 
 namespace scann {
 
-// 8 warps per scan CTA (2 CTAs/SM).  Measured on B200 at C3: 8 warps 35.6 ms, 4 warps 35.8 ms, 2 warps 44.7 ms
-// (profiles/r1_scan_kernel.md).
-constexpr int kScanWarps = 8;
 constexpr size_t kScanSmemMax = 227 * 1024;  // dynamic shared memory a CTA may opt in to
 
-template <int G, int MODE, int NW, bool FILT>
-static scann_status launch_scan_mode(ScanArgs a, int sms, cudaStream_t s) {
-  a.cap = scan_list_cap(a.R, NW);
-  size_t smem = scan_smem_bytes(G, a.SG * 4, a.dim, a.cap, NW, FILT);
+// A persistent scan kernel of kScanWarps warps per CTA with smem bytes of dynamic shared memory, on as many CTAs as
+// the device holds at once
+template <typename... Params, typename... Args>
+static scann_status launch_scan_kernel(void (*kern)(Params...), size_t smem, int sms, cudaStream_t s, Args... args) {
   SCANN_REQUIRE(smem <= kScanSmemMax, SCANN_RESOURCE_EXHAUSTED, "scan kernel needs %zu B of shared memory (R too large)",
                 smem);
-  SCANN_CUDA(cudaFuncSetAttribute(lut16_scan_kernel<G, MODE, NW, FILT>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  static_cast<int>(smem)));
-  int occ = 0;
-  SCANN_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, lut16_scan_kernel<G, MODE, NW, FILT>, NW * 32, smem));
-  if (occ < 1) occ = 1;
-  lut16_scan_kernel<G, MODE, NW, FILT><<<sms * occ, NW * 32, smem, s>>>(a);
-  SCANN_CUDA(cudaGetLastError());
-  return SCANN_OK;
-}
-
-// The restrict filter is a template flag so the unfiltered kernel carries none of it.
-template <int G, int MODE>
-static scann_status launch_scan_nw(const ScanArgs& a, int sms, cudaStream_t s) {
-  if (a.allow != nullptr) return launch_scan_mode<G, MODE, kScanWarps, true>(a, sms, s);
-  return launch_scan_mode<G, MODE, kScanWarps, false>(a, sms, s);
-}
-
-template <int G>
-static scann_status launch_scan(const ScanArgs& a, int sms, cudaStream_t s) {
-  switch (scan_acc_mode(a.S)) {
-    case 0: return launch_scan_nw<G, 0>(a, sms, s);
-    case 1: return launch_scan_nw<G, 1>(a, sms, s);
-    case 3: return launch_scan_nw<G, 3>(a, sms, s);
-    default: return launch_scan_nw<G, 2>(a, sms, s);
-  }
-}
-
-// blocks of each closest leaf the probe launch scans (256 points each); SCANN_PROBE_BLOCKS overrides (tuning)
-static int probe_blocks() {
-  const char* e = getenv("SCANN_PROBE_BLOCKS");
-  const int v = e ? atoi(e) : 16;
-  return v >= 1 && v <= 4096 ? v : 16;
-}
-
-static scann_status launch_scan_g(int G, const ScanArgs& a, int sms, cudaStream_t s) {
-  switch (G) {
-    case 8: return launch_scan<8>(a, sms, s);
-    case 4: return launch_scan<4>(a, sms, s);
-    case 2: return launch_scan<2>(a, sms, s);
-    default: return launch_scan<1>(a, sms, s);
-  }
-}
-
-// the byte-code scan (lut_f32_scan_kernel.cuh); C = codes per subspace
-template <int G, bool FILT>
-static scann_status launch_f32_scan(ScanArgs a, int C, int sms, cudaStream_t s) {
-  a.cap = scan_list_cap(a.R, kScanWarps);
-  const size_t smem = lut_f32_scan_smem_bytes(G, a.S, C, a.dim, a.cap, kScanWarps);
-  SCANN_REQUIRE(smem <= kScanSmemMax, SCANN_RESOURCE_EXHAUSTED, "scan kernel needs %zu B of shared memory (R too large)",
-                smem);
-  auto kern = lut_f32_scan_kernel<G, kScanWarps, FILT>;
   SCANN_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
   int occ = 0;
   SCANN_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, kScanWarps * 32, smem));
   if (occ < 1) occ = 1;
-  kern<<<sms * occ, kScanWarps * 32, smem, s>>>(a, C);
+  kern<<<sms * occ, kScanWarps * 32, smem, s>>>(args...);
   SCANN_CUDA(cudaGetLastError());
   return SCANN_OK;
 }
 
+// The scan kernel of the handle's code format with G queries per work item: the register-LUT scan of nibble codes
+// (lut16_scan_kernel.cuh) in the accumulation mode of S, or the f32-table scan of byte codes (lut_f32_scan_kernel.cuh).
+// The restrict filter is a template flag so the unfiltered kernels carry none of it.
 template <int G>
-static scann_status launch_f32_scan_filt(const ScanArgs& a, int C, int sms, cudaStream_t s) {
-  if (a.allow != nullptr) return launch_f32_scan<G, true>(a, C, sms, s);
-  return launch_f32_scan<G, false>(a, C, sms, s);
+static scann_status launch_scan_g(const scann_treeah* h, ScanArgs a, cudaStream_t s) {
+  a.cap = scan_list_cap(a.R);
+  const bool filt = a.allow != nullptr;
+  if (h->f32lut) {
+    const int C = static_cast<int>(h->C);
+    return launch_scan_kernel(filt ? lut_f32_scan_kernel<G, true> : lut_f32_scan_kernel<G, false>,
+                              lut_f32_scan_smem_bytes(G, a.S, C, a.dim, a.cap), h->sms, s, a, C);
+  }
+  auto kern = filt ? lut16_scan_kernel<G, 2, true> : lut16_scan_kernel<G, 2, false>;
+  if (scan_acc_mode(a.S) == 3) kern = filt ? lut16_scan_kernel<G, 3, true> : lut16_scan_kernel<G, 3, false>;
+  return launch_scan_kernel(kern, scan_smem_bytes(G, a.SG * 4, a.dim, a.cap, filt), h->sms, s, a);
 }
 
-// the scan kernel of the handle's code format, G queries per work item
 static scann_status launch_handle_scan(const scann_treeah* h, int G, const ScanArgs& a, cudaStream_t s) {
-  if (!h->f32lut) return launch_scan_g(G, a, h->sms, s);
-  const int C = static_cast<int>(h->C);
   switch (G) {
-    case 8: return launch_f32_scan_filt<8>(a, C, h->sms, s);
-    case 4: return launch_f32_scan_filt<4>(a, C, h->sms, s);
-    case 2: return launch_f32_scan_filt<2>(a, C, h->sms, s);
-    default: return launch_f32_scan_filt<1>(a, C, h->sms, s);
+    case 8: return launch_scan_g<8>(h, a, s);
+    case 4: return launch_scan_g<4>(h, a, s);
+    case 2: return launch_scan_g<2>(h, a, s);
+    default: return launch_scan_g<1>(h, a, s);
   }
 }
+
+// blocks of each closest leaf the probe launch scans: 16 x 256 = 4096 points (scann_b200.h)
+constexpr int kProbeBlocks = 16;
 
 // shared memory of one scan CTA of the handle's code format with G queries per work item
 static size_t scan_cta_bytes(const scann_treeah* h, int G, int cap, bool filt) {
   if (h->f32lut)
-    return lut_f32_scan_smem_bytes(G, static_cast<int>(h->S), static_cast<int>(h->C), static_cast<int>(h->dim), cap,
-                                   kScanWarps);
-  return scan_smem_bytes(G, static_cast<int>(h->SG) * 4, static_cast<int>(h->dim), cap, kScanWarps, filt);
+    return lut_f32_scan_smem_bytes(G, static_cast<int>(h->S), static_cast<int>(h->C), static_cast<int>(h->dim), cap);
+  return scan_smem_bytes(G, static_cast<int>(h->SG) * 4, static_cast<int>(h->dim), cap, filt);
 }
 
 // Worklist of the register-LUT scan over `tokens` (buffers in h->ck): count -> scans -> scatter -> items.  with_stats:
@@ -845,7 +801,7 @@ static void treeah_plan(const scann_treeah* h, size_t nq, size_t L, size_t R, co
   int G = avg >= 6.0 ? 8 : (avg >= 3.0 ? 4 : (avg >= 1.5 ? 2 : 1));
   // the scan CTA holds G queries' residuals, tables and candidate buffers: smaller groups where they do not fit (each
   // pair's per-leaf top-R does not depend on which queries share its item, so results stay the same)
-  const int cap = scan_list_cap(static_cast<int>(R), kScanWarps);
+  const int cap = scan_list_cap(static_cast<int>(R));
   while (G > 1 && scan_cta_bytes(h, G, cap, filtered) > kScanSmemMax) G /= 2;
   ck.nq = nq;
   ck.L = L;
@@ -940,7 +896,6 @@ static scann_status treeah_phase1(scann_treeah* h, const float* dq, size_t k, bo
   a.cand_cnt = ck.cand_cnt;
   a.qthr = ck.qthr;
   a.mul.one = 1u;
-  a.mul.sh24 = 1u << 24;
   a.mul.w15 = 0x80000001u;
   a.dim = static_cast<int>(h->dim);
   a.S = static_cast<int>(h->S);
@@ -948,19 +903,19 @@ static scann_status treeah_phase1(scann_treeah* h, const float* dq, size_t k, bo
   a.SG = static_cast<int>(h->SG);
   a.L = static_cast<int>(L);
   a.R = static_cast<int>(R);
-  a.cap = 0;  // set per CTA shape in launch_scan_mode
+  a.cap = 0;  // set per CTA shape in launch_scan_g
   a.pos_bits = h->pos_bits;
   a.use_residuals = h->use_residuals;
   h->prof_launches += (ck.partition ? h->part.launches() : 0) + 7;  // partition + 7 worklist kernels
   if (two_phase) {
-    // 3a. probe of the class-A items: the first probe_blocks() blocks of every query's closest leaf prove a bound in
+    // 3a. probe of the class-A items: the first kProbeBlocks blocks of every query's closest leaf prove a bound in
     // bounded time (a full scan of the largest leaves would serialise on a few CTAs); phase 2 scans them in full
     h->span_begin(2, s);
     a.end_idx = 2;
     // tensor-core mode: the class-A ranks are scanned in full here (their per-leaf lists are final, phase 2 does not
     // come back to them); otherwise a bounded probe of the closest leaf
-    a.max_blocks = ck.use_tc ? 0 : probe_blocks();
-    SCANN_TRY(launch_scan_g(ck.G, a, h->sms, s));
+    a.max_blocks = ck.use_tc ? 0 : kProbeBlocks;
+    SCANN_TRY(launch_handle_scan(h, ck.G, a, s));
     h->prof_launches += 1;
     if (ck.use_tc) {  // the class-A lists are final: their union bounds the tensor-core pass
       union_bound_kernel<<<static_cast<unsigned>((nq + 7) / 8), 256, 0, s>>>(
@@ -1292,7 +1247,7 @@ static scann_status treeah_create(const float* centers, size_t K, size_t dim, co
     SCANN_REQUIRE(C >= 1 && C <= 256, SCANN_INVALID_ARGUMENT, "num_codes %zu outside 1..256", C);
     // the scan CTA holds one query's S x C table: a geometry that does not fit with one query and R = 1 cannot be searched
     const size_t smem = lut_f32_scan_smem_bytes(1, static_cast<int>(S), static_cast<int>(C), static_cast<int>(dim),
-                                                scan_list_cap(1, kScanWarps), kScanWarps);
+                                                scan_list_cap(1));
     SCANN_REQUIRE(smem <= kScanSmemMax, SCANN_OUT_OF_RANGE,
                   "S=%zu x C=%zu f32 lookup table: the scan needs %zu B of shared memory per query (> %zu)", S, C, smem,
                   kScanSmemMax);

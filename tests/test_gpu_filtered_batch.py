@@ -274,10 +274,10 @@ def test_filtered_search_from_two_threads(gpu_lib, small):
     assert not errors, errors
 
 
-def test_cpp_mirror_filtered_batch(gpu_lib):
+def test_cpp_mirror_filtered_batch(gpu_lib, tmp_path):
     libdir = os.path.dirname(gpu_lib.build_lib.build())
     src = os.path.join(ROOT, "tests", "cpp", "test_hpp_filtered.cpp")
-    exe = os.path.join(ROOT, "tests", "cpp", "test_hpp_filtered.bin")
+    exe = str(tmp_path / "test_hpp_filtered.bin")
     subprocess.check_call(["g++", "-std=c++17", "-O1", "-Wall", "-I", os.path.join(ROOT, "include"), src, "-o", exe,
                            "-L", libdir, "-lscann_b200", f"-Wl,-rpath,{libdir}"])
     out = subprocess.run([exe], capture_output=True, text=True, timeout=120)

@@ -64,13 +64,11 @@ def test_lut16_scan_accumulators_bit_exact(gpu_lib, oracle, S, n):
     assert (got == want).all()
 
 
-@pytest.mark.parametrize("mode", [0, 1, 2, 3])
 @pytest.mark.parametrize("S", [48, 128, 129])
-def test_lut16_scan_every_accumulation_mode(gpu_lib, oracle, monkeypatch, mode, S):
-    # the four accumulation variants of scan_block (ALU adds, IMAD/IMAD.HI, IMAD/LEA.HI, IDP.2A) give the same
-    # integers; S = 128 with all-255 tables is the largest sum the 15-bit IDP.2A fields must hold (32640),
-    # S = 129 must fall back to mode 2 by itself
-    monkeypatch.setenv("SCANN_ACC_MODE", str(mode))
+def test_lut16_scan_accumulation_mode_of_s(gpu_lib, oracle, S):
+    # scan_block accumulates with IDP.2A (mode 3) for S <= 128 and with IMAD/ALU adds (mode 2) above; S = 128 with
+    # all-255 tables is the largest sum the 15-bit IDP.2A fields must hold (32640), S = 129 is the first S of mode 2
+    mode = 3 if S <= 128 else 2  # scan_acc_mode(S)
     rng = np.random.default_rng(S * 7 + mode)
     n = 10_007
     codes = rng.integers(0, 16, (n, S), dtype=np.uint8)
